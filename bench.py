@@ -358,6 +358,18 @@ def hbm_peak_gbs():
         return 6550.0, "fallback (B200_PROFILING.md: ~6.55 TB/s measured copy bandwidth)"
 
 
+def dump_outputs(out_dir, fit):
+    """Write what one oem_fit_big call returned as float64 .npy files, one set per penalty (a few MB at p = 1000), so that
+    two builds run with the same arguments, and therefore on the same seeded inputs, can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"d": np.array([fit["d"]])}
+    for k, pen in enumerate(PENALTIES):
+        for key in ("beta", "lambda_", "niter", "loss"):
+            arrays[f"{key.rstrip('_')}_{pen}"] = fit[key][k]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     import oem_b200
@@ -437,6 +449,8 @@ def run_ours(args):
     ms_step, outs = timed(step_dev, args.steps)
     walls_dev = timed.last_walls
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs[-1])
     st = outs[-1]["stats"]
     gram_ms = float(np.mean([o["stats"]["ms_gram"] / max(1, o["stats"]["gram_launches"]) for o in outs]))
     gram_flops = st["gram_flops"] / max(1, st["gram_launches"])
@@ -812,7 +826,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--allow-partial-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed fit returned (beta, lambda, niter, loss per "
+                         "penalty, and d) as float64 DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

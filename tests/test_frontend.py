@@ -264,3 +264,36 @@ def test_bench_reference_arm_smoke(tmp_path):
     assert cb["cores"] == len(os.sched_getaffinity(0)) or cb["cores"] >= 1          # the pool size that was set, not the env's 1
     if len(os.sched_getaffinity(0)) > 1:
         assert cb["cores"] > 1
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_match_a_fit_of_the_seeded_inputs(lib, tmp_path):
+    """bench.py --dump-outputs on a small shard: the timed steps run as many times as --steps says, and the dumped arrays
+    (float64, one file per returned array and penalty) equal a fit of the same seeded inputs made here."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import torch
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    rows, dump = 20_000, tmp_path / "dump"
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "3",
+                          "--rows", str(rows), "--no-e2e", "--no-cpu", "--no-secondary", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=900, cwd=root)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and len(line["config"]["host_wall_ms_per_step"]) == 2
+    sys.path.insert(0, root)
+    import bench
+    X, y = bench.gen_shard(torch, rows, 105_000, torch.device("cuda", 0))
+    ref = lib.oem_fit_big(*bench.fit_args(X, y))
+    names = {"d.npy"}
+    for k, pen in enumerate(bench.PENALTIES):
+        for key in ("beta", "lambda_", "niter", "loss"):
+            name = f"{key.rstrip('_')}_{pen}.npy"
+            names.add(name)
+            got = np.load(dump / name)
+            assert got.dtype == np.float64 and got.shape == ref[key][k].shape, name
+            assert np.allclose(got, ref[key][k], rtol=1e-10, atol=1e-12), name
+    assert set(os.listdir(dump)) == names
+    assert np.load(dump / "d.npy")[0] == pytest.approx(ref["d"], rel=1e-12)

@@ -192,6 +192,17 @@ int oemb200_xval_dense(const double *x, int64_t n, int p, int64_t ldx, const dou
                        const oemb200_spec *spec, int nfolds, const int *foldid,
                        const char *type_measure, const oemb200_opts *opts, oemb200_result *res);
 
+/* Binomial cross-validation (the reference's xval.oem stops on the binomial family, R/oem_xval.R:160-163): the full-data
+ * model is oemb200_fit_logistic_dense on all rows, fold model k the same fit on the rows with foldid != k at the full
+ * model's lambda sequence; every IRLS data pass serves all nfolds + 1 models in one sweep of x.  Result as for
+ * oemb200_xval_dense (beta / lambda / niter / loss / d of the full model).  cvm / cvsd: mean over all n rows of the
+ * held-out measure of cv.oem (R/cv_oem.R:288-330) and sqrt(M2 / (n - 1)) / sqrt(n); type_measure "deviance" (default,
+ * NULL) | "class" | "mse" | "mae" ("auc" needs per-fold ranks: OEMB200_EINVAL).  OEMB200_EUNSUPPORTED for
+ * opts->hessian_full, observation weights, row-sharded calls and p outside 8..2048. */
+int oemb200_xval_logistic_dense(const double *x, int64_t n, int p, int64_t ldx, const double *y,
+                                const oemb200_spec *spec, int nfolds, const int *foldid,
+                                const char *type_measure, const oemb200_opts *opts, oemb200_result *res);
+
 /* src/oem_logistic_dense.cpp:29 -- y in {0,1}. */
 int oemb200_fit_logistic_dense(const double *x, int64_t n, int p, int64_t ldx, const double *y,
                                const oemb200_spec *spec, const oemb200_opts *opts,
@@ -266,6 +277,9 @@ int oemb200_xval_dense_h(const oemb200_matrix *x, const double *y, const oemb200
                          oemb200_result *res);
 int oemb200_predict_h(const oemb200_matrix *x, const double *beta, int beta_rows, int nlambda, int type,
                       double *out, int64_t ldo, const oemb200_opts *opts, oemb200_stats *stats);
+int oemb200_xval_logistic_dense_h(const oemb200_matrix *x, const double *y, const oemb200_spec *spec, int nfolds,
+                                  const int *foldid, const char *type_measure, const oemb200_opts *opts,
+                                  oemb200_result *res);
 
 /* ------------------------------------------------------------------------------------------
  * Phase-level entries (device pointers only) used by bench.py for the roofline numbers and by
@@ -299,6 +313,18 @@ int oemb200_xb_logistic(const double *x_dev, int64_t n, int p, int64_t ldx, cons
 int oemb200_logit_slab_pass(const double *x_dev, int64_t n, int p, int64_t ldx, const double *b_dev, double b0,
                             const double *y_dev, double *prob_dev, double *w_dev, double *grad_dev, int reps,
                             void *stream, double *ms_out, double *ms_relayout_out);
+
+/* The fused data pass of oemb200_xval_logistic_dense for M models: model g uses the rows i with fold_dev[i] not 0 and
+ * not g (model 0: every row with a non-zero fold), grad_dev row g (M x (p + 1), row-major) = [sum r, X' r] over its rows
+ * with r_i = y_i - 1/(1 + exp(-(b0_dev[g] + x_i . b_dev[g]))); b_dev is M x p row-major, b0_dev M values.  conv_dev (M
+ * ints, may be NULL): models with a non-zero flag are skipped and their grad rows left untouched.  A 4-row slab copy of
+ * x is built inside the call (*ms_relayout_out); the pass (ceil(M / models-per-sweep) sweeps) runs `reps` times and
+ * *ms_out is the average of one pass; *sweeps_out (may be NULL) = sweeps per pass.  OEMB200_EUNSUPPORTED for p
+ * outside 8..2048. */
+int oemb200_logit_fold_pass(const double *x_dev, int64_t n, int p, int64_t ldx, const double *b_dev,
+                            const double *b0_dev, const double *y_dev, const int *fold_dev, int M, const int *conv_dev,
+                            double *grad_dev, int reps, void *stream, double *ms_out, double *ms_relayout_out,
+                            int *sweeps_out);
 
 /* Largest eigenvalue of the symmetric q x q matrix (device, col-major) by on-device Lanczos.
  * Stands in for Spectra::SymEigsSolver at src/oem_dense.h:485-498. */

@@ -102,6 +102,10 @@ def load():
     L.oemb200_fit_logistic_dense.argtypes = [vp, i64, ci, i64, vp, sp, op, rp]
     L.oemb200_xtx.argtypes = [vp, vp, ci, sp, vp, ci, op, rp]
     L.oemb200_xval_dense.argtypes = [vp, i64, ci, i64, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
+    L.oemb200_xval_logistic_dense.argtypes = [vp, i64, ci, i64, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
+    L.oemb200_xval_logistic_dense_h.argtypes = [vp, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
+    L.oemb200_logit_fold_pass.argtypes = [vp, i64, ci, i64, vp, vp, vp, vp, ci, vp, vp, ci, vp, ctypes.POINTER(dbl),
+                                          ctypes.POINTER(dbl), ctypes.POINTER(ci)]
     L.oemb200_gram.argtypes = [vp, i64, ci, i64, vp, vp, vp, vp, ctypes.POINTER(dbl)]
     L.oemb200_colstats.argtypes = [vp, i64, ci, i64, vp, vp, vp, vp, ctypes.POINTER(dbl)]
     L.oemb200_xb_logistic.argtypes = [vp, i64, ci, i64, vp, dbl, vp, vp, vp, vp, vp, ctypes.POINTER(dbl)]
@@ -141,7 +145,8 @@ EXPORTS = ["oemb200_last_error", "oemb200_version", "oemb200_device_count", "oem
            "oemb200_matrix_create", "oemb200_matrix_create_from_file", "oemb200_matrix_destroy", "oemb200_matrix_info",
            "oemb200_fit_dense_h", "oemb200_fit_big_h", "oemb200_fit_logistic_dense_h", "oemb200_xval_dense_h",
            "oemb200_predict_h", "oemb200_comm_unique_id", "oemb200_comm_create", "oemb200_comm_from_nccl", "oemb200_comm_destroy",
-           "oemb200_comm_allreduce", "oemb200_comm_p2p_enabled"]
+           "oemb200_comm_allreduce", "oemb200_comm_p2p_enabled", "oemb200_xval_logistic_dense",
+           "oemb200_xval_logistic_dense_h", "oemb200_logit_fold_pass"]
 
 
 def lambda_grid(lmax, nlambda, lmin_ratio):
@@ -372,7 +377,7 @@ def _run_xy(fn_name, x, y, family, penalty, weights, groups, unique_groups, grou
                       lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept, compute_loss)
     o = opts if isinstance(opts, Opts) else make_opts(opts, comm)
     Lmax = L.oemb200_nlambda_max(ctypes.byref(spec))
-    out = _Out(len(penalty), Lmax, p + 1, xval=fn_name.startswith("oemb200_xval_dense"))
+    out = _Out(len(penalty), Lmax, p + 1, xval=fn_name.startswith(("oemb200_xval_dense", "oemb200_xval_logistic_dense")))
     fn = getattr(L, fn_name)
     if extra is None:
         rc = fn(*xargs, yp, ctypes.byref(spec), ctypes.byref(o), ctypes.byref(out.res))
@@ -477,6 +482,40 @@ def oem_xval_dense(x, y, family, penalty, weights, groups, unique_groups, group_
     return _run_xy("oemb200_xval_dense", x, y, family, penalty, weights, groups, unique_groups, group_weights,
                    lambda_, nlambda, lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept,
                    compute_loss, opts, comm, extra=extra)
+
+
+def oem_xval_logistic_dense(x, y, family, penalty, weights, groups, unique_groups, group_weights, lambda_, nlambda,
+                            lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept, nfolds, foldid,
+                            compute_loss, type_measure, opts, comm=None):
+    """Binomial cross-validation (include/oem_b200.h: oemb200_xval_logistic_dense): the full-data logistic fit plus
+    nfolds leave-fold-out fits at its lambdas, all IRLS passes fused; type_measure deviance | class | mse | mae."""
+    def extra(keep):
+        f = keep.arr(foldid, np.int32)
+        return [int(nfolds), f.ctypes.data, type_measure.encode()]
+    return _run_xy("oemb200_xval_logistic_dense", x, y, family, penalty, weights, groups, unique_groups, group_weights,
+                   lambda_, nlambda, lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept,
+                   compute_loss, opts, comm, extra=extra)
+
+
+def logit_fold_pass(x, B, b0, y, fold, conv=None, reps=1, stream=None):
+    """Phase-level fused data pass of the binomial xval (oemb200_logit_fold_pass) on CUDA tensors: x (n x p,
+    column-major float64), B (M x p), b0 (M), y (n), fold (n, int32; 0 = no model), conv (M, int32, optional).
+    Returns (grad M x (p + 1), ms per pass, ms of the slab re-layout, sweeps per pass)."""
+    import torch
+    keep = _Keep()
+    xp, n, p, ld = _matrix_arg(x, keep)
+    M = int(B.shape[0])
+    for name, t, dt in (("B", B, torch.float64), ("b0", b0, torch.float64), ("y", y, torch.float64), ("fold", fold, torch.int32)):
+        if not _is_torch_cuda(t) or t.dtype != dt or not t.is_contiguous():
+            raise ValueError(f"{name} must be a contiguous CUDA tensor of {dt}")
+    if conv is not None and (not _is_torch_cuda(conv) or conv.dtype != torch.int32):
+        raise ValueError("conv must be a CUDA int32 tensor")
+    grad = torch.full((M, p + 1), float("nan"), dtype=torch.float64, device=B.device)
+    ms, msr, sw = ctypes.c_double(), ctypes.c_double(), ctypes.c_int()
+    _check(load().oemb200_logit_fold_pass(xp, n, p, ld, B.data_ptr(), b0.data_ptr(), y.data_ptr(), fold.data_ptr(), M,
+                                          conv.data_ptr() if conv is not None else None, grad.data_ptr(), int(reps),
+                                          stream, ctypes.byref(ms), ctypes.byref(msr), ctypes.byref(sw)))
+    return grad, ms.value, msr.value, sw.value
 
 
 def oem_xtx(xtx, xty, family, penalty, groups, unique_groups, group_weights, lambda_, nlambda, lmin_ratio,

@@ -9,7 +9,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "liboem_b200.so")
 SOURCES = ["runtime.cu", "gram_syrk.cu", "colstats.cu", "assemble.cu", "path_kernel.cu", "host_common.cu",
-           "entries.cu", "entry_logistic.cu", "entry_xval.cu", "entry_sparse.cu", "cvscore.cu", "logit_slab.cu", "comm.cu", "ingest.cu"]
+           "entries.cu", "entry_logistic.cu", "entry_xval.cu", "entry_xval_logistic.cu", "entry_sparse.cu", "cvscore.cu", "logit_slab.cu", "comm.cu", "ingest.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]
 

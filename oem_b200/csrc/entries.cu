@@ -501,6 +501,8 @@ void predict_sparse_entry(const int *row_idx, const int *col_ptr, const double *
                           int nrows, int L, int type, double *out, int64_t ldo, const oemb200_opts *o, oemb200_stats *stats);
 void fit_xval(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s, int nfolds,
               const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res);
+void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s, int nfolds,
+                       const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res);
 
 template <typename F>
 static int guarded(F &&f) {
@@ -644,6 +646,11 @@ int oemb200_xval_dense(const double *x, int64_t n, int p, int64_t ldx, const dou
                        int nfolds, const int *foldid, const char *type_measure, const oemb200_opts *opts,
                        oemb200_result *res) {
     return guarded([&] { fit_xval(x, n, p, ldx, y, spec, nfolds, foldid, type_measure, opts, res); });
+}
+int oemb200_xval_logistic_dense(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *spec,
+                                int nfolds, const int *foldid, const char *type_measure, const oemb200_opts *opts,
+                                oemb200_result *res) {
+    return guarded([&] { fit_xval_logistic(x, n, p, ldx, y, spec, nfolds, foldid, type_measure, opts, res); });
 }
 
 int oemb200_predict(const double *x, int64_t n, int p, int64_t ldx, const double *beta, int beta_rows, int nlambda, int type,
@@ -832,6 +839,14 @@ int oemb200_xval_dense_h(const oemb200_matrix *x, const double *y, const oemb200
         fit_xval(x->dev, x->n, x->p, x->ld, y, spec, nfolds, foldid, type_measure, &h.o, res);
     });
 }
+int oemb200_xval_logistic_dense_h(const oemb200_matrix *x, const double *y, const oemb200_spec *spec, int nfolds,
+                                  const int *foldid, const char *type_measure, const oemb200_opts *opts, oemb200_result *res) {
+    return guarded([&] {
+        check_handle(x);
+        HandleOpts h(x, opts);
+        fit_xval_logistic(x->dev, x->n, x->p, x->ld, y, spec, nfolds, foldid, type_measure, &h.o, res);
+    });
+}
 int oemb200_predict_h(const oemb200_matrix *x, const double *beta, int beta_rows, int nlambda, int type, double *out,
                       int64_t ldo, const oemb200_opts *opts, oemb200_stats *stats) {
     return guarded([&] {
@@ -901,6 +916,33 @@ int oemb200_logit_slab_pass(const double *x_dev, int64_t n, int p, int64_t ldx, 
         cx.sync();
         if (ms_relayout_out) *ms_relayout_out = elapsed_ms(e0, e1);
         if (ms_out) *ms_out = elapsed_ms(e1, e2) / nrep;
+        cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(e2);
+    });
+}
+int oemb200_logit_fold_pass(const double *x_dev, int64_t n, int p, int64_t ldx, const double *b_dev, const double *b0_dev,
+                            const double *y_dev, const int *fold_dev, int M, const int *conv_dev, double *grad_dev, int reps,
+                            void *stream, double *ms_out, double *ms_relayout_out, int *sweeps_out) {
+    return guarded([&] {
+        if (!x_dev || !b_dev || !b0_dev || !y_dev || !fold_dev || !grad_dev || n < 1 || p < 1 || ldx < n || M < 1)
+            fail(OEMB200_EINVAL, "logit_fold_pass: bad arguments");
+        if (!logit_fold_models(p)) fail(OEMB200_EUNSUPPORTED, "the fused fold pass covers 8 <= p <= 2048 (p = %d)", p);
+        oemb200_opts o_; phase_ctx_opts(o_, stream);
+        Ctx cx(&o_);
+        cudaEvent_t e0, e1, e2;
+        OEM_CUDA(cudaEventCreate(&e0)); OEM_CUDA(cudaEventCreate(&e1)); OEM_CUDA(cudaEventCreate(&e2));
+        DBuf<double> slabs(logit_fold_doubles(n, p));
+        OEM_CUDA(cudaEventRecord(e0, cx.stream));
+        logit_fold_relayout(cx, x_dev, n, p, ldx, slabs.p);
+        OEM_CUDA(cudaEventRecord(e1, cx.stream));
+        const int nrep = reps < 1 ? 1 : reps;
+        int sweeps = 0;
+        for (int r = 0; r < nrep; ++r)
+            sweeps = logit_fold_launch(cx, slabs.p, n, p, b_dev, b0_dev, y_dev, fold_dev, M, conv_dev, nullptr, nullptr, grad_dev);
+        OEM_CUDA(cudaEventRecord(e2, cx.stream));
+        cx.sync();
+        if (ms_relayout_out) *ms_relayout_out = elapsed_ms(e0, e1);
+        if (ms_out) *ms_out = elapsed_ms(e1, e2) / nrep;
+        if (sweeps_out) *sweeps_out = sweeps;
         cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(e2);
     });
 }

@@ -54,6 +54,13 @@ __global__ void logistic_loss_kernel(const double *__restrict__ y, const double 
     }
 }
 
+void logistic_loss_launch(Ctx &cx, const double *y, const double *prob, int64_t n, double *partial, double *tot2) {
+    logistic_loss_kernel<<<1024, 256, 0, cx.stream>>>(y, prob, n, partial);
+    OEM_CUDA(cudaGetLastError());
+    cx.st.kernel_launches += 1;
+    vecsum_launch(cx, partial, 1024, 0.0, tot2, false);
+}
+
 // per-block min / max of v (partial[2 b], partial[2 b + 1]); the host folds the blocks
 __global__ void __launch_bounds__(256) minmax_kernel(const double *__restrict__ v, long long n, double *__restrict__ partial) {
     double lo = INFINITY, hi = -INFINITY;

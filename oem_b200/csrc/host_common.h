@@ -80,6 +80,24 @@ void sparse_gram_launch(Ctx &cx, const SparseDesign *sd, const double *roww, dou
 void sparse_xb_logistic_launch(Ctx &cx, const SparseDesign *sd, const double *b, const double *b0_dev, const double *y,
                                double *prob, double *resid, double *w);
 
+// ---- entry_xval.cu: steps 1-3 shared by the gaussian and the binomial xval drivers ----
+struct XvalSystems {
+    int F = 0, NG = 0;                       // folds, systems (0 = full data, k = without fold k)
+    std::vector<int64_t> cnt, off;           // rows per fold; fold k = sorted rows [off[k], off[k] + cnt[k]), padded to off[k + 1]
+    int64_t npad = 0;                        // rows of the fold-sorted copy
+    DBuf<double> Xs, ys, ws;                 // fold-sorted X (column-major, ld npad), y, weights (zero padding rows)
+    DBuf<double> XX, XY, cinv, nout;         // NG assembled systems (assemble_aug_launch)
+    std::vector<double> hXY, hcinv, hn;      // host: XY of system 0, cinv of every system, row count of every system
+};
+// weights may be NULL.  hess_scale scales the Grams, column sums and corners before assembly (the binomial driver's
+// upper-bound Hessian X'WX at beta = 0 has W = 1/4; a power of two, so the scaled sums are exact); 1 = no launch.
+void xval_build_systems(Ctx &cx, const double *x, int64_t n, int p, int64_t ldx, const double *y, const double *weights,
+                        int F, const int *foldid, int icpt, bool stdz, double hess_scale, XvalSystems &xs);
+
+// ---- entry_logistic.cu ----
+// tot[0] = get_loss() of prob (src/oem_logistic_dense.h:1057-1088) summed over n rows; partial: 1024 doubles of scratch
+void logistic_loss_launch(Ctx &cx, const double *y, const double *prob, int64_t n, double *partial, double *tot2);
+
 // row-slab copy of X kept across logistic fits (owned by an oemb200_matrix handle); `rt` = rows per slab it was built with
 struct SlabCache { double *slabs = nullptr; int rt = 0; };
 void finish_stats(Ctx &cx, PhaseTimers &tm, size_t total_id, oemb200_result *res);

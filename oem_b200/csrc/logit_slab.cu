@@ -323,4 +323,267 @@ void logit_slab_launch(Ctx &cx, const double *slabs, int64_t n, int p, const dou
     cx.st.data_passes += 1;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Fused multi-model pass of binomial cross-validation: ONE sweep of the slabs serves up to MK logistic models that share X
+// but not their rows.  Model g (g = m0 + m) uses the rows whose fold is neither 0 (padding) nor g, so model 0 is the
+// full-data fit and model k leaves fold k out; for each one the pass forms grad_g = [sum r, X' r] with
+// r_i = y_i - sigma(b0_g + x_i . b_g) on its rows and 0 elsewhere.
+//
+// Layout: one 512-thread CTA per SM, 4-row slabs in a 2-stage ring.  Thread t owns the columns j = t, t + 512, ... (NC of
+// them) for the whole pass, as in logit_slab_kernel, but the per-model state no longer fits in registers next to the slab:
+//   the MK coefficient vectors live in shared memory (MK x p, read conflict-free by consecutive columns),
+//   the MK x NC gradient accumulators stay in registers (at most 64 doubles per thread),
+//   eta of every (row, model) is a per-model multi-value butterfly + a fixed-order sum over the warps, as in the single pass.
+// Per slab and model the work is 2 NC RT FMAs per thread against one RT-value butterfly, so at p = 1000 and 11 models the
+// pass is bound by the FP64 pipe and the shuffles, not by HBM.  A model whose `conv` flag is set (its IRLS loop has
+// converged for this lambda) takes no part: no arithmetic, and its gradient row is left untouched.
+// ---------------------------------------------------------------------------------------------
+constexpr int LF_THREADS = 512, LF_RT = 4, LF_STAGES = 2;
+
+template <int NC, int MK>
+__global__ void __launch_bounds__(LF_THREADS, 1)
+logit_fold_kernel(const double *__restrict__ slabs, long long n, int p, size_t stage_stride, const double *__restrict__ B,
+                  const double *__restrict__ b0, int m0, int nm, const double *__restrict__ y, const int *__restrict__ fold,
+                  const int *__restrict__ conv, double *__restrict__ prob0, double *__restrict__ partial) {
+    constexpr int RT = LF_RT, WARPS = LF_THREADS / 32;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    double *stages = reinterpret_cast<double *>(smem_raw);
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw + LF_STAGES * stage_stride * 8);
+    uint64_t *empty = full + LF_STAGES;
+    double *bsm = reinterpret_cast<double *>(empty + LF_STAGES);          // [MK][p]
+    double *wsum = bsm + (size_t)MK * p;                                  // [WARPS][MK][RT]
+    double *rsm = wsum + WARPS * MK * RT;                                 // [MK][RT]
+    double *b0s = rsm + MK * RT;                                          // [MK]
+    __shared__ int act[MK];
+    __shared__ int nact;
+
+    const long long ntiles = (n + RT - 1) / RT;
+    const long long mine = ntiles > blockIdx.x ? (ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, t = threadIdx.x;
+    const uint32_t tile_bytes = (uint32_t)RT * (uint32_t)p * 8u;
+
+    if (t == 0) {
+        int c = 0;
+        for (int m = 0; m < MK; ++m) {
+            act[m] = m < nm && !(conv && conv[m0 + m]);
+            c += act[m];
+        }
+        nact = c;
+        for (int s = 0; s < LF_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], WARPS); }
+        mbar_fence_init();
+    }
+    for (int e = t; e < nm * p; e += LF_THREADS) bsm[e] = B[(size_t)m0 * p + e];
+    if (t < nm) b0s[t] = b0[m0 + t];
+    __syncthreads();
+    if (nact == 0) return;
+
+    uint64_t pol = 0;
+    const uint32_t pair_bytes = (uint32_t)p * 16u;
+    auto issue = [&](long long k) {
+        const int s = (int)(k % LF_STAGES);
+        const double *src = slabs + (size_t)(blockIdx.x + k * gridDim.x) * RT * p;
+        double *dst = stages + (size_t)s * stage_stride;
+        mbar_arrive_expect_tx(&full[s], tile_bytes);
+#pragma unroll
+        for (int kk = 0; kk < RT / 2; ++kk)
+            bulk_load(dst + (size_t)kk * 2 * p, src + (size_t)kk * 2 * p, pair_bytes, &full[s], pol);
+    };
+    if (t == 0) {
+        asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+        for (long long k = 0; k < LF_STAGES && k < mine; ++k) issue(k);
+    }
+
+    double gacc[MK][NC];
+#pragma unroll
+    for (int m = 0; m < MK; ++m)
+#pragma unroll
+        for (int c = 0; c < NC; ++c) gacc[m][c] = 0.0;
+    double rsum = 0.0;                       // threads t < MK: sum r of model t
+
+    for (long long k = 0; k < mine; ++k) {
+        const int s = (int)(k % LF_STAGES);
+        const uint32_t ph = (uint32_t)((k / LF_STAGES) & 1);
+        mbar_wait(&full[s], ph);
+        const double2 *tile = reinterpret_cast<const double2 *>(stages + (size_t)s * stage_stride);
+        double x[NC][RT];
+#pragma unroll
+        for (int c = 0; c < NC; ++c) {
+            const int j = t + c * LF_THREADS;
+#pragma unroll
+            for (int kk = 0; kk < RT / 2; ++kk) {
+                const double2 v = j < p ? tile[(size_t)kk * p + j] : make_double2(0.0, 0.0);
+                x[c][2 * kk] = v.x; x[c][2 * kk + 1] = v.y;
+            }
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty[s]);
+        if (t == 0 && k + LF_STAGES < mine) {
+            mbar_wait(&empty[s], ph);
+            issue(k + LF_STAGES);
+        }
+
+#pragma unroll
+        for (int m = 0; m < MK; ++m) {
+            if (!act[m]) continue;
+            double acc[RT];
+#pragma unroll
+            for (int i = 0; i < RT; ++i) acc[i] = 0.0;
+#pragma unroll
+            for (int c = 0; c < NC; ++c) {
+                const int j = t + c * LF_THREADS;
+                const double bj = j < p ? bsm[(size_t)m * p + j] : 0.0;
+#pragma unroll
+                for (int i = 0; i < RT; ++i) acc[i] = fma(x[c][i], bj, acc[i]);
+            }
+            // RT = 4 row sums over the 32 lanes: two halving steps, then three full steps; lane l ends with row l >> 3
+            {
+                const bool up16 = (lane & 16) != 0;
+                acc[0] = (up16 ? acc[2] : acc[0]) + __shfl_xor_sync(0xffffffffu, up16 ? acc[0] : acc[2], 16);
+                acc[1] = (up16 ? acc[3] : acc[1]) + __shfl_xor_sync(0xffffffffu, up16 ? acc[1] : acc[3], 16);
+                const bool up8 = (lane & 8) != 0;
+                acc[0] = (up8 ? acc[1] : acc[0]) + __shfl_xor_sync(0xffffffffu, up8 ? acc[0] : acc[1], 8);
+                acc[0] += __shfl_xor_sync(0xffffffffu, acc[0], 4);
+                acc[0] += __shfl_xor_sync(0xffffffffu, acc[0], 2);
+                acc[0] += __shfl_xor_sync(0xffffffffu, acc[0], 1);
+            }
+            if ((lane & 7) == 0) wsum[(warp * MK + m) * RT + (lane >> 3)] = acc[0];
+        }
+        __syncthreads();
+        const long long row0 = (blockIdx.x + k * gridDim.x) * RT;
+        if (t < MK * RT) {
+            const int m = t / RT, i = t - m * RT;
+            if (act[m]) {
+                double e = b0s[m];
+#pragma unroll
+                for (int w = 0; w < WARPS; ++w) e += wsum[(w * MK + m) * RT + i];
+                const long long row = row0 + i;
+                double r = 0.0;
+                if (row < n) {
+                    const int f = fold[row];
+                    if (f != 0 && f != m0 + m) {
+                        const double pr = 1.0 / (1.0 + exp(-e));
+                        r = y[row] - pr;
+                        if (prob0 && m0 + m == 0) prob0[row] = pr;
+                    }
+                }
+                rsm[m * RT + i] = r;
+            }
+        }
+        __syncthreads();
+#pragma unroll
+        for (int m = 0; m < MK; ++m) {
+            if (!act[m]) continue;
+            double r[RT];
+#pragma unroll
+            for (int i = 0; i < RT; ++i) r[i] = rsm[m * RT + i];
+#pragma unroll
+            for (int c = 0; c < NC; ++c) {
+                double tt = x[c][0] * r[0];
+#pragma unroll
+                for (int i = 1; i < RT; ++i) tt = fma(x[c][i], r[i], tt);
+                gacc[m][c] += tt;
+            }
+        }
+        if (t < MK && act[t]) {
+            double tt = rsm[t * RT];
+#pragma unroll
+            for (int i = 1; i < RT; ++i) tt += rsm[t * RT + i];
+            rsum += tt;
+        }
+    }
+    double *out = partial + (size_t)blockIdx.x * MK * (p + 1);
+#pragma unroll
+    for (int m = 0; m < MK; ++m) {
+        if (!act[m]) continue;
+#pragma unroll
+        for (int c = 0; c < NC; ++c) {
+            const int j = t + c * LF_THREADS;
+            if (j < p) out[(size_t)m * (p + 1) + 1 + j] = gacc[m][c];
+        }
+    }
+    if (t < MK && act[t]) out[(size_t)t * (p + 1)] = rsum;
+}
+
+// out[(m0 + m) (p + 1) + e] = sum over the CTAs of partial[c][m][e], in CTA order (same order as ls_sum_partials_kernel);
+// rows of converged models are left untouched
+__global__ void __launch_bounds__(256) lf_sum_partials_kernel(const double *__restrict__ partial, int nparts, int mk, int p,
+                                                              int m0, int nm, const int *__restrict__ conv, double *__restrict__ out) {
+    __shared__ double sm[8][33];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int width = nm * (p + 1);
+    const int k = blockIdx.x * 32 + tx;
+    const int m = k / (p + 1);
+    const bool live = k < width && !(conv && conv[m0 + m]);
+    double s = 0.0;
+    if (live)
+        for (int c = ty; c < nparts; c += 8) s += partial[(size_t)c * mk * (p + 1) + k];
+    sm[ty][tx] = s;
+    __syncthreads();
+    if (ty == 0 && live) {
+        double t = sm[0][tx];
+#pragma unroll
+        for (int r = 1; r < 8; ++r) t += sm[r][tx];
+        out[(size_t)m0 * (p + 1) + k] = t;
+    }
+}
+
+// Models per sweep for a given p: the MK x NC accumulators must stay within 64 doubles per thread (128 registers is the
+// ceiling of a 512-thread CTA) and MK coefficient vectors must fit next to the 2-stage ring in shared memory.
+static int logit_fold_nc(int p) { return (p + LF_THREADS - 1) / LF_THREADS; }
+int logit_fold_models(int p) {
+    if (p < 8 || p > 2048) return 0;
+    static const int mk[4] = {16, 16, 8, 4};
+    return mk[logit_fold_nc(p) - 1];
+}
+
+size_t logit_fold_doubles(int64_t n, int p) { return (size_t)((n + LF_RT - 1) / LF_RT) * LF_RT * p; }
+
+void logit_fold_relayout(Ctx &cx, const double *X, int64_t n, int p, int64_t ld, double *slabs) {
+    if (!logit_fold_models(p)) fail(OEMB200_EINVAL, "fused fold pass does not apply to p = %d", p);
+    if (n >= (1ll << 31) * RL_ROWS) fail(OEMB200_EUNSUPPORTED, "slab re-layout: too many rows");
+    dim3 grid((unsigned)((n + RL_ROWS - 1) / RL_ROWS), (unsigned)((p + RL_COLS - 1) / RL_COLS));
+    slab_relayout_kernel<<<grid, 256, 0, cx.stream>>>(X, n, p, ld, LF_RT, slabs);
+    OEM_CUDA(cudaGetLastError());
+    cx.st.kernel_launches += 1;
+}
+
+int logit_fold_launch(Ctx &cx, const double *slabs, int64_t n, int p, const double *B, const double *b0, const double *y,
+                      const int *fold, int M, const int *conv, const std::vector<char> *active, double *prob0, double *grad) {
+    const int MK = logit_fold_models(p), NC = logit_fold_nc(p);
+    if (!MK) fail(OEMB200_EINVAL, "fused fold pass does not apply to p = %d", p);
+    void *kern = nullptr;
+    if (NC == 1) kern = (void *)logit_fold_kernel<1, 16>;
+    else if (NC == 2) kern = (void *)logit_fold_kernel<2, 16>;
+    else if (NC == 3) kern = (void *)logit_fold_kernel<3, 8>;
+    else kern = (void *)logit_fold_kernel<4, 4>;
+    const size_t stage_stride = ((size_t)LF_RT * p + 15) / 16 * 16;
+    const size_t smem = LF_STAGES * stage_stride * 8 + 2 * LF_STAGES * 8 +
+                        ((size_t)MK * p + (size_t)(LF_THREADS / 32) * MK * LF_RT + (size_t)MK * LF_RT + MK) * 8;
+    if (smem > cx.smem_optin) fail(OEMB200_EUNSUPPORTED, "fused fold pass: %zu bytes of shared memory for p = %d", smem, p);
+    OEM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t ntiles = (n + LF_RT - 1) / LF_RT;
+    const int grid = (int)std::min<int64_t>(ntiles, (int64_t)cx.num_sms);
+    DBuf<double> partial((size_t)grid * MK * (p + 1));
+    long long nn = n;
+    int sweeps = 0;
+    for (int m0 = 0; m0 < M; m0 += MK) {
+        int nm = std::min(MK, M - m0);
+        if (active) {
+            bool any = false;
+            for (int m = m0; m < m0 + nm; ++m) any = any || (*active)[m];
+            if (!any) continue;
+        }
+        void *args[] = {(void *)&slabs, &nn, &p, (void *)&stage_stride, (void *)&B, (void *)&b0, &m0, &nm, (void *)&y,
+                        (void *)&fold, (void *)&conv, &prob0, &partial.p};
+        OEM_CUDA(cudaLaunchKernel(kern, dim3(grid), dim3(LF_THREADS), args, smem, cx.stream));
+        lf_sum_partials_kernel<<<(nm * (p + 1) + 31) / 32, 256, 0, cx.stream>>>(partial.p, grid, MK, p, m0, nm, conv, grad);
+        OEM_CUDA(cudaGetLastError());
+        cx.st.kernel_launches += 2;
+        cx.st.xb_launches += 1;
+        cx.st.data_passes += 1;
+        ++sweeps;
+    }
+    return sweeps;
+}
+
 }  // namespace oemb200

@@ -282,6 +282,16 @@ void logit_slab_relayout(Ctx &cx, const double *X, int64_t n, int p, int64_t ld,
 void logit_slab_launch(Ctx &cx, const double *slabs, int64_t n, int p, const double *b, const double *b0_dev,
                        const double *y, double *prob, double *w, double *grad_out, const int *skip = nullptr,
                        unsigned long long *t_clock = nullptr);   // t_clock (device, 2 words): [0] += ns of the pass, [1] scratch
+// Fused pass of M logistic models over one 4-row slab copy (logit_fold_relayout): model g uses the rows whose fold[i] is
+// neither 0 nor g; grad (M x (p + 1)): row g = [sum r, X' r] of model g.  B: M x p, b0: M (device).  conv (device, M ints,
+// may be NULL) / active (host, may be NULL): converged models are skipped and their grad rows left untouched; a group of
+// models with no active member costs no launch.  prob0 (may be NULL): sigma(eta) of model 0 on its rows.  Returns the
+// number of sweeps over X (ceil(M / logit_fold_models(p)) when every group is active).
+int logit_fold_models(int p);                     // models per sweep (0: 8 <= p <= 2048 does not hold)
+size_t logit_fold_doubles(int64_t n, int p);
+void logit_fold_relayout(Ctx &cx, const double *X, int64_t n, int p, int64_t ld, double *slabs);
+int logit_fold_launch(Ctx &cx, const double *slabs, int64_t n, int p, const double *B, const double *b0, const double *y,
+                      const int *fold, int M, const int *conv, const std::vector<char> *active, double *prob0, double *grad);
 
 // ---------------- cvscore.cu ----------------
 // order[i]: for every tile of fold_gather_tile_rows() source rows, the tile-local row indices grouped by fold
@@ -298,6 +308,11 @@ int cv_ncld(int nc);     // leading dimension (columns) of the coefficient matri
 void cvscore_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys,
                     const double *ws, int nfolds, const std::vector<std::array<int64_t, 3>> &segs, const double *B,
                     const double *b0, int nc, bool mae, double *out3);
+// the same moments of cv.oem's binomial measures (R/cv_oem.R:288-330) on p = 1 / (1 + exp(-(x . b + b0))), unweighted:
+// measure 0 = deviance (p clamped to [1e-5, 1 - 1e-5]), 1 = class error (p > 0.5) != y, 2 = 2 (y - p)^2, 3 = 2 |y - p|
+void cvscore_binomial_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys, int nfolds,
+                             const std::vector<std::array<int64_t, 3>> &segs, const double *B, const double *b0, int nc,
+                             int measure, double *out3);
 // B / b0 operands of cvscore_launch built on the device from the path kernel's raw iterates (chains (k+1) * P + pp)
 void cv_build_coef_launch(Ctx &cx, const double *beta_raw, const double *cinv, int nfolds, int P, int L, int p, int q, int icpt,
                           bool standardize, const int *nlam_run_dev, double *B, double *b0);

@@ -242,14 +242,33 @@ def oem_xtx(xtx, xty, family="gaussian", penalty=None, lambda_=(), nlambda=100, 
     return out
 
 
-def xval_oem(x, y, nfolds=10, foldid=None, type_measure="mse", ncores=-1, family="gaussian", penalty=None, weights=(),
+def xval_oem(x, y, nfolds=10, foldid=None, type_measure=None, ncores=-1, family="gaussian", penalty=None, weights=(),
              lambda_=(), nlambda=100, lambda_min_ratio=None, alpha=1.0, gamma=3.0, tau=0.5, groups=(),
              penalty_factor=None, group_weights=None, standardize=True, intercept=True, maxit=500, tol=1e-7,
-             irls_maxit=100, irls_tol=1e-3, compute_loss=False, varnames=None, seed=None, comm=None):
-    """R/oem_xval.R:107-460: fit + fast cross-validation in one call; adds lambda.min / lambda.1se / cvup / cvlo."""
-    if family != "gaussian":
-        raise NotImplementedError("binomial models not yet supported for xval, use cv.oem() instead")   # R/oem_xval.R:160-163
-    if type_measure not in ("mse", "deviance", "mae"):
+             irls_maxit=100, irls_tol=1e-3, compute_loss=False, varnames=None, seed=None, comm=None,
+             hessian_type="upper.bound"):
+    """R/oem_xval.R:107-460: fit + fast cross-validation in one call; adds lambda.min / lambda.1se / cvup / cvlo.
+    type.measure: gaussian mse (default) | deviance | mae; binomial deviance (default) | class | mse | mae.
+    family = "binomial" (which the reference's xval.oem refuses, R/oem_xval.R:160-163) runs oem_xval_logistic_dense:
+    the full-data logistic fit of oem() plus one fit per fold at its lambdas, scored with cv.oem's binomial measures
+    over all rows; `auc` needs per-fold ranks and stays with cv_oem()."""
+    if family not in ("gaussian", "binomial"):
+        raise ValueError("'arg' should be one of 'gaussian', 'binomial'")
+    binomial = family == "binomial"
+    if type_measure is None:
+        type_measure = "deviance" if binomial else "mse"
+    if binomial:
+        if type_measure == "auc":
+            raise ValueError("type.measure = 'auc' needs per-fold ranks: use cv_oem(family='binomial', type_measure='auc')")
+        if type_measure not in ("deviance", "class", "mse", "mae"):
+            raise ValueError("type.measure must be 'deviance', 'class', 'mse' or 'mae' for the binomial family")
+        if hessian_type != "upper.bound":
+            raise ValueError("xval_oem(family='binomial') supports hessian_type='upper.bound' only; use cv_oem for 'full'")
+        if len(weights) > 0:
+            raise ValueError("weights not implemented yet.")                       # oem() itself rejects them (R/oem.R:244)
+        if not hasattr(y, "is_cuda") and np.unique(np.asarray(y)).size > 2:
+            raise ValueError("y must be a binary outcome")
+    elif type_measure not in ("mse", "deviance", "mae"):
         raise ValueError("type.measure must be 'mse', 'deviance' or 'mae' for the gaussian family")
     penalty = _match_penalty(penalty)
     n, p = _shape(x)
@@ -269,9 +288,14 @@ def xval_oem(x, y, nfolds=10, foldid=None, type_measure="mse", ncores=-1, family
     g, ug, gw = _groups(penalty, groups, group_weights, p, explicit_intercept=bool(intercept))
     lam = _lambda_list(lambda_, len(penalty))
     opts = dict(maxit=int(maxit), tol=float(tol), irls_maxit=int(irls_maxit), irls_tol=float(irls_tol), ncores=int(ncores))
-    res = api.oem_xval_dense(x, y, family, penalty, weights, g, ug, gw, lam, int(nlambda), lmr, float(alpha), gamma, float(tau), pf,
-                             bool(standardize), bool(intercept), int(nfolds), foldid.astype(np.int32), bool(compute_loss),
-                             "mse" if type_measure == "deviance" else type_measure, opts, comm=comm)
+    if binomial:
+        res = api.oem_xval_logistic_dense(x, y, family, penalty, [], g, ug, gw, lam, int(nlambda), lmr, float(alpha), gamma,
+                                          float(tau), pf, bool(standardize), bool(intercept), int(nfolds),
+                                          foldid.astype(np.int32), bool(compute_loss), type_measure, opts, comm=comm)
+    else:
+        res = api.oem_xval_dense(x, y, family, penalty, weights, g, ug, gw, lam, int(nlambda), lmr, float(alpha), gamma,
+                                 float(tau), pf, bool(standardize), bool(intercept), int(nfolds), foldid.astype(np.int32),
+                                 bool(compute_loss), "mse" if type_measure == "deviance" else type_measure, opts, comm=comm)
     out = _decorate(res, penalty, n, p, family, varnames)
     out.update(getmin(out["lambda"], out["cvm"], out["cvsd"]))
     out["cvup"] = [m + s for m, s in zip(out["cvm"], out["cvsd"])]

@@ -198,24 +198,17 @@ static void fit_big(const double *x, int64_t n, int p, int64_t ldx, const double
     for (int j = 0; j < q; ++j) lmax = std::max(lmax, std::fabs(hXY[j]));
     su.build_lambdas(s, lmax, false);
 
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
+    PenaltyTables tb(cx, su, s, p, icpt);
     PathBuffers pb;
     const size_t t_p = tm.start(&cx.st.ms_path);
-    run_paths(cx, su, o, q, 1, XX.p, XY.p, pf, 1.0, 1.005, false, nullptr, pb);
+    run_paths(cx, su, tb, o, 1, XX.p, XY.p, 1.005, false, nullptr, pb);
     tm.stop(t_p);
 
     const int L = su.Lmax;
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)su.P * (p + 1) * L);
+    write_beta(su, pb.h_beta.data(), p, icpt, s->standardize ? hcinv.data() : nullptr, res);
     for (int pp = 0; pp < su.P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &pb.h_beta[((size_t)pp * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = s->standardize ? raw[icpt + j] * hcinv[j] : raw[icpt + j];
-            res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)pp * L + i];
-        }
+        for (int i = 0; i < su.nlam_run[pp]; ++i) res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)pp * L + i];
     *res->d = pb.h_d[0];
     finish_stats(cx, tm, t_total, res);
 }
@@ -341,10 +334,10 @@ static void fit_dense(const double *x, int64_t n, int p, int64_t ldx, const doub
     for (int j = 0; j < p; ++j) lmax = std::max(lmax, std::fabs(hXY[j]));
     lmax *= scaleY;                                   // src/oem_dense.cpp:176
     su.build_lambdas(s, lmax, false);
-    std::vector<double> pf(s->penalty_factor, s->penalty_factor + p);
+    PenaltyTables tb(cx, su, s, p, 0, scaleY);
     PathBuffers pb;
     const size_t t_p = tm.start(&cx.st.ms_path);
-    run_paths(cx, su, o, p, 1, XX.p, XY.p, pf, scaleY, 1.005, o->accelerate != 0, nullptr, pb);
+    run_paths(cx, su, tb, o, 1, XX.p, XY.p, 1.005, o->accelerate != 0, nullptr, pb);
     tm.stop(t_p);
 
     // ---- recover (DataStd.h:269-293) ----
@@ -474,10 +467,10 @@ static void fit_xtx(const double *xtx, const double *xty, int p, const oemb200_s
     double lmax = 0.0;
     for (int j = 0; j < p; ++j) lmax = std::max(lmax, std::fabs(hXY[j]));
     su.build_lambdas(s, lmax, false);
-    std::vector<double> pf(s->penalty_factor, s->penalty_factor + p);
+    PenaltyTables tb(cx, su, s, p, 0);
     PathBuffers pb;
     const size_t t_p = tm.start(&cx.st.ms_path);
-    run_paths(cx, su, o, p, 1, XX.p, XY.p, pf, 1.0, 1.005, false, n_sf ? sinv.p : nullptr, pb);
+    run_paths(cx, su, tb, o, 1, XX.p, XY.p, 1.005, false, n_sf ? sinv.p : nullptr, pb);
     tm.stop(t_p);
     const int L = su.Lmax;
     fill_common_outputs(su, res);

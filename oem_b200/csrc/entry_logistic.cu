@@ -54,11 +54,17 @@ __global__ void logistic_loss_kernel(const double *__restrict__ y, const double 
     }
 }
 
-void logistic_loss_launch(Ctx &cx, const double *y, const double *prob, int64_t n, double *partial, double *tot2) {
-    logistic_loss_kernel<<<1024, 256, 0, cx.stream>>>(y, prob, n, partial);
+double logistic_loss(Ctx &cx, const double *y, const double *prob, int64_t n) {
+    DBuf<double> buf(1024 + 2);        // per-block partial sums, then their [sum, sum of squares]
+    logistic_loss_kernel<<<1024, 256, 0, cx.stream>>>(y, prob, n, buf.p);
     OEM_CUDA(cudaGetLastError());
     cx.st.kernel_launches += 1;
-    vecsum_launch(cx, partial, 1024, 0.0, tot2, false);
+    vecsum_launch(cx, buf.p, 1024, 0.0, buf.p + 1024, false);
+    cx.all_reduce(buf.p + 1024, 2);
+    double h[2];
+    OEM_CUDA(cudaMemcpyAsync(h, buf.p + 1024, sizeof h, cudaMemcpyDeviceToHost, cx.stream));
+    cx.sync();
+    return h[0];
 }
 
 // per-block min / max of v (partial[2 b], partial[2 b + 1]); the host folds the blocks
@@ -150,16 +156,18 @@ struct WallMarks {
                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
     }
 };
-struct PinnedFlag {          // four verdict slots: the host reads slot (iteration & 3) after that iteration's event
-    int *p = nullptr;
-    PinnedFlag() { OEM_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&p), 64, cudaHostAllocMapped)); memset(p, 0, 64); }
-    ~PinnedFlag() { if (p) cudaFreeHost(p); }
-};
-struct ScratchHolder {
-    PathScratch *s;
-    ScratchHolder() : s(path_scratch_create()) {}
-    ~ScratchHolder() { path_scratch_destroy(s); }
-};
+// 1 / sd of every column from its sum of squares h0[2p + j] (uncentred, divisor n - 1, a zero column keeps scale 1);
+// ones when the fit is not standardised
+std::vector<double> logistic_cinv(const std::vector<double> &h0, int p, double n_tot, bool stdz) {
+    std::vector<double> cinv(p, 1.0);
+    if (stdz)
+        for (int j = 0; j < p; ++j) {
+            double sq = h0[2 * (size_t)p + j] / (n_tot - 1.0);
+            if (sq == 0.0) sq = 1.0;
+            cinv[j] = 1.0 / std::sqrt(sq);
+        }
+    return cinv;
+}
 }  // namespace
 
 void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s,
@@ -206,13 +214,7 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
     if (!(n_tot > q)) fail(OEMB200_EUNSUPPORTED, "oem_fit_logistic_dense with n <= p + intercept: the reference takes least-squares steps on the 0/1 "
                                           "response there, with a step matrix its d does not bound (src/oem_logistic_dense.h:478-483, 530-568; "
                                           "restated in oracle/oracle.py:_logistic_wide, which diverges) -- not built");
-    std::vector<double> cinv(p, 1.0);
-    if (stdz)
-        for (int j = 0; j < p; ++j) {
-            double sq = h0[2 * (size_t)p + j] / (n_tot - 1.0);
-            if (sq == 0.0) sq = 1.0;
-            cinv[j] = 1.0 / std::sqrt(sq);
-        }
+    const std::vector<double> cinv = logistic_cinv(h0, p, n_tot, stdz);
     std::vector<double> XY0(q, 0.0);
     if (icpt) XY0[0] = h0[3 * (size_t)p];
     for (int j = 0; j < p; ++j) XY0[icpt + j] = stdz ? h0[(size_t)p + j] * cinv[j] : h0[(size_t)p + j];
@@ -255,11 +257,10 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
     }
 
     // ---- device state ----
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
     const int L = su.Lmax;
-    DBuf<double> d_pf(q), d_cinv(p), d_b(p), d_b0(2), d_g((size_t)p + 2), d_XY(q), d_XX((size_t)q * q), d_d(1);
-    DBuf<double> d_iter(2 * (size_t)q), d_path((size_t)su.P * L * q), d_lams((size_t)su.P * L);
+    PenaltyTables tb(cx, su, s, p, icpt);
+    DBuf<double> d_cinv(p), d_b(p), d_b0(2), d_g((size_t)p + 2), d_XY(q), d_XX((size_t)q * q), d_d(1);
+    DBuf<double> d_iter(2 * (size_t)q), d_path((size_t)su.P * L * q);
     DBuf<double> d_prob(n + (n & 1)), d_res, d_W(n + (n & 1));
     DBuf<long long> d_iters_total(1);
     DBuf<int> d_niter(1), d_lz(1);
@@ -268,38 +269,17 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
     d_W.zero(cx.stream);
     d_iters_total.zero(cx.stream);
     d_path.zero(cx.stream);
-    d_pf.upload(pf.data(), q, cx.stream);
     d_cinv.upload(cinv.data(), p, cx.stream);
-    {
-        std::vector<double> lam_flat((size_t)su.P * L, 0.0);
-        for (int pp = 0; pp < su.P; ++pp)
-            for (size_t i = 0; i < su.lam[pp].size() && (int)i < L; ++i) lam_flat[(size_t)pp * L + i] = su.lam[pp][i];
-        d_lams.upload(lam_flat.data(), lam_flat.size(), cx.stream);
-        cx.sync();                                  // lam_flat is a host temporary
-    }
-    DBuf<int> g_unique, g_ptr, g_idx, g_cover;
-    DBuf<double> g_w;
-    if (su.any_group) {
-        g_unique.alloc(su.unique.size()); g_unique.upload(su.unique.data(), su.unique.size(), cx.stream);
-        g_ptr.alloc(su.ptr.size());       g_ptr.upload(su.ptr.data(), su.ptr.size(), cx.stream);
-        g_idx.alloc(std::max<size_t>(1, su.idx.size()));
-        if (!su.idx.empty()) g_idx.upload(su.idx.data(), su.idx.size(), cx.stream);
-        g_w.alloc(su.gw.size());          g_w.upload(su.gw.data(), su.gw.size(), cx.stream);
-        g_cover.alloc(q);                 g_cover.upload(su.cover.data(), q, cx.stream);
-    }
     // Hessian bundle: [G p*p | stats 3p | sum W, sum W^2]
     const size_t nbh = (size_t)p * p + 3 * (size_t)p + 2;
     DBuf<double> bh(nbh), d_nobs(1);
     d_nobs.upload(&n_tot, 1, cx.stream);
     DBuf<double> gradb(3 * (size_t)p + 2);   // two-sweep route: [stats 3p | sum r, sum r^2]
-    DBuf<double> d_losspart(1024);
-    PinnedFlag flag;
-    ScratchHolder scratch;
+    PinnedFlags flag(4);          // verdict slots: the host reads slot (iteration & 3) after that iteration's event
+    PathScratches scratch(1);
     wm.mark("setup (stats, slabs, buffers)");
 
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)su.P * (p + 1) * L);
-    double dval = 0.0;
     const double *cinv_dev = stdz ? d_cinv.p : nullptr;
 
     // One IRLS iteration as a chain of kernels on the stream (k = IRLS counter of this lambda).  Every kernel of the chain
@@ -417,23 +397,10 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
                     }
                     form_xy = true;           // XY = XX beta + grad (:999): formed by the path launch below
                 }
-                // inner OEM loop: one chain, one lambda, warm start (oem_logistic_dense.h:1010-1022)
-                PathProblem pr;
-                pr.q = q; pr.ngram = 1; pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p;
-                pr.compute_eig = rebuilt; pr.eig_factor = 1.0005; pr.eig_tol = 1e-10;
-                ChainDesc c;
-                c.gram = 0; c.penalty = su.pen[pp]; c.nlam = 1; c.lam_off = 0; c.alpha = su.alpha;
-                c.gamma = su.gamma[pp]; c.tau = su.tau; c.out_off = 0;
-                pr.chains.push_back(c);
-                pr.lambdas = d_lams.p + (size_t)pp * L + i; pr.Lmax = 1; pr.pen_fact = d_pf.p;
-                pr.ngroups = su.any_group ? (int)su.unique.size() : 0;
-                pr.ngidx = su.any_group ? (int)su.idx.size() : 0;
-                pr.unique_groups = g_unique.p; pr.grp_ptr = g_ptr.p; pr.grp_idx = g_idx.p;
-                pr.group_weights = g_w.p; pr.grp_cover = g_cover.p;
-                pr.beta_init = cur; pr.beta_final = nullptr;
-                pr.maxit = o->maxit; pr.tol = o->tol;
-                pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
-                pr.scratch = scratch.s;
+                PathProblem pr = irls_path_problem(tb, su, pp, i, o);
+                pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p; pr.compute_eig = rebuilt;
+                pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
+                pr.scratch = scratch.s[0];
                 pr.skip = skip;
                 if (form_xy) { pr.xy_grad = d_g.p; pr.xy_cinv = cinv_dev; pr.xy_n = n_tot; pr.xy_icpt = icpt; pr.xy_out = d_XY.p; }
                 pr.t_acc = d_clk.p + 2;
@@ -475,42 +442,17 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
             double *fin = d_iter.p + (size_t)par0 * q;
             OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, fin, sizeof(double) * q, cudaMemcpyDeviceToDevice,
                                      cx.stream));
-            if (s->compute_loss && res->loss) {
-                logistic_loss_kernel<<<1024, 256, 0, cx.stream>>>(yv.p, d_prob.p, n, d_losspart.p);
-                cx.st.kernel_launches += 1;
-                DBuf<double> tot(2);
-                vecsum_launch(cx, d_losspart.p, 1024, 0.0, tot.p, false);
-                cx.all_reduce(tot.p, 2);
-                double h[2];
-                tot.download(h, 2, cx.stream);
-                cx.sync();
-                res->loss[(size_t)pp * L + i] = h[0];
-            }
+            if (s->compute_loss && res->loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, yv.p, d_prob.p, n);
         }
     }
     wm.mark("IRLS loops enqueued");
     // ---- bring the path back, un-scale (get_beta, oem_logistic_dense.h:1038-1055) ----
-    std::vector<double> hpath((size_t)su.P * L * q);
-    long long iters_total = 0;
-    d_path.download(hpath.data(), hpath.size(), cx.stream);
-    d_iters_total.download(&iters_total, 1, cx.stream);
-    d_d.download(&dval, 1, cx.stream);
     unsigned long long hclk[4] = {0, 0, 0, 0};
     d_clk.download(hclk, 4, cx.stream);
-    cx.sync();
+    irls_write_path(cx, su, p, icpt, d_path.p, d_iters_total.p, d_d.p, stdz ? cinv.data() : nullptr, res);
     cx.st.ms_irls_xb += (double)hclk[0] * 1e-6;
     cx.st.ms_path += (double)hclk[2] * 1e-6;
     cx.st.ms_allreduce += (double)hclk[3] * 1e-6;
-    cx.st.d2h_bytes += (int64_t)hpath.size() * 8;
-    cx.st.total_oem_iters += iters_total;
-    for (int pp = 0; pp < su.P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &hpath[((size_t)pp * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = stdz ? raw[icpt + j] * cinv[j] : raw[icpt + j];
-        }
-    *res->d = dval;
     wm.mark("path downloaded");
     finish_stats(cx, tm, t_total, res);
     wm.mark("stats collected");
@@ -604,13 +546,7 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
     if (!(n_tot > q)) fail(OEMB200_EUNSUPPORTED, "oem_fit_logistic_sparse with n <= p + intercept: the reference takes least-squares steps on the 0/1 "
                                           "response there, with a step matrix its d does not bound (src/oem_logistic_sparse.h:503-509, 534-580; "
                                           "restated in oracle/oracle.py:_logistic_wide, which diverges) -- not built");
-    std::vector<double> cinv(p, 1.0);
-    if (stdz)
-        for (int j = 0; j < p; ++j) {
-            double sq = h0[2 * (size_t)p + j] / (n_tot - 1.0);
-            if (sq == 0.0) sq = 1.0;
-            cinv[j] = 1.0 / std::sqrt(sq);
-        }
+    const std::vector<double> cinv = logistic_cinv(h0, p, n_tot, stdz);
     double lmax = 0.0;      // compute_lambda_zero: the X entries of XY = (X'y o colsq_inv) / n only (:808-818)
     for (int j = 0; j < p; ++j) {
         double v = h0[(size_t)p + j];
@@ -620,45 +556,25 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
     su.build_lambdas(s, lmax, /*logistic_fudge=*/true);
 
     // ---- device state ----
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
     const int L = su.Lmax;
+    PenaltyTables tb(cx, su, s, p, icpt);
     const size_t pp2 = (size_t)p * p;
     // per-pass bundle: [G p*p | statsW 3p | sum W, sum W^2 | statsR 3p | sum r, sum r^2]
     const size_t nbp = pp2 + 6 * (size_t)p + 4;
     DBuf<double> bundle(nbp);
     double *G = bundle.p, *statsW = G + pp2, *ws = statsW + 3 * (size_t)p, *statsR = ws + 2, *rs = statsR + 3 * (size_t)p;
-    DBuf<double> d_pf(q), d_cinv(p), d_b(p), d_b0(2), d_g((size_t)p + 2), d_XY(q), d_XX((size_t)q * q), d_d(1), d_diag(p);
-    DBuf<double> d_iter(2 * (size_t)q), d_path((size_t)su.P * L * q), d_lams((size_t)su.P * L);
-    DBuf<double> d_prob(n + 2), d_res(n + 2), d_W(n + 2), d_losspart(1024);
+    DBuf<double> d_cinv(p), d_b(p), d_b0(2), d_g((size_t)p + 2), d_XY(q), d_XX((size_t)q * q), d_d(1), d_diag(p);
+    DBuf<double> d_iter(2 * (size_t)q), d_path((size_t)su.P * L * q);
+    DBuf<double> d_prob(n + 2), d_res(n + 2), d_W(n + 2);
     DBuf<long long> d_iters_total(1);
     DBuf<int> d_niter(1), d_lz(1);
     d_prob.zero(cx.stream);
     d_iters_total.zero(cx.stream);
     d_path.zero(cx.stream);
-    d_pf.upload(pf.data(), q, cx.stream);
     d_cinv.upload(cinv.data(), p, cx.stream);
-    {
-        std::vector<double> lam_flat((size_t)su.P * L, 0.0);
-        for (int pp = 0; pp < su.P; ++pp)
-            for (size_t i = 0; i < su.lam[pp].size() && (int)i < L; ++i) lam_flat[(size_t)pp * L + i] = su.lam[pp][i];
-        d_lams.upload(lam_flat.data(), lam_flat.size(), cx.stream);
-        cx.sync();
-    }
-    DBuf<int> g_unique, g_ptr, g_idx, g_cover;
-    DBuf<double> g_w;
-    if (su.any_group) {
-        g_unique.alloc(su.unique.size()); g_unique.upload(su.unique.data(), su.unique.size(), cx.stream);
-        g_ptr.alloc(su.ptr.size());       g_ptr.upload(su.ptr.data(), su.ptr.size(), cx.stream);
-        g_idx.alloc(std::max<size_t>(1, su.idx.size()));
-        if (!su.idx.empty()) g_idx.upload(su.idx.data(), su.idx.size(), cx.stream);
-        g_w.alloc(su.gw.size());          g_w.upload(su.gw.data(), su.gw.size(), cx.stream);
-        g_cover.alloc(q);                 g_cover.upload(su.cover.data(), q, cx.stream);
-    }
-    PinnedFlag flag;
-    ScratchHolder scratch;
+    PinnedFlags flag(1);
+    PathScratches scratch(1);
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)su.P * (p + 1) * L);
     const double *cinv_dev = stdz ? d_cinv.p : nullptr;
     double xxdiag = 0.0, intval = 0.0;
 
@@ -715,22 +631,10 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
                     path_xy_launch(cx, q, icpt, d_XX.p, cur, d_g.p, cinv_dev, n_tot, d_XY.p, nullptr);
                     rebuilt = true;
                 }
-                PathProblem pr;
-                pr.q = q; pr.ngram = 1; pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p;
-                pr.compute_eig = rebuilt; pr.eig_factor = 1.0005; pr.eig_tol = 1e-10;
-                ChainDesc c;
-                c.gram = 0; c.penalty = su.pen[pp]; c.nlam = 1; c.lam_off = 0; c.alpha = su.alpha;
-                c.gamma = su.gamma[pp]; c.tau = su.tau; c.out_off = 0;
-                pr.chains.push_back(c);
-                pr.lambdas = d_lams.p + (size_t)pp * L + i; pr.Lmax = 1; pr.pen_fact = d_pf.p;
-                pr.ngroups = su.any_group ? (int)su.unique.size() : 0;
-                pr.ngidx = su.any_group ? (int)su.idx.size() : 0;
-                pr.unique_groups = g_unique.p; pr.grp_ptr = g_ptr.p; pr.grp_idx = g_idx.p;
-                pr.group_weights = g_w.p; pr.grp_cover = g_cover.p;
-                pr.beta_init = cur; pr.beta_final = nullptr;
-                pr.maxit = o->maxit; pr.tol = o->tol;
-                pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
-                pr.scratch = scratch.s;
+                PathProblem pr = irls_path_problem(tb, su, pp, i, o);
+                pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p; pr.compute_eig = rebuilt;
+                pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
+                pr.scratch = scratch.s[0];
                 const size_t t3 = tm.start(&cx.st.ms_path);
                 path_launch(cx, pr);
                 tm.stop(t3);
@@ -747,36 +651,10 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
             }
             OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, cur, sizeof(double) * q, cudaMemcpyDeviceToDevice,
                                      cx.stream));
-            if (s->compute_loss && res->loss) {
-                logistic_loss_kernel<<<1024, 256, 0, cx.stream>>>(yv.p, d_prob.p, n, d_losspart.p);
-                cx.st.kernel_launches += 1;
-                DBuf<double> tot(2);
-                vecsum_launch(cx, d_losspart.p, 1024, 0.0, tot.p, false);
-                cx.all_reduce(tot.p, 2);
-                double h[2];
-                tot.download(h, 2, cx.stream);
-                cx.sync();
-                res->loss[(size_t)pp * L + i] = h[0];
-            }
+            if (s->compute_loss && res->loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, yv.p, d_prob.p, n);
         }
     }
-    std::vector<double> hpath((size_t)su.P * L * q);
-    long long iters_total = 0;
-    double dval = 0.0;
-    d_path.download(hpath.data(), hpath.size(), cx.stream);
-    d_iters_total.download(&iters_total, 1, cx.stream);
-    d_d.download(&dval, 1, cx.stream);
-    cx.sync();
-    cx.st.d2h_bytes += (int64_t)hpath.size() * 8;
-    cx.st.total_oem_iters += iters_total;
-    for (int pp = 0; pp < su.P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &hpath[((size_t)pp * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = stdz ? raw[icpt + j] * cinv[j] : raw[icpt + j];
-        }
-    *res->d = dval;
+    irls_write_path(cx, su, p, icpt, d_path.p, d_iters_total.p, d_d.p, stdz ? cinv.data() : nullptr, res);
     finish_stats(cx, tm, t_total, res);
 }
 

@@ -687,25 +687,18 @@ void fit_sparse(const int *row_idx, const int *col_ptr, const double *values, in
     for (int j = icpt; j < q; ++j) lmax = std::max(lmax, std::fabs(hXYlam.empty() ? hXY[j] : hXYlam[j]));
     su.build_lambdas(s, lmax, false);
 
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
+    PenaltyTables tb(cx, su, s, p, icpt);
     PathBuffers pb;
     const size_t t_p = tm.start(&cx.st.ms_path);
     // get_beta() multiplies the member beta(0) by intval in place (src/oem_sparse.h:895-900): the path kernel's post-scale
-    run_paths(cx, su, o, q, 1, pXX, pXY, pf, 1.0, 1.005, false, icpt ? dscale.p : nullptr, pb);
+    run_paths(cx, su, tb, o, 1, pXX, pXY, 1.005, false, icpt ? dscale.p : nullptr, pb);
     tm.stop(t_p);
 
     const int L = su.Lmax;
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)su.P * (p + 1) * L);
+    write_beta(su, pb.h_beta.data(), p, icpt, s->standardize ? hcinv.data() : nullptr, res);
     for (int pp = 0; pp < su.P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &pb.h_beta[((size_t)pp * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = s->standardize ? raw[icpt + j] * hcinv[j] : raw[icpt + j];
-            res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)pp * L + i];
-        }
+        for (int i = 0; i < su.nlam_run[pp]; ++i) res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)pp * L + i];
     *res->d = pb.h_d[0];
 
     // ---- compute.loss: all (penalty, lambda) columns in one pass over the CSR copy ----

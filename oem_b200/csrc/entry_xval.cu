@@ -218,24 +218,17 @@ void fit_xval(const double *x, int64_t n, int p, int64_t ldx, const double *y, c
     su.build_lambdas(s, lmax, false);
 
     // ---- 4. all chains in one persistent launch ----
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
+    PenaltyTables tb(cx, su, s, p, icpt);
     PathBuffers pb;
     const size_t t_p = tm.start(&cx.st.ms_path);
-    run_paths(cx, su, o, q, NG, XX.p, XY.p, pf, 1.0, 1.005, false, nullptr, pb);
+    run_paths(cx, su, tb, o, NG, XX.p, XY.p, 1.005, false, nullptr, pb);
     tm.stop(t_p);
 
     const int L = su.Lmax, P = su.P;
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)P * (p + 1) * L);
+    write_beta(su, pb.h_beta.data(), p, icpt, s->standardize ? hcinv.data() : nullptr, res);   // the full-data chains
     for (int pp = 0; pp < P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &pb.h_beta[((size_t)(0 * P + pp) * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = s->standardize ? raw[icpt + j] * hcinv[j] : raw[icpt + j];
-            res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)(0 * P + pp) * L + i];
-        }
+        for (int i = 0; i < su.nlam_run[pp]; ++i) res->niter[(size_t)pp * L + i] = pb.h_niter[(size_t)pp * L + i];
     *res->d = pb.h_d[0];
 
     // ---- 5. CV scoring: coefficient matrices [fold][p][ncld], intercepts [fold][ncld] ----

@@ -26,22 +26,6 @@
 
 namespace oemb200 {
 
-namespace {
-struct PinnedFlags {          // one verdict slot per model, written by its path launch
-    int *p = nullptr;
-    explicit PinnedFlags(int m) {
-        OEM_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&p), sizeof(int) * (size_t)m, cudaHostAllocMapped));
-        memset(p, 0, sizeof(int) * (size_t)m);
-    }
-    ~PinnedFlags() { if (p) cudaFreeHost(p); }
-};
-struct Scratches {
-    std::vector<PathScratch *> s;
-    explicit Scratches(int m) { for (int i = 0; i < m; ++i) s.push_back(path_scratch_create()); }
-    ~Scratches() { for (auto *x : s) path_scratch_destroy(x); }
-};
-}  // namespace
-
 void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s, int nfolds,
                        const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res) {
     check_common(s, o, res, "binomial");
@@ -99,11 +83,9 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
 
     // ---- device state: one slice per model ----
     const int L = su.Lmax, P = su.P;
-    std::vector<double> pf(q, 0.0);
-    for (int j = 0; j < p; ++j) pf[icpt + j] = s->penalty_factor[j];
-    DBuf<double> d_pf(q), d_B((size_t)M * p), d_b0(M), d_G((size_t)M * (p + 1)), d_XY((size_t)M * q), d_d(M);
-    DBuf<double> d_iter((size_t)M * 2 * q), d_path((size_t)M * P * L * q), d_lams((size_t)P * L), d_prob(npad);
-    DBuf<double> d_losspart(1024), d_losstot(2);
+    PenaltyTables tb(cx, su, s, p, icpt);
+    DBuf<double> d_B((size_t)M * p), d_b0(M), d_G((size_t)M * (p + 1)), d_XY((size_t)M * q), d_d(M);
+    DBuf<double> d_iter((size_t)M * 2 * q), d_path((size_t)M * P * L * q), d_prob(npad);
     DBuf<long long> d_iters_total(1);
     DBuf<int> d_niter(M), d_lz(M), d_conv(M);
     DBuf<unsigned long long> d_clk(1);
@@ -111,28 +93,9 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
     d_path.zero(cx.stream);
     d_iters_total.zero(cx.stream);
     d_clk.zero(cx.stream);
-    d_pf.upload(pf.data(), q, cx.stream);
-    {
-        std::vector<double> lam_flat((size_t)P * L, 0.0);
-        for (int pp = 0; pp < P; ++pp)
-            for (size_t i = 0; i < su.lam[pp].size() && (int)i < L; ++i) lam_flat[(size_t)pp * L + i] = su.lam[pp][i];
-        d_lams.upload(lam_flat.data(), lam_flat.size(), cx.stream);
-        cx.sync();
-    }
-    DBuf<int> g_unique, g_ptr, g_idx, g_cover;
-    DBuf<double> g_w;
-    if (su.any_group) {
-        g_unique.alloc(su.unique.size()); g_unique.upload(su.unique.data(), su.unique.size(), cx.stream);
-        g_ptr.alloc(su.ptr.size());       g_ptr.upload(su.ptr.data(), su.ptr.size(), cx.stream);
-        g_idx.alloc(std::max<size_t>(1, su.idx.size()));
-        if (!su.idx.empty()) g_idx.upload(su.idx.data(), su.idx.size(), cx.stream);
-        g_w.alloc(su.gw.size());          g_w.upload(su.gw.data(), su.gw.size(), cx.stream);
-        g_cover.alloc(q);                 g_cover.upload(su.cover.data(), q, cx.stream);
-    }
-    PinnedFlags flags(M);
-    Scratches scratch(M);
+    PinnedFlags flags(M);         // one verdict slot per model, written by its path launch
+    PathScratches scratch(M);
     fill_common_outputs(su, res);
-    memset(res->beta, 0, sizeof(double) * (size_t)P * (p + 1) * L);
     const double *cinv_all = stdz ? xs.cinv.p : nullptr;
     const bool want_loss = s->compute_loss && res->loss;
 
@@ -163,21 +126,9 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
                     double *base = d_iter.p + 2 * qm;
                     double *cur = base + (size_t)((par0[m] + k) & 1) * q, *nxt = base + (size_t)((par0[m] + k + 1) & 1) * q;
                     const double *cinv_m = cinv_all ? cinv_all + (size_t)m * p : nullptr;
-                    PathProblem pr;
-                    pr.q = q; pr.ngram = 1; pr.XX = xs.XX.p + qm * q; pr.XY = d_XY.p + qm; pr.d = d_d.p + m;
-                    pr.compute_eig = (k == 0 && i == 0); pr.eig_factor = 1.0005; pr.eig_tol = 1e-10;
-                    ChainDesc c;
-                    c.gram = 0; c.penalty = su.pen[pp]; c.nlam = 1; c.lam_off = 0; c.alpha = su.alpha;
-                    c.gamma = su.gamma[pp]; c.tau = su.tau; c.out_off = 0;
-                    pr.chains.push_back(c);
-                    pr.lambdas = d_lams.p + (size_t)pp * L + i; pr.Lmax = 1; pr.pen_fact = d_pf.p;
-                    pr.ngroups = su.any_group ? (int)su.unique.size() : 0;
-                    pr.ngidx = su.any_group ? (int)su.idx.size() : 0;
-                    pr.unique_groups = g_unique.p; pr.grp_ptr = g_ptr.p; pr.grp_idx = g_idx.p;
-                    pr.group_weights = g_w.p; pr.grp_cover = g_cover.p;
-                    pr.beta_init = cur; pr.beta_final = nullptr;
-                    pr.maxit = o->maxit; pr.tol = o->tol;
-                    pr.beta_out = nxt; pr.niter_out = d_niter.p + m; pr.lanczos_steps = d_lz.p + m;
+                    PathProblem pr = irls_path_problem(tb, su, pp, i, o);
+                    pr.XX = xs.XX.p + qm * q; pr.XY = d_XY.p + qm; pr.d = d_d.p + m; pr.compute_eig = (k == 0 && i == 0);
+                    pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p + m; pr.lanczos_steps = d_lz.p + m;
                     pr.scratch = scratch.s[m];
                     pr.skip = d_conv.p + m;
                     if (pass) {
@@ -211,37 +162,16 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
                 OEM_CUDA(cudaMemcpyAsync(d_path.p + (((size_t)m * P + pp) * L + i) * q, fin, sizeof(double) * q,
                                          cudaMemcpyDeviceToDevice, cx.stream));
             }
-            if (want_loss) {          // padding rows hold prob = 0 and y = 0: their terms are log(1) = 0
-                logistic_loss_launch(cx, xs.ys.p, d_prob.p, npad, d_losspart.p, d_losstot.p);
-                double h[2];
-                d_losstot.download(h, 2, cx.stream);
-                cx.sync();
-                res->loss[(size_t)pp * L + i] = h[0];
-            }
+            // padding rows hold prob = 0 and y = 0: their terms are log(1) = 0
+            if (want_loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, xs.ys.p, d_prob.p, npad);
         }
     }
 
     // ---- full model back to the host, un-scaled (get_beta) ----
-    std::vector<double> hpath((size_t)P * L * q);
-    long long iters_total = 0;
-    double dval = 0.0;
     unsigned long long hclk = 0;
-    OEM_CUDA(cudaMemcpyAsync(hpath.data(), d_path.p, hpath.size() * 8, cudaMemcpyDeviceToHost, cx.stream));
-    d_iters_total.download(&iters_total, 1, cx.stream);
-    d_d.download(&dval, 1, cx.stream);
     d_clk.download(&hclk, 1, cx.stream);
-    cx.sync();
+    irls_write_path(cx, su, p, icpt, d_path.p, d_iters_total.p, d_d.p, stdz ? xs.hcinv.data() : nullptr, res);
     cx.st.ms_path += (double)hclk * 1e-6;
-    cx.st.d2h_bytes += (int64_t)hpath.size() * 8;
-    cx.st.total_oem_iters += iters_total;
-    for (int pp = 0; pp < P; ++pp)
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            const double *raw = &hpath[((size_t)pp * L + i) * q];
-            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
-            if (icpt) out[0] = raw[0];
-            for (int j = 0; j < p; ++j) out[1 + j] = stdz ? raw[icpt + j] * xs.hcinv[j] : raw[icpt + j];
-        }
-    *res->d = dval;
 
     // ---- CV scoring: fold k's rows against fold model k ----
     const int nc = P * L, ncld = cv_ncld(nc);

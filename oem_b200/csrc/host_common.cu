@@ -1,5 +1,6 @@
 // host_common.cu -- see host_common.h.  Host logic only (no kernels): penalty / group / lambda
-// bookkeeping restated from the reference's entry functions, and the path-kernel round trip.
+// bookkeeping restated from the reference's entry functions, its device tables, the path-kernel round trip and the
+// write-back of the raw iterates into the reported beta.
 #include <algorithm>
 #include <cstring>
 #include "host_common.h"
@@ -129,28 +130,38 @@ void Setup::build_lambdas(const oemb200_spec *s, double lmax, bool logistic_fudg
     }
 }
 
-void run_paths(Ctx &cx, const Setup &su, const oemb200_opts *o, int q, int ngram, const double *XX, const double *XY,
-               const std::vector<double> &pen_fact_q, double lam_scale, double eig_factor, bool accelerate,
-               const double *post_scale_dev, PathBuffers &pb) {
-    const int P = su.P, L = su.Lmax;
-    std::vector<double> lam_flat;
-    pb.lam_off.assign(P, 0);
-    for (int pp = 0; pp < P; ++pp) {
-        pb.lam_off[pp] = (int)lam_flat.size();
-        for (double x : su.lam[pp]) lam_flat.push_back(x / lam_scale);
-    }
-    pb.lambdas.alloc(std::max<size_t>(1, lam_flat.size()));
-    pb.lambdas.upload(lam_flat.data(), lam_flat.size(), cx.stream);
-    pb.pen_fact.alloc(q);
-    pb.pen_fact.upload(pen_fact_q.data(), q, cx.stream);
+PenaltyTables::PenaltyTables(Ctx &cx, const Setup &su, const oemb200_spec *s, int p, int icpt, double lam_scale)
+    : q(p + icpt), Lmax(su.Lmax), ngroups(su.any_group ? (int)su.unique.size() : 0),
+      ngidx(su.any_group ? (int)su.idx.size() : 0), h_pf(q, 0.0) {
+    for (int pp = 0; pp < su.P; ++pp)
+        for (double x : su.lam[pp]) h_lam.push_back(x / lam_scale);
+    for (int j = 0; j < p; ++j) h_pf[icpt + j] = s->penalty_factor[j];
+    lambdas.alloc(h_lam.size());
+    lambdas.upload(h_lam.data(), h_lam.size(), cx.stream);
+    pen_fact.alloc(q);
+    pen_fact.upload(h_pf.data(), q, cx.stream);
     if (su.any_group) {
-        pb.unique.alloc(su.unique.size()); pb.unique.upload(su.unique.data(), su.unique.size(), cx.stream);
-        pb.ptr.alloc(su.ptr.size());       pb.ptr.upload(su.ptr.data(), su.ptr.size(), cx.stream);
-        pb.idx.alloc(std::max<size_t>(1, su.idx.size()));
-        if (!su.idx.empty()) pb.idx.upload(su.idx.data(), su.idx.size(), cx.stream);
-        pb.gw.alloc(su.gw.size());         pb.gw.upload(su.gw.data(), su.gw.size(), cx.stream);
-        pb.cover.alloc(q);                 pb.cover.upload(su.cover.data(), q, cx.stream);
+        unique.alloc(su.unique.size()); unique.upload(su.unique.data(), su.unique.size(), cx.stream);
+        ptr.alloc(su.ptr.size());       ptr.upload(su.ptr.data(), su.ptr.size(), cx.stream);
+        idx.alloc(std::max<size_t>(1, su.idx.size()));
+        if (!su.idx.empty()) idx.upload(su.idx.data(), su.idx.size(), cx.stream);
+        gw.alloc(su.gw.size());         gw.upload(su.gw.data(), su.gw.size(), cx.stream);
+        cover.alloc(q);                 cover.upload(su.cover.data(), q, cx.stream);
     }
+}
+
+// the penalty-factor and group fields of a path launch
+static void use_tables(PathProblem &pr, const PenaltyTables &tb) {
+    pr.pen_fact = tb.pen_fact.p;
+    pr.ngroups = tb.ngroups;
+    pr.ngidx = tb.ngidx;
+    pr.unique_groups = tb.unique.p; pr.grp_ptr = tb.ptr.p; pr.grp_idx = tb.idx.p;
+    pr.group_weights = tb.gw.p; pr.grp_cover = tb.cover.p;
+}
+
+void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int ngram, const double *XX,
+               const double *XY, double eig_factor, bool accelerate, const double *post_scale_dev, PathBuffers &pb) {
+    const int P = su.P, L = su.Lmax, q = tb.q;
     const int nchains = ngram * P;
     pb.beta_out.alloc((size_t)nchains * L * q);
     pb.beta_out.zero(cx.stream);
@@ -166,15 +177,12 @@ void run_paths(Ctx &cx, const Setup &su, const oemb200_opts *o, int q, int ngram
     for (int g = 0; g < ngram; ++g)
         for (int k = 0; k < P; ++k) {
             ChainDesc c;
-            c.gram = g; c.penalty = su.pen[k]; c.nlam = su.nlam_run[k]; c.lam_off = pb.lam_off[k];
+            c.gram = g; c.penalty = su.pen[k]; c.nlam = su.nlam_run[k]; c.lam_off = k * L;
             c.alpha = su.alpha; c.gamma = su.gamma[k]; c.tau = su.tau; c.out_off = g * P + k;
             pp.chains.push_back(c);
         }
-    pp.lambdas = pb.lambdas.p; pp.Lmax = L; pp.pen_fact = pb.pen_fact.p;
-    pp.ngroups = su.any_group ? (int)su.unique.size() : 0;
-    pp.ngidx = su.any_group ? (int)su.idx.size() : 0;
-    pp.unique_groups = pb.unique.p; pp.grp_ptr = pb.ptr.p; pp.grp_idx = pb.idx.p;
-    pp.group_weights = pb.gw.p; pp.grp_cover = pb.cover.p;
+    pp.lambdas = tb.lambdas.p; pp.Lmax = L;
+    use_tables(pp, tb);
     pp.post_scale = post_scale_dev;
     pp.maxit = o->maxit; pp.tol = o->tol; pp.accelerate = accelerate;
     pp.beta_out = pb.beta_out.p; pp.niter_out = pb.niter.p; pp.lanczos_steps = pb.lz.p;
@@ -193,6 +201,47 @@ void run_paths(Ctx &cx, const Setup &su, const oemb200_opts *o, int q, int ngram
     cx.st.d2h_bytes += (int64_t)(pb.h_beta.size() * 8 + pb.h_niter.size() * 4);
     for (int v : pb.h_niter) cx.st.total_oem_iters += v;
     for (int v : pb.h_lz) cx.st.lanczos_steps += v;
+}
+
+PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o) {
+    PathProblem pr;
+    pr.q = tb.q; pr.ngram = 1;
+    pr.eig_factor = 1.0005; pr.eig_tol = 1e-10;
+    ChainDesc c;
+    c.gram = 0; c.penalty = su.pen[pp]; c.nlam = 1; c.lam_off = 0; c.alpha = su.alpha;
+    c.gamma = su.gamma[pp]; c.tau = su.tau; c.out_off = 0;
+    pr.chains.push_back(c);
+    pr.lambdas = tb.lambdas.p + (size_t)pp * tb.Lmax + i; pr.Lmax = 1;
+    use_tables(pr, tb);
+    pr.maxit = o->maxit; pr.tol = o->tol;
+    return pr;
+}
+
+void write_beta(const Setup &su, const double *raw, int p, int icpt, const double *cinv, oemb200_result *res) {
+    const int L = su.Lmax, q = p + icpt;
+    memset(res->beta, 0, sizeof(double) * (size_t)su.P * (p + 1) * L);
+    for (int pp = 0; pp < su.P; ++pp)
+        for (int i = 0; i < su.nlam_run[pp]; ++i) {
+            const double *r = raw + ((size_t)pp * L + i) * q;
+            double *out = res->beta + ((size_t)pp * L + i) * (p + 1);
+            if (icpt) out[0] = r[0];
+            for (int j = 0; j < p; ++j) out[1 + j] = cinv ? r[icpt + j] * cinv[j] : r[icpt + j];
+        }
+}
+
+void irls_write_path(Ctx &cx, const Setup &su, int p, int icpt, const double *path_dev, const long long *iters_total_dev,
+                     const double *d_dev, const double *cinv, oemb200_result *res) {
+    std::vector<double> hpath((size_t)su.P * su.Lmax * (p + icpt));
+    long long iters_total = 0;
+    double dval = 0.0;
+    OEM_CUDA(cudaMemcpyAsync(hpath.data(), path_dev, hpath.size() * 8, cudaMemcpyDeviceToHost, cx.stream));
+    OEM_CUDA(cudaMemcpyAsync(&iters_total, iters_total_dev, sizeof iters_total, cudaMemcpyDeviceToHost, cx.stream));
+    OEM_CUDA(cudaMemcpyAsync(&dval, d_dev, sizeof dval, cudaMemcpyDeviceToHost, cx.stream));
+    cx.sync();
+    cx.st.d2h_bytes += (int64_t)hpath.size() * 8;
+    cx.st.total_oem_iters += iters_total;
+    write_beta(su, hpath.data(), p, icpt, cinv, res);
+    *res->d = dval;
 }
 
 }  // namespace oemb200

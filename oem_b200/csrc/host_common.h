@@ -1,6 +1,7 @@
-// host_common.h -- host-side bookkeeping shared by the five entry points: penalty / group / lambda
-// setup (the part of the reference's entry functions that is not arithmetic on X), and the helper
-// that runs a set of chains through the path kernel and brings the raw iterates back.
+// host_common.h -- host-side bookkeeping shared by the fit drivers: penalty / group / lambda setup (the part of the
+// reference's entry functions that is not arithmetic on X) and its device mirror, the helper that runs a set of chains
+// through the path kernel and brings the raw iterates back, the one-lambda path problem of the IRLS drivers, and the
+// layout of the reported beta.
 #pragma once
 #include <cmath>
 #include <string>
@@ -26,7 +27,8 @@ struct Setup {
     std::vector<int> pen;                 // penalty ids
     std::vector<double> gamma;            // per penalty
     double alpha = 1.0, tau = 0.5;        // call-wide scalars
-    std::vector<std::vector<double>> lam; // per penalty (filled by build_lambdas)
+    std::vector<std::vector<double>> lam; // per penalty (filled by build_lambdas), Lmax entries each: parse requires
+                                          // equal-length user sequences, the generated grid has nlambda = Lmax
     std::vector<int> nlam_run;            // lambdas actually run (ols: 1)
     bool lambda_given = false;
     // groups (CSR over unique groups)
@@ -41,22 +43,59 @@ struct Setup {
     void build_lambdas(const oemb200_spec *s, double lmax, bool logistic_fudge);
 };
 
-// Device-side mirrors of a Setup + the buffers a path launch fills.
+// Device mirror of a Setup, uploaded once per fit: the lambdas (P x Lmax, penalty pp at pp * Lmax) divided by lam_scale
+// (scaleY for oem_fit_dense, else 1), the penalty factor of length q = p + icpt (0 in the unpenalised intercept slot)
+// and the group CSR.  h_lam / h_pf are the host sources of the asynchronous uploads and live as long as the tables.
+struct PenaltyTables {
+    int q = 0, Lmax = 0, ngroups = 0, ngidx = 0;
+    std::vector<double> h_lam, h_pf;
+    DBuf<double> lambdas, pen_fact, gw;
+    DBuf<int> unique, ptr, idx, cover;
+    PenaltyTables(Ctx &cx, const Setup &su, const oemb200_spec *s, int p, int icpt, double lam_scale = 1.0);
+};
+
+// The buffers a path launch fills.
 struct PathBuffers {
-    DBuf<double> lambdas, pen_fact, gw, beta_out, d, beta_final;
-    DBuf<int> unique, ptr, idx, cover, niter, lz;
-    std::vector<int> lam_off;     // per penalty
+    DBuf<double> beta_out, d;
+    DBuf<int> niter, lz;
     std::vector<double> h_beta;   // nchains x Lmax x q raw iterates
     std::vector<int> h_niter;     // nchains x Lmax
     std::vector<double> h_d;      // ngram
     std::vector<int> h_lz;
 };
 
-// Run chains = ngram x P (chain index = g * P + pp) on XX / XY.  pen_fact_q: host, length q.
-// lam_scale: lambdas handed to the solver are lam / lam_scale (scaleY for oem_fit_dense, else 1).
-void run_paths(Ctx &cx, const Setup &su, const oemb200_opts *o, int q, int ngram, const double *XX, const double *XY,
-               const std::vector<double> &pen_fact_q, double lam_scale, double eig_factor, bool accelerate,
-               const double *post_scale_dev, PathBuffers &pb);
+// Run chains = ngram x P (chain index = g * P + pp) on XX / XY.
+void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int ngram, const double *XX,
+               const double *XY, double eig_factor, bool accelerate, const double *post_scale_dev, PathBuffers &pb);
+
+// The inner OEM loop of one IRLS iteration (src/oem_logistic_dense.h:1010-1022): one chain, lambda i of penalty pp, warm
+// start, eigenvalue factor 1.0005.  The caller sets XX / XY / d, compute_eig, beta_init / beta_out, niter_out /
+// lanczos_steps / scratch, skip and the irls_* / xy_* / t_acc fields.
+PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o);
+
+// res->beta (P x Lmax x (p + 1): intercept row first, zero where no lambda ran) from the raw q-vectors of a fit, iterate
+// (pp, i) at raw + (pp * Lmax + i) * q with q = p + icpt; cinv (host, p) undoes the standardisation, NULL if none.
+void write_beta(const Setup &su, const double *raw, int p, int icpt, const double *cinv, oemb200_result *res);
+// End of an IRLS driver: one sync brings the raw path (P x Lmax x q at path_dev), d of the first model and the count of
+// inner iterations to the host, after whatever the caller enqueued before; then res->beta (write_beta) and *res->d.
+void irls_write_path(Ctx &cx, const Setup &su, int p, int icpt, const double *path_dev, const long long *iters_total_dev,
+                     const double *d_dev, const double *cinv, oemb200_result *res);
+
+// n mapped pinned ints: the IRLS verdict slots a path launch writes (PathProblem::irls_host_flag) and the host reads
+struct PinnedFlags {
+    int *p = nullptr;
+    explicit PinnedFlags(int n) {
+        OEM_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&p), sizeof(int) * (size_t)n, cudaHostAllocMapped));
+        memset(p, 0, sizeof(int) * (size_t)n);
+    }
+    ~PinnedFlags() { if (p) cudaFreeHost(p); }
+};
+// n PathScratch tables, one per chain layout that is launched over and over
+struct PathScratches {
+    std::vector<PathScratch *> s;
+    explicit PathScratches(int n) { for (int i = 0; i < n; ++i) s.push_back(path_scratch_create()); }
+    ~PathScratches() { for (auto *x : s) path_scratch_destroy(x); }
+};
 
 // ---- shared by the entry drivers (entries.cu) ----
 void check_common(const oemb200_spec *s, const oemb200_opts *o, const oemb200_result *r, const char *want_family,
@@ -95,8 +134,8 @@ void xval_build_systems(Ctx &cx, const double *x, int64_t n, int p, int64_t ldx,
                         int F, const int *foldid, int icpt, bool stdz, double hess_scale, XvalSystems &xs);
 
 // ---- entry_logistic.cu ----
-// tot[0] = get_loss() of prob (src/oem_logistic_dense.h:1057-1088) summed over n rows; partial: 1024 doubles of scratch
-void logistic_loss_launch(Ctx &cx, const double *y, const double *prob, int64_t n, double *partial, double *tot2);
+// get_loss() of prob (src/oem_logistic_dense.h:1057-1088) summed over the n rows and over ranks
+double logistic_loss(Ctx &cx, const double *y, const double *prob, int64_t n);
 
 // row-slab copy of X kept across logistic fits (owned by an oemb200_matrix handle); `rt` = rows per slab it was built with
 struct SlabCache { double *slabs = nullptr; int rt = 0; };

@@ -101,18 +101,9 @@ static void fit_big(const double *x, int64_t n, int p, int64_t ldx, const double
     vecsum_launch(cx, yv.p, n, 0.0, ysum, false);
     tm.stop(t_y);
 
-    // column sums, X'y and sum x^2 ride in the Gram launch (diagonal-tile CTAs); OEMB200_SEPARATE_COLSTATS=1 keeps the
-    // separate HBM sweep (colstats_kernel) for A/B measurements
-    const bool fused_stats = getenv("OEMB200_SEPARATE_COLSTATS") == nullptr;
+    // column sums, X'y and sum x^2 ride in the Gram launch (diagonal-tile CTAs)
     if (is_device_ptr(x)) {
-        if (fused_stats) {
-            gram_launch(cx, x, n, p, ldx, {RowSegment{0, n, 0}}, 1, nullptr, nullptr, G, false, yv.p, stats);
-        } else {
-            const size_t t1 = tm.start(&cx.st.ms_colstats);
-            colstats_launch(cx, x, n, p, ldx, nullptr, yv.p, nullptr, stats, false);
-            tm.stop(t1);
-            gram_launch(cx, x, n, p, ldx, {RowSegment{0, n, 0}}, 1, nullptr, nullptr, G, false);
-        }
+        gram_launch(cx, x, n, p, ldx, {RowSegment{0, n, 0}}, 1, nullptr, nullptr, G, false, yv.p, stats);
     } else {
         // host X: double-buffered row chunks; H2D of chunk c+1 overlaps the kernels of chunk c
         const double gigs = o->gigs > 0 ? o->gigs : 1.0;
@@ -158,12 +149,7 @@ static void fit_big(const double *x, int64_t n, int p, int64_t ldx, const double
             const int b = (int)(c & 1);
             const int64_t r0 = c * rows, nr = std::min(rows, n - r0);
             OEM_CUDA(cudaStreamWaitEvent(cx.stream, ready[b], 0));
-            if (fused_stats) {
-                gram_launch(cx, stage[b].p, nr, p, rows, {RowSegment{0, nr, 0}}, 1, nullptr, nullptr, G, c > 0, yv.p + r0, stats);
-            } else {
-                colstats_launch(cx, stage[b].p, nr, p, rows, nullptr, yv.p + r0, nullptr, stats, c > 0);
-                gram_launch(cx, stage[b].p, nr, p, rows, {RowSegment{0, nr, 0}}, 1, nullptr, nullptr, G, c > 0);
-            }
+            gram_launch(cx, stage[b].p, nr, p, rows, {RowSegment{0, nr, 0}}, 1, nullptr, nullptr, G, c > 0, yv.p + r0, stats);
             OEM_CUDA(cudaEventRecord(freed[b], cx.stream));
             // chunk c's kernels are queued: now stage the copy after next (pinned sources: an asynchronous DMA, queued one
             // chunk further ahead; pageable sources: the reader threads fill the bounce ring while those kernels run)
@@ -287,19 +273,14 @@ static void fit_dense(const double *x, int64_t n, int p, int64_t ldx, const doub
     const size_t nb2 = (size_t)p * p + 2 * (size_t)p;
     DBuf<double> b2(nb2), stats2(3 * (size_t)p);
     double *G = b2.p, *xy = G + (size_t)p * p, *css = xy + p;
-    // X'ys and the (centred) sums of squares can ride in the Gram launch (diagonal-tile CTAs, CENTER + STATS variant), but
-    // for this entry it does not pay: the centred variant masks the tail rows of every fragment, and measured on a B200
-    // the fused launch lost at both ends -- n = 1e6 x p = 100: 2.84 ms per fit against 2.41 ms; n = 2e6 x p = 512:
-    // 28.9 ms against 27.3 ms (Gram 19.9 vs 18.4 ms for a 1.2 ms sweep saved; tools/bench_dense_stats.py).  The separate
-    // HBM sweep therefore stays the default whenever X is centred; OEMB200_FUSED_COLSTATS=1 selects the fused launch
-    // (kept under test).  Uncentred, unscaled fits (flag 0) use the plain STATS variant that already pays for big.oem and
-    // xval.oem from p = 500 up.
-    const bool forced = getenv("OEMB200_FUSED_COLSTATS") != nullptr;
-    const bool fused_stats = getenv("OEMB200_SEPARATE_COLSTATS") == nullptr &&
-                             ((flag != 1 && forced) || (flag == 0 && p >= 256 && (double)n * p >= 268435456.0));
+    // Uncentred, unscaled fits (flag 0) take X'y and the sums of squares from the Gram launch (diagonal-tile CTAs), which
+    // pays for big.oem and xval.oem from p = 500 up.  Centred statistics from the Gram launch do not pay for this entry:
+    // masking the tail rows of every fragment slowed the Gram more than the sweep it saved, and measured on a B200 the
+    // fused launch lost at both ends -- n = 1e6 x p = 100: 2.84 ms per fit against 2.41 ms; n = 2e6 x p = 512: 28.9 ms
+    // against 27.3 ms (Gram 19.9 vs 18.4 ms for a 1.2 ms sweep saved).  Every other fit takes them from a separate HBM sweep.
+    const bool fused_stats = flag == 0 && p >= 256 && (double)n * p >= 268435456.0;
     if (fused_stats) {
-        gram_launch(cx, X.p, n, p, X.ld, {RowSegment{0, n, 0}}, 1, center_x ? d_mean.p : nullptr, nullptr, G, false, yuse,
-                    stats2.p);
+        gram_launch(cx, X.p, n, p, X.ld, {RowSegment{0, n, 0}}, 1, nullptr, nullptr, G, false, yuse, stats2.p);
         OEM_CUDA(cudaMemcpyAsync(xy, stats2.p + (size_t)p, (size_t)p * 8, cudaMemcpyDeviceToDevice, cx.stream));
         OEM_CUDA(cudaMemcpyAsync(css, stats2.p + 2 * (size_t)p, (size_t)p * 8, cudaMemcpyDeviceToDevice, cx.stream));
     } else {

@@ -119,20 +119,20 @@ void xval_build_systems(Ctx &cx, const double *x, int64_t n, int p, int64_t ldx,
     double *corner = nobs + F;
     std::vector<RowSegment> segs;
     for (int k = 0; k < F; ++k) segs.push_back(RowSegment{off[k], off[k + 1], k});
-    // unweighted: the per-fold column sums / X'y / sum x^2 ride in the Gram launch (diagonal-tile CTAs)
-    const bool fused_stats = !weighted && getenv("OEMB200_SEPARATE_COLSTATS") == nullptr;
-    if (fused_stats) gram_launch(cx, Xs.p, npad, p, npad, segs, F, nullptr, nullptr, G, false, ys.p, stats);
-    else gram_launch(cx, Xs.p, npad, p, npad, segs, F, nullptr, weighted ? ws.p : nullptr, G, false);
+    // unweighted: the per-fold column sums / X'y / sum x^2 ride in the Gram launch (diagonal-tile CTAs); weighted: a
+    // separate sweep per fold (the Gram launch's statistics are unweighted)
+    if (!weighted) gram_launch(cx, Xs.p, npad, p, npad, segs, F, nullptr, nullptr, G, false, ys.p, stats);
+    else gram_launch(cx, Xs.p, npad, p, npad, segs, F, nullptr, ws.p, G, false);
     const size_t t_c = tm.start(&cx.st.ms_colstats);
     for (int k = 0; k < F; ++k) {
         const int64_t len = off[k + 1] - off[k];
         if (len > 0) {
-            if (!fused_stats)
-                colstats_launch(cx, Xs.p + off[k], len, p, npad, weighted ? ws.p + off[k] : nullptr,
-                                (weighted ? yws.p : ys.p) + off[k], nullptr, stats + (size_t)k * 3 * p, false);
+            if (weighted)
+                colstats_launch(cx, Xs.p + off[k], len, p, npad, ws.p + off[k], yws.p + off[k], nullptr,
+                                stats + (size_t)k * 3 * p, false);
             vecsum_launch(cx, (weighted ? yws.p : ys.p) + off[k], len, 0.0, ysum + (size_t)k * 2, false);
         } else {
-            if (!fused_stats) OEM_CUDA(cudaMemsetAsync(stats + (size_t)k * 3 * p, 0, 3 * (size_t)p * 8, cx.stream));
+            if (weighted) OEM_CUDA(cudaMemsetAsync(stats + (size_t)k * 3 * p, 0, 3 * (size_t)p * 8, cx.stream));
             OEM_CUDA(cudaMemsetAsync(ysum + (size_t)k * 2, 0, 16, cx.stream));
         }
     }

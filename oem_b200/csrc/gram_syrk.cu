@@ -26,7 +26,6 @@
 // no atomics) and mirrors the lower triangle.
 #include <algorithm>
 #include <functional>
-#include <cstdlib>
 #include <type_traits>
 #include <mutex>
 #include "runtime.h"
@@ -57,7 +56,8 @@ struct GramTile {
 // STATS: the diagonal-tile CTAs also accumulate, for the 128 columns of their panel, sum x and sum x*y over the item's
 // rows (the column sweeps of src/oem_big.h:743-837; sum x^2 is the Gram's own diagonal) from the A fragments they load
 // anyway: warp w owns atom rows w and 15-w, so the 8 warps cover the panel's 16 column atoms exactly once.  A separate
-// HBM sweep of X (colstats_kernel) is no longer needed.
+// HBM sweep of X (colstats_kernel) is no longer needed.  The statistics are those of the raw columns: STATS excludes
+// CENTER and WEIGHT (gram_launch refuses the combinations).
 template <bool CENTER, bool WEIGHT, bool USE_TMA, bool STATS>
 __global__ void __launch_bounds__(G_THREADS, 1)
 gram_syrk_kernel(const __grid_constant__ CUtensorMap tmap, const double *__restrict__ X, long long ld,
@@ -305,10 +305,8 @@ gram_syrk_kernel(const __grid_constant__ CUtensorMap tmap, const double *__restr
                 if (CENTER) { alo -= mlo; ahi -= mhi; }
                 if (STATS) {
                     // rows past the item's end only occur in the matrix's last k-tile, where the loader zero-fills them
-                    // (centred: they hold -mean there and are masked like the B operand below)
-                    const double xl = (CENTER && !valid) ? 0.0 : alo, xh = (CENTER && !valid) ? 0.0 : ahi;
-                    st_lo[0] += xl; st_lo[1] = fma(xl, yv[ks], st_lo[1]);         // sum x^2 is the Gram's own diagonal
-                    st_hi[0] += xh; st_hi[1] = fma(xh, yv[ks], st_hi[1]);
+                    st_lo[0] += alo; st_lo[1] = fma(alo, yv[ks], st_lo[1]);       // sum x^2 is the Gram's own diagonal
+                    st_hi[0] += ahi; st_hi[1] = fma(ahi, yv[ks], st_hi[1]);
                 }
                 if (WEIGHT) { alo *= wv[ks]; ahi *= wv[ks]; }
 #pragma unroll
@@ -436,6 +434,7 @@ void gram_launch(Ctx &cx, const double *X, int64_t n, int q, int64_t ld, const s
                  int nout, const double *mean, const double *roww, double *G, bool accumulate, const double *stats_y,
                  double *stats_out) {
     if (stats_out && roww) fail(OEMB200_EINVAL, "gram: fused column statistics are not available with row weights");
+    if (stats_out && mean) fail(OEMB200_EINVAL, "gram: fused column statistics are not available with centring");
     if (n <= 0 || q <= 0) fail(OEMB200_EINVAL, "gram: empty matrix (n=%lld, p=%d)", (long long)n, q);
     if (n >= (1ll << 31)) fail(OEMB200_EINVAL, "gram: more than 2^31-1 rows per call; shard or chunk the rows");
     const int P = (q + G_TILE - 1) / G_TILE;
@@ -453,58 +452,53 @@ void gram_launch(Ctx &cx, const double *X, int64_t n, int q, int64_t ld, const s
     }
     // Row-chunk length: a few waves of items, chosen by simulating the block scheduler (items in launch order onto the
     // earliest free SM) with the three tile-class costs, so that the class sizes divide well over the SMs and the tail
-    // of cheap diagonal items is short.  OEMB200_GRAM_WAVES pins the old "waves x SMs / tiles" rule for experiments.
+    // of cheap diagonal items is short.
     const int64_t min_rows = 32 * G_KT;
     auto round_chunk = [&](int64_t target_chunks) {
         int64_t cr = (rows_total + target_chunks - 1) / std::max<int64_t>(1, target_chunks);
         return std::max<int64_t>(min_rows, ((cr + G_KT - 1) / G_KT) * G_KT);
     };
-    int64_t chunk_rows;
-    if (const char *e = getenv("OEMB200_GRAM_WAVES")) {
-        chunk_rows = round_chunk(std::max<int64_t>(1, (int64_t)std::max(1, atoi(e)) * cx.num_sms / ntile_pairs));
-    } else {
-        const bool partial = (q % G_TILE) != 0;
-        const int nfull = partial ? (P - 1) * (P - 2) / 2 : P * (P - 1) / 2;       // tiles per class
-        const int nlast = partial ? P - 1 : 0;
-        const double cost_last = partial ? (8.0 + std::max(0, std::min(8, (q - (P - 1) * G_TILE - 64 + 7) / 8)) +
-                                            std::min(8, (q - (P - 1) * G_TILE + 7) / 8) - 8.0) / 16.0 : 1.0;
-        const double cost_diag = stats_out ? 0.60 : 0.54;
-        auto makespan = [&](int64_t cr) {
-            std::vector<double> cost;      // launch order: class by class, chunk-major
-            std::vector<double> len;       // k-tiles (+3 for pipeline fill / epilogue) of every chunk
-            for (auto &sg : segs) {
-                const int64_t l = sg.row1 - sg.row0;
-                if (l <= 0) continue;
-                const int64_t nc = (l + cr - 1) / cr;
-                const int64_t per = (((l + nc - 1) / nc) + G_KT - 1) / G_KT * G_KT;
-                for (int64_t r = 0; r < l; r += per) len.push_back((double)((std::min(l, r + per) - r + G_KT - 1) / G_KT) + 3.0);
-            }
-            for (double c : {1.0, cost_last, cost_diag}) {
-                const int nt = c == 1.0 ? nfull : (c == cost_diag ? P : nlast);
-                for (double l : len)
-                    for (int t = 0; t < nt; ++t) cost.push_back(l * c);
-            }
-            std::vector<double> sm(cx.num_sms, 0.0);       // min-heap of SM free times
-            std::make_heap(sm.begin(), sm.end(), std::greater<double>());
-            double end = 0.0;
-            for (double c : cost) {
-                std::pop_heap(sm.begin(), sm.end(), std::greater<double>());
-                sm.back() += c;
-                end = std::max(end, sm.back());
-                std::push_heap(sm.begin(), sm.end(), std::greater<double>());
-            }
-            return end;
-        };
-        const int64_t c_lo = std::max<int64_t>(1, (int64_t)6 * cx.num_sms / ntile_pairs);
-        const int64_t c_hi = std::max<int64_t>(c_lo, (int64_t)14 * cx.num_sms / ntile_pairs);
-        chunk_rows = round_chunk(c_lo);
-        double best = makespan(chunk_rows);
-        for (int64_t c = c_lo + 1; c <= c_hi; ++c) {
-            const int64_t cr = round_chunk(c);
-            if (cr == chunk_rows) continue;
-            const double m = makespan(cr);
-            if (m < best * 0.999) { best = m; chunk_rows = cr; }
+    const bool partial = (q % G_TILE) != 0;
+    const int nfull = partial ? (P - 1) * (P - 2) / 2 : P * (P - 1) / 2;       // tiles per class
+    const int nlast = partial ? P - 1 : 0;
+    const double cost_last = partial ? (8.0 + std::max(0, std::min(8, (q - (P - 1) * G_TILE - 64 + 7) / 8)) +
+                                        std::min(8, (q - (P - 1) * G_TILE + 7) / 8) - 8.0) / 16.0 : 1.0;
+    const double cost_diag = stats_out ? 0.60 : 0.54;
+    auto makespan = [&](int64_t cr) {
+        std::vector<double> cost;      // launch order: class by class, chunk-major
+        std::vector<double> len;       // k-tiles (+3 for pipeline fill / epilogue) of every chunk
+        for (auto &sg : segs) {
+            const int64_t l = sg.row1 - sg.row0;
+            if (l <= 0) continue;
+            const int64_t nc = (l + cr - 1) / cr;
+            const int64_t per = (((l + nc - 1) / nc) + G_KT - 1) / G_KT * G_KT;
+            for (int64_t r = 0; r < l; r += per) len.push_back((double)((std::min(l, r + per) - r + G_KT - 1) / G_KT) + 3.0);
         }
+        for (double c : {1.0, cost_last, cost_diag}) {
+            const int nt = c == 1.0 ? nfull : (c == cost_diag ? P : nlast);
+            for (double l : len)
+                for (int t = 0; t < nt; ++t) cost.push_back(l * c);
+        }
+        std::vector<double> sm(cx.num_sms, 0.0);       // min-heap of SM free times
+        std::make_heap(sm.begin(), sm.end(), std::greater<double>());
+        double end = 0.0;
+        for (double c : cost) {
+            std::pop_heap(sm.begin(), sm.end(), std::greater<double>());
+            sm.back() += c;
+            end = std::max(end, sm.back());
+            std::push_heap(sm.begin(), sm.end(), std::greater<double>());
+        }
+        return end;
+    };
+    const int64_t c_lo = std::max<int64_t>(1, (int64_t)6 * cx.num_sms / ntile_pairs);
+    const int64_t c_hi = std::max<int64_t>(c_lo, (int64_t)14 * cx.num_sms / ntile_pairs);
+    int64_t chunk_rows = round_chunk(c_lo);
+    double best = makespan(chunk_rows);
+    for (int64_t c = c_lo + 1; c <= c_hi; ++c) {
+        const int64_t cr = round_chunk(c);
+        if (cr == chunk_rows) continue;
+        const double m = makespan(cr);
+        if (m < best * 0.999) { best = m; chunk_rows = cr; }
     }
     // cap the workspace at ~1.5 GB of partial tiles
     const int64_t max_slots = (1536ll << 20) / (G_TILE * G_TILE * 8);
@@ -541,14 +535,13 @@ void gram_launch(Ctx &cx, const double *X, int64_t n, int q, int64_t ld, const s
     // class (row-range-major inside a class) makes the tiles of a row range start together and stream the same rows at
     // the same time -- that is what lets them share column panels through L2.  Mixed classes drift apart within a wave
     // and re-read the panels from HBM (measured 5.6x the matrix; class-major order: see profiles/gram_traffic.json).
-    const bool partial_last = (q % G_TILE) != 0;
     for (int cls = 0; cls < 3; ++cls)
         for (size_t ci = 0; ci < chunks.size(); ++ci) {
             const Chunk &c = chunks[ci];
             int tp = 0;
             for (int pi = 0; pi < P; ++pi)
                 for (int pj = 0; pj <= pi; ++pj, ++tp) {
-                    const int tcls = pi == pj ? 2 : (partial_last && pi == P - 1) ? 1 : 0;
+                    const int tcls = pi == pj ? 2 : (partial && pi == P - 1) ? 1 : 0;
                     if (tcls != cls) continue;
                     GramItem it;
                     it.pi = pi; it.pj = pj; it.pad = (int)ci;
@@ -613,8 +606,7 @@ void gram_launch(Ctx &cx, const double *X, int64_t n, int q, int64_t ld, const s
 #define OEM_GRAM_DISPATCH(CC, WW, SS)                                                                               \
     if (use_tma) launch_variant<CC, WW, true, SS>(cx, tm, X, ld, n, q, d_items.p, ni, mean, roww, ws.p, stats_y, stats_ws.p, P);  \
     else launch_variant<CC, WW, false, SS>(cx, tm, X, ld, n, q, d_items.p, ni, mean, roww, ws.p, stats_y, stats_ws.p, P)
-    if (stats_out && C) { OEM_GRAM_DISPATCH(true, false, true); }
-    else if (stats_out) { OEM_GRAM_DISPATCH(false, false, true); }
+    if (stats_out) { OEM_GRAM_DISPATCH(false, false, true); }
     else if (C && W) { OEM_GRAM_DISPATCH(true, true, false); }
     else if (C) { OEM_GRAM_DISPATCH(true, false, false); }
     else if (W) { OEM_GRAM_DISPATCH(false, true, false); }

@@ -24,7 +24,6 @@
 // Only the per-CTA column sums leave the SM; ls_sum_partials adds them in fixed order, so the pass is
 // bit-reproducible for a given grid.
 #include <algorithm>
-#include <cstdlib>
 #include "runtime.h"
 
 namespace oemb200 {
@@ -249,18 +248,16 @@ slab_relayout_kernel(const double *__restrict__ X, long long n, int p, long long
     }
 }
 
-// Shape of the pass for a given p: rows per slab, columns per thread, threads per CTA, CTAs per SM.  Default up to
-// p = 1024: two CTAs of 256 threads per SM, each with its own ring of three <= 32 KB slabs -- two independent pipelines
-// per SM hide the per-slab reduction latency (measured on a B200, 16 GB: 2.36 ms against 2.43 ms with one 512-thread CTA
-// and 64 KB slabs at p = 1000; 1.20 against 1.45 ms at p = 500).  OEMB200_SLAB_CTAS=1 selects the one-CTA shape, which is
-// also the only one for 1024 < p <= 2048.
+// Shape of the pass for a given p: rows per slab, columns per thread, threads per CTA, CTAs per SM.  Up to p = 1024: two
+// CTAs of 256 threads per SM, each with its own ring of three <= 32 KB slabs -- two independent pipelines per SM hide the
+// per-slab reduction latency (measured on a B200, 16 GB: 2.36 ms against 2.43 ms with one 512-thread CTA and 64 KB slabs
+// at p = 1000; 1.20 against 1.45 ms at p = 500).  For 1024 < p <= 2048, one CTA of 512 threads per SM.
 struct SlabShape { int rt, nc, threads, ctas; };
 static SlabShape slab_shape(int p) {
     SlabShape z{0, 0, 0, 0};
     if (p < 8 || p > 2048) return z;
-    static const bool two = [] { const char *e = getenv("OEMB200_SLAB_CTAS"); return !(e && e[0] == '1'); }();
-    if (p <= 512) return two ? SlabShape{8, (p + 255) / 256, 256, 2} : SlabShape{16, 1, 512, 1};
-    if (p <= 1024) return two ? SlabShape{4, (p + 255) / 256, 256, 2} : SlabShape{8, 2, 512, 1};
+    if (p <= 512) return SlabShape{8, (p + 255) / 256, 256, 2};
+    if (p <= 1024) return SlabShape{4, (p + 255) / 256, 256, 2};
     return SlabShape{4, (p + 511) / 512, 512, 1};
 }
 
@@ -300,7 +297,7 @@ void logit_slab_launch(Ctx &cx, const double *slabs, int64_t n, int p, const dou
     const int rt = sh.rt;
     void *kern = nullptr;
 #define LS_PICK(R, N, T) if (rt == R && sh.nc == N && sh.threads == T) kern = (void *)logit_slab_kernel<R, N, T>
-    LS_PICK(16, 1, 512); LS_PICK(8, 2, 512); LS_PICK(4, 3, 512); LS_PICK(4, 4, 512);
+    LS_PICK(4, 3, 512); LS_PICK(4, 4, 512);
     LS_PICK(8, 1, 256); LS_PICK(8, 2, 256); LS_PICK(4, 3, 256); LS_PICK(4, 4, 256);
 #undef LS_PICK
     if (!kern) fail(OEMB200_EINVAL, "slab route: no kernel for p = %d", p);

@@ -1533,8 +1533,8 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
 
     // ---- small coordinate-wise problems: register-resident variant (d comes from a Lanczos-only generic launch) ----
     {
-        bool reg_ok = getenv("OEMB200_PATH_GENERIC") == nullptr && q <= 256 && !pp.accelerate && !pp.post_scale &&
-                      !pp.beta_init && !pp.beta_final && !pp.skip && !pp.irls_conv && max_ct <= PR_MAXCT && !pp.chains.empty();
+        bool reg_ok = q <= 256 && !pp.accelerate && !pp.post_scale && !pp.beta_init && !pp.beta_final && !pp.skip &&
+                      !pp.irls_conv && max_ct <= PR_MAXCT && !pp.chains.empty();
         for (auto &c : pp.chains) reg_ok = reg_ok && c.penalty < OEMB200_PEN_GRP_LASSO;
         const int NC = q <= 128 ? 1 : (q + 31) / 32;
         const int QP = q <= 128 ? 128 : 256;
@@ -1610,11 +1610,7 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
     const int q4 = (q + 3) / 4 * 4;
     const int qs = q4 + (((4 - q4) % 16) + 16) % 16;      // smallest value >= roundup(q,4) that is 4 (mod 16)
     const int ng = pp.ngroups, ngidx = ng ? pp.ngidx : 0;
-    auto fixed_for = [&](int nbuf) {
-        (void)nbuf;     // two ping-pong buffers in every mode
-        return path_fixed_smem_bytes(q, max_ct, pp.Lmax, ng, ngidx, pp.post_scale != nullptr);
-    };
-    size_t fixed_bytes = fixed_for(1);
+    const size_t fixed_bytes = path_fixed_smem_bytes(q, max_ct, pp.Lmax, ng, ngidx, pp.post_scale != nullptr);
     const size_t smem_cap = cx.smem_optin;
     if (fixed_bytes > smem_cap)
         fail(OEMB200_EUNSUPPORTED, "path: q=%d with %d chains per Gram and %d lambdas exceeds shared memory", q, max_ct, pp.Lmax);
@@ -1627,8 +1623,8 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
     else {
         int cs = 0;
         for (int c : {8, 4, 2})      // more members = less mat-vec work each; the cluster barrier costs the same
-            if (slice_bytes(c) + fixed_for(2) <= smem_cap && (q + c - 1) / c >= 16) { cs = c; break; }
-        if (cs && G * cs <= cx.num_sms) { mode = MODE_CLUSTER; team = cs; fixed_bytes = fixed_for(2); }
+            if (slice_bytes(c) + fixed_bytes <= smem_cap && (q + c - 1) / c >= 16) { cs = c; break; }
+        if (cs && G * cs <= cx.num_sms) { mode = MODE_CLUSTER; team = cs; }
         else { mode = MODE_GLOBAL; team = 0; }
     }
     void *kern = mode == MODE_SINGLE ? (void *)oem_path_kernel<MODE_SINGLE, 0>
@@ -1651,10 +1647,6 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
         const int max_ctas = std::max(1, per_sm) * cx.num_sms;
         if (G > max_ctas) fail(OEMB200_EUNSUPPORTED, "path: %d Grams exceed the %d co-resident CTAs", G, max_ctas);
         team = std::max(1, std::min(max_ctas / G, (q + 7) / 8));       // at least one 8-column MMA atom per member
-        if (const char *e = getenv("OEMB200_PATH_MIN_CPC")) {          // experiment: fewer, fatter members (exchange traffic ~ team size)
-            const int mc = std::max(8, atoi(e));
-            team = std::max(1, std::min(team, (q + mc - 1) / mc));
-        }
     }
     int cpc = (q + team - 1) / team;
     if (mode == MODE_GLOBAL) {
@@ -1664,7 +1656,7 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
     const int cpc_pad = (cpc + 7) / 8 * 8;
     // one 8-column atom per member and <= 4 chains: the register-resident mat-vec (matvec_reg)
     int rpt = 0;
-    if (mode == MODE_GLOBAL && cpc_pad == 8 && max_ct <= 4 && qs <= 5 * PK_THREADS && getenv("OEMB200_PATH_DMMA") == nullptr) {
+    if (mode == MODE_GLOBAL && cpc_pad == 8 && max_ct <= 4 && qs <= 5 * PK_THREADS) {
         rpt = std::max(2, (qs + PK_THREADS - 1) / PK_THREADS);
         void *kr = rpt == 2 ? (void *)oem_path_kernel<MODE_GLOBAL, 2> : rpt == 3 ? (void *)oem_path_kernel<MODE_GLOBAL, 3>
                  : rpt == 4 ? (void *)oem_path_kernel<MODE_GLOBAL, 4> : (void *)oem_path_kernel<MODE_GLOBAL, 5>;

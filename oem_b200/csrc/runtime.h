@@ -24,19 +24,17 @@ struct PhaseTimers {
     struct Rec { cudaEvent_t a, b; double *acc; };
     std::vector<Rec> recs;
     cudaStream_t s;
-    bool off = getenv("OEMB200_NO_PHASE_TIMERS") != nullptr;   // experiment: what do the event records themselves cost?
     explicit PhaseTimers(cudaStream_t s_) : s(s_) {}
     PhaseTimers(const PhaseTimers &) = delete;
     ~PhaseTimers() { for (auto &r : recs) { event_release(r.a); event_release(r.b); } }
     size_t start(double *acc) {
-        if (off) return 0;
         Rec r; r.acc = acc;
         r.a = event_acquire(); r.b = event_acquire();
         OEM_CUDA(cudaEventRecord(r.a, s));
         recs.push_back(r);
         return recs.size() - 1;
     }
-    void stop(size_t i) { if (!off) OEM_CUDA(cudaEventRecord(recs[i].b, s)); }
+    void stop(size_t i) { OEM_CUDA(cudaEventRecord(recs[i].b, s)); }
     void collect() {   // call after the stream is synchronized
         for (auto &r : recs) {
             float ms = 0.f;
@@ -158,8 +156,8 @@ bool comm_can_skip(const oemb200_comm *c, int64_t count);
 struct RowSegment { int64_t row0, row1; int out; };   // rows [row0,row1) accumulate into Gram #out
 // G[out] (q x q col-major, full symmetric; nout matrices, stride q*q) (+)= X_seg' diag(w) X_seg with
 // optional column centring.  Segment boundaries must be multiples of 36 rows except at n.
-// stats_out (optional, not with row weights): nout x 3 x q = [sum xs, sum xs*stats_y, sum xs^2] (xs = x - mean) per output, in the layout of
-// colstats_launch, accumulated by the diagonal-tile CTAs of the same launch (stats_y may be NULL: sum x*y = 0)
+// stats_out (optional, not with row weights or centring): nout x 3 x q = [sum x, sum x*stats_y, sum x^2] per output, in the
+// layout of colstats_launch, accumulated by the diagonal-tile CTAs of the same launch (stats_y may be NULL: sum x*y = 0)
 void gram_launch(Ctx &cx, const double *X, int64_t n, int q, int64_t ld, const std::vector<RowSegment> &segs,
                  int nout, const double *mean, const double *roww, double *G, bool accumulate,
                  const double *stats_y = nullptr, double *stats_out = nullptr);

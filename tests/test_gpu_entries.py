@@ -465,19 +465,6 @@ def test_dense_n_le_p_branch(lib, oracle, n, p, standardize, intercept):
     assert_same_fit(got, ref)
 
 
-@pytest.mark.parametrize("standardize,intercept", [(True, True), (False, True), (False, False)])
-@pytest.mark.parametrize("n,p", [(5000, 37), (20011, 300)])
-def test_dense_fused_centred_column_statistics(lib, oracle, monkeypatch, n, p, standardize, intercept):
-    # OEMB200_FUSED_COLSTATS=1: oem_fit_dense takes X'y and the centred sums of squares from the Gram launch's diagonal
-    # CTAs (opt-in: measured slower than the separate sweep for this entry); ragged n exercises the masked last k-tile
-    monkeypatch.setenv("OEMB200_FUSED_COLSTATS", "1")
-    X, y = gaussian_problem(900 + p, n, p, mean_x=1.5, sd_x=2.0)
-    a = args_xy(X, y, "gaussian", ["lasso", "mcp"], nlambda=15, standardize=standardize, intercept=intercept,
-                opts=dict(tol=1e-9))
-    got, ref = lib.oem_fit_dense(*a), oracle.oem_fit_dense(*a)
-    assert_same_fit(got, ref)
-
-
 def test_wide_problem_streams_A_from_l2(lib, oracle):
     # q = 2400: a member's column slice of A (24 x 2404 doubles) no longer fits shared memory next to the iterate
     # buffers, so the path kernel streams its slice from L2 (a_in_smem = false) -- same answers

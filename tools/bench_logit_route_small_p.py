@@ -24,7 +24,7 @@ for n, p in ((50000, 8), (50000, 16), (50000, 32), (50000, 64), (1000000, 16), (
     out["n=%%d p=%%d" %% (n, p)] = round(best * 1e3, 2)
 print(json.dumps(out))
 ''' % ROOT
-for m in ("8", "128"):
-    env = dict(os.environ, OEMB200_SLAB_MIN_P=m)
+for route in ("slab", "sweeps"):
+    env = dict(os.environ, OEMB200_LOGIT_ROUTE=route)
     r = subprocess.run([sys.executable, "-c", CHILD], env=env, capture_output=True, text=True)
-    print("slab_min_p", m, r.stdout.strip().splitlines()[-1] if r.stdout.strip() else r.stderr[-400:])
+    print("route", route, r.stdout.strip().splitlines()[-1] if r.stdout.strip() else r.stderr[-400:])

@@ -1,5 +1,5 @@
 """Where does a logistic fit at an 8-GPU shard size (n = 2.5e5 x 1000 on one GPU) spend its wall time?  A/B of the driver's
-knobs: legacy default stream vs an explicit stream, one-ahead speculation on / off, phase timers on / off."""
+knobs: legacy default stream vs an explicit stream, one-ahead speculation on / off."""
 import json
 import os
 import sys
@@ -21,10 +21,8 @@ y = (torch.rand(n, generator=g, dtype=torch.float64, device=dev) < torch.sigmoid
 X = Xt.t()
 stream = torch.cuda.Stream()
 for label, env, use_stream in (("legacy stream", {}, False), ("explicit stream", {}, True),
-                               ("explicit, no speculation", {"OEMB200_IRLS_NO_SPECULATION": "1"}, True),
-                               ("explicit, no phase timers", {"OEMB200_NO_PHASE_TIMERS": "1"}, True)):
-    for k in ("OEMB200_IRLS_NO_SPECULATION", "OEMB200_NO_PHASE_TIMERS"):
-        os.environ.pop(k, None)
+                               ("explicit, no speculation", {"OEMB200_IRLS_NO_SPECULATION": "1"}, True)):
+    os.environ.pop("OEMB200_IRLS_NO_SPECULATION", None)
     os.environ.update(env)
     opts = dict(maxit=500, tol=1e-7)
     if use_stream:

@@ -139,24 +139,4 @@ void scale_sym_launch(Ctx &cx, int p, const double *sinv, const double *XXin, co
     cx.st.kernel_launches += 1;
 }
 
-// y[r] = sum_c M[r + c*q] x[c]   (q x q col-major, symmetric use) + add[r]: the logistic
-// XY = XX * beta + grad step (src/oem_logistic_dense.h:999).  One warp per row.
-__global__ void symv_add_kernel(int q, const double *__restrict__ M, const double *__restrict__ x,
-                                const double *__restrict__ add, double *__restrict__ y) {
-    const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (r >= q) return;
-    const int lane = threadIdx.x & 31;
-    double s = 0.0;
-    for (int c = lane; c < q; c += 32) s = fma(M[(size_t)r * q + c], x[c], s);   // row r == column r (symmetric)
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) y[r] = s + (add ? add[r] : 0.0);
-}
-
-void symv_add_launch(Ctx &cx, int q, const double *M, const double *x, const double *add, double *y) {
-    symv_add_kernel<<<(q + 7) / 8, 256, 0, cx.stream>>>(q, M, x, add, y);
-    OEM_CUDA(cudaGetLastError());
-    cx.st.kernel_launches += 1;
-}
-
 }  // namespace oemb200

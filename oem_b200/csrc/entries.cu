@@ -929,7 +929,7 @@ int oemb200_top_eig(const double *xx_dev, int q, double *lambda_max_out, int *st
         xy.zero(cx.stream);
         PathProblem pp;
         pp.q = q; pp.ngram = 1; pp.XX = xx_dev; pp.XY = xy.p; pp.d = d.p; pp.compute_eig = true;
-        pp.eig_factor = 1.0; pp.eig_tol = 1e-10; pp.Lmax = 1; pp.lanczos_steps = lz.p;
+        pp.eig_factor = 1.0; pp.Lmax = 1; pp.lanczos_steps = lz.p;
         path_launch(cx, pp);
         double h; int k;
         d.download(&h, 1, cx.stream);

@@ -1,19 +1,19 @@
-// entry_logistic.cu -- host driver of oem_fit_logistic_dense (src/oem_logistic_dense.cpp:29-313,
-// solver src/oem_logistic_dense.h:721-1036) on the sm_100a kernels.
+// entry_logistic.cu -- host drivers of oem_fit_logistic_dense (src/oem_logistic_dense.cpp:29-313, solver
+// src/oem_logistic_dense.h:721-1036) and oem_fit_logistic_sparse (below) on the sm_100a kernels.
 //
 // Per IRLS iteration the reference makes two passes over X:
 //   prob = sigma(X (beta o w) + beta0)        (oem_logistic_dense.h:864-949)
 //   grad = [sum(y-prob), X'(y-prob) o w] / n  (oem_logistic_dense.h:970-992)
 // Here both come out of ONE sweep of a row-slab copy of X (logit_slab.cu; built once per fit), or, for shapes the
 // slab kernel does not cover, out of the two HBM-bound sweeps xb_kernel + colstats_kernel.  When the Hessian bound is
-// (re)built, X'WX runs on the FP64 tensor pipe with the row weight fused into the fragment load
-// (gram_syrk_kernel<WEIGHT>) and the Lanczos eigenvalue inside the path kernel.
+// (re)built, X'WX runs on the FP64 tensor pipe (gram_syrk_kernel; the row weight fused into the fragment load for
+// hessian.type = "full") and the Lanczos eigenvalue inside the path kernel.
 //
 // The IRLS state never leaves the device.  An iteration of the dense driver is three launches on one stream: the data pass
 // (+ its partial-sum kernel), in row-sharded runs the sum of the (p+1)-vector gradient (comm.cu), and the path launch, which
-// forms XY = XX beta + grad from the XX slice its members load anyway, runs the inner OEM loop, applies the outer stop rule
-// and leaves the next pass's coefficients (PathProblem::xy_grad / irls_*); their phase clocks are kept on the device.  The
-// only host round trip per IRLS iteration is ONE event synchronisation that reads the stop-rule flag from pinned memory,
+// forms XY = XX beta + grad, runs the inner OEM loop, applies the outer stop rule and leaves the next pass's coefficients
+// (irls_path_problem); their phase clocks are kept on the device.  The only host round trip per IRLS iteration is ONE
+// event synchronisation that reads the stop-rule verdict from pinned memory (IrlsLoop, shared with the sparse driver),
 // and it is hidden behind the next iteration, which is enqueued one ahead and predicated on the device-side verdict.
 // The reference's quirks are kept (SURVEY.md Appendix B item 5): the data pass is skipped on the first IRLS
 // iteration of a warm lambda, W is clamped at index = IRLS counter, eigen factor 1.0005.
@@ -67,26 +67,6 @@ double logistic_loss(Ctx &cx, const double *y, const double *prob, int64_t n) {
     return h[0];
 }
 
-// per-block min / max of v (partial[2 b], partial[2 b + 1]); the host folds the blocks
-__global__ void __launch_bounds__(256) minmax_kernel(const double *__restrict__ v, long long n, double *__restrict__ partial) {
-    double lo = INFINITY, hi = -INFINITY;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const double x = v[i];
-        lo = fmin(lo, x); hi = fmax(hi, x);
-    }
-    __shared__ double slo[8], shi[8];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        lo = fmin(lo, __shfl_xor_sync(0xffffffffu, lo, o));
-        hi = fmax(hi, __shfl_xor_sync(0xffffffffu, hi, o));
-    }
-    if ((threadIdx.x & 31) == 0) { slo[threadIdx.x >> 5] = lo; shi[threadIdx.x >> 5] = hi; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        for (int w = 1; w < 8; ++w) { lo = fmin(lo, slo[w]); hi = fmax(hi, shi[w]); }
-        partial[2 * blockIdx.x] = lo; partial[2 * blockIdx.x + 1] = hi;
-    }
-}
 __global__ void scale_inplace_kernel(double *v, size_t n, double f) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) v[i] *= f;
@@ -106,43 +86,6 @@ __global__ void irls_pack_grad_kernel(const double *__restrict__ xr, const doubl
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j < p) g[1 + j] = xr[j];
     if (j == 0) g[0] = sr[0];
-}
-
-// stopRule(beta_new, beta_prev, irls_tol) (src/utils.cpp:537-549) on the device; the verdict goes to pinned host
-// memory, the inner loop's iteration count is accumulated for the statistics.  One CTA.
-// `conv` (device) is the predicate of speculatively enqueued work: once an IRLS loop has converged, every later kernel
-// of that lambda -- this one included -- returns at once, so the host may enqueue iteration it + 1 before it has read
-// iteration it's verdict.
-// With `b` given it also prepares the NEXT data pass: b = beta_new[icpt:] o colsq_inv, b0 = beta_new[0] (what
-// irls_coef_kernel computes).  The dense driver no longer launches this kernel -- the same steps are the last thing its
-// path launch does (oem_path_kernel, "IRLS epilogue") -- the sparse driver does.
-__global__ void irls_stop_kernel(const double *__restrict__ cur, const double *__restrict__ prev, int q, double tol,
-                                 const int *__restrict__ niter, long long *__restrict__ iters_total,
-                                 volatile int *__restrict__ host_flag, int *__restrict__ conv,
-                                 const double *__restrict__ cinv = nullptr, int p = 0, int icpt = 0, double *__restrict__ b = nullptr,
-                                 double *__restrict__ b0 = nullptr) {
-    if (conv && *conv) return;
-    if (b) {
-        for (int j = threadIdx.x; j < p; j += blockDim.x) b[j] = cinv ? cur[icpt + j] * cinv[j] : cur[icpt + j];
-        if (threadIdx.x == 0) *b0 = icpt ? cur[0] : 0.0;
-    }
-    __shared__ int bad;
-    if (threadIdx.x == 0) bad = 0;
-    __syncthreads();
-    int v = 0;
-    for (int i = threadIdx.x; i < q; i += blockDim.x) {
-        const double ac = fabs(cur[i]), ap = fabs(prev[i]);
-        if ((ac > 1e-13 && ap <= 1e-13) || (ac <= 1e-13 && ap > 1e-13)) v = 1;
-        else if (ac > 1e-13 && ap > 1e-13 && fabs((cur[i] - prev[i]) / prev[i]) > tol) v = 1;
-    }
-    if (v) bad = 1;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        *iters_total += niter[0];
-        if (conv && !bad) *conv = 1;
-        *host_flag = bad ? 0 : 1;
-        __threadfence_system();
-    }
 }
 
 namespace {
@@ -168,6 +111,61 @@ std::vector<double> logistic_cinv(const std::vector<double> &h0, int p, double n
         }
     return cinv;
 }
+
+// The outer IRLS loop of one lambda (src/oem_logistic_dense.h:1000-1035) around a driver's enqueue(k, verdict), which puts
+// iteration k of the lambda on the stream: it starts from the iterate in slot (par0 + k) & 1, writes the other slot, and
+// its path launch writes the stop rule's verdict to *verdict and to the device flag that predicates every later kernel of
+// the lambda.  The host's one round trip per iteration is an event wait and a read of that verdict.  With `speculate`
+// iteration k + 1 is enqueued before iteration k's verdict is read, so the GPU never waits for the host (the gap was
+// ~100 us per iteration: 5 % of a dense fit on one GPU, 25 % row-sharded over eight); an iteration enqueued after
+// convergence is a few empty launches, and its counters are rolled back.  Only a driver whose every kernel of the chain
+// can be predicated may speculate.
+struct IrlsLoop {
+    bool speculate;
+    PinnedFlags flag{4};                  // verdict slots: the host reads slot (gi & 3) after that iteration's event
+    cudaEvent_t ev[2] = {event_acquire(), event_acquire()};
+    long long gi = 0;                     // global IRLS iteration counter (verdict slot = gi & 3, event = gi & 1)
+    explicit IrlsLoop(bool speculate_) : speculate(speculate_) {}
+    IrlsLoop(const IrlsLoop &) = delete;
+    ~IrlsLoop() { event_release(ev[0]); event_release(ev[1]); }
+
+    // Returns niter as the reference reports it: executed iterations + 1 on convergence, irls_maxit + 1 at the cap.  par0
+    // moves to the slot of the iterate the last EXECUTED iteration wrote.
+    template <typename F>
+    int run(Ctx &cx, int irls_maxit, int &par0, F &&enqueue_iteration) {
+        auto enqueue = [&](int k) {
+            enqueue_iteration(k, flag.p + (gi & 3));
+            OEM_CUDA(cudaEventRecord(ev[gi & 1], cx.stream));
+            ++gi;
+        };
+        int it = 0;
+        bool broke = false;
+        enqueue(0);
+        for (;;) {
+            // iteration `it` is in the stream (event (gi - 1) & 1 if nothing was enqueued after it)
+            const bool ahead = speculate && it + 1 < irls_maxit;
+            const oemb200_stats before = cx.st;
+            if (ahead) enqueue(it + 1);
+            const long long gi_it = gi - 1 - (ahead ? 1 : 0);
+            cx.st.host_syncs += 1;
+            OEM_CUDA(cudaEventSynchronize(ev[gi_it & 1]));
+            if (flag.p[gi_it & 3]) {
+                broke = true;
+                if (ahead) {           // the speculative iteration found the lambda converged: nothing of it ran
+                    cx.st.data_passes = before.data_passes; cx.st.xb_launches = before.xb_launches;
+                    cx.st.gemv_bytes = before.gemv_bytes; cx.st.allreduce_calls = before.allreduce_calls;
+                    cx.st.allreduce_doubles = before.allreduce_doubles;
+                }
+                break;
+            }
+            ++it;
+            if (it >= irls_maxit) { it = irls_maxit - 1; break; }
+            if (!ahead) enqueue(it);
+        }
+        par0 = (par0 + it + 1) & 1;
+        return (broke ? it : irls_maxit) + 1;
+    }
+};
 }  // namespace
 
 void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s,
@@ -275,7 +273,6 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
     DBuf<double> bh(nbh), d_nobs(1);
     d_nobs.upload(&n_tot, 1, cx.stream);
     DBuf<double> gradb(3 * (size_t)p + 2);   // two-sweep route: [stats 3p | sum r, sum r^2]
-    PinnedFlags flag(4);          // verdict slots: the host reads slot (iteration & 3) after that iteration's event
     PathScratches scratch(1);
     wm.mark("setup (stats, slabs, buffers)");
 
@@ -290,16 +287,17 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
     //   [0] data passes (slab kernel start -> end of its partial-sum kernel), [1] scratch, [2] path launches, [3] all-reduces
     DBuf<unsigned long long> d_clk(4);
     d_clk.zero(cx.stream);
+    IrlsModel md;
+    md.XX = d_XX.p; md.XY = d_XY.p; md.d = d_d.p; md.niter = d_niter.p; md.lz = d_lz.p; md.scratch = scratch.s[0];
+    md.conv = d_conv.p; md.iters_total = d_iters_total.p; md.icpt = icpt; md.cinv = cinv_dev; md.b = d_b.p; md.b0 = d_b0.p;
+    md.t_acc = d_clk.p + 2;
     const bool clk_allreduce = cx.comm != nullptr && cx.all_reduce_can_skip((int64_t)p + 1);     // the peer-memory kernel
-    // Speculation: enqueue iteration k + 1 before reading iteration k's verdict, so the GPU never waits for the host round
-    // trip (the gap was ~100 us per iteration: 5 % of the fit on one GPU, 25 % row-sharded over eight).  Possible when every
-    // kernel of the chain can be predicated: slab route, upper-bound Hessian (the Gram launch cannot), and a cross-rank sum
-    // that runs on the peer-memory transport (an NCCL collective cannot be predicated from the device).
+    // Speculation (IrlsLoop) needs every kernel of the chain to be predicated: slab route, upper-bound Hessian (the Gram
+    // launch cannot), and a cross-rank sum that runs on the peer-memory transport (an NCCL collective cannot be predicated
+    // from the device).
     const bool speculate = slab && !o->hessian_full && cx.all_reduce_can_skip((int64_t)p + 1) &&
                            getenv("OEMB200_IRLS_NO_SPECULATION") == nullptr;
-    cudaEvent_t ev_done[2] = {event_acquire(), event_acquire()};
-    struct EvGuard { cudaEvent_t *e; ~EvGuard() { event_release(e[0]); event_release(e[1]); } } ev_guard{ev_done};
-    long long gi = 0;                            // global IRLS iteration counter (verdict slot = gi & 3, event = gi & 1)
+    IrlsLoop loop(speculate);
 
     for (int pp = 0; pp < su.P; ++pp) {
         int par0 = 0;                            // d_iter.p + par0 * q holds the iterate the next iteration starts from
@@ -309,7 +307,7 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
             OEM_CUDA(cudaMemsetAsync(d_conv.p, 0, sizeof(int), cx.stream));
             const int *skip = d_conv.p;
 
-            auto enqueue_iteration = [&](int k) {
+            auto enqueue_iteration = [&](int k, volatile int *verdict) {
                 double *cur = d_iter.p + (size_t)((par0 + k) & 1) * q, *nxt = d_iter.p + (size_t)((par0 + k + 1) & 1) * q;
                 bool rebuilt = false, form_xy = false;
                 if (!(k == 0 && !on_lam_1)) {
@@ -338,28 +336,14 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
                     if (need_w) {
                         // X'WX / n with the intercept border (oem_logistic_dense.h:458-522)
                         double *G = bh.p, *st = G + (size_t)p * p, *ws = st + 3 * (size_t)p;
-                        // The upper-bound Hessian is built at beta = 0, where every W_i is prob (1 - prob) = 0.25 exactly.
-                        // A uniform power-of-two weight commutes with every rounding of the Gram, so X'WX == w0 * X'X to the
-                        // bit, and the unweighted DMMA variant (no multiply in the fragment load: 34.7 against 31 TFLOP/s)
-                        // followed by one scaling pass over p x p gives the identical matrix.  Decided per rank from its own
-                        // rows; the all-reduced bundle has the same shape either way.
-                        double w_uniform = 0.0;
+                        // The upper-bound Hessian is built on the first pass of a penalty, at beta = 0 (b = 0, b0 = 0): every
+                        // row has eta = 0, prob = 1/2 and W = prob (1 - prob) = 1/4 exactly.  A power-of-two weight commutes
+                        // with every rounding of the Gram, so X'WX == X'X / 4 to the bit, and the unweighted DMMA variant (no
+                        // multiply in the fragment load: 34.7 against 31 TFLOP/s) followed by one scaling pass over p x p
+                        // gives the identical matrix.
+                        gram_launch(cx, X.p, n, p, X.ld, {RowSegment{0, n, 0}}, 1, nullptr, o->hessian_full ? d_W.p : nullptr, G, false);
                         if (!o->hessian_full) {
-                            const int nblk = 1024;
-                            DBuf<double> mm(2 * (size_t)nblk);
-                            minmax_kernel<<<nblk, 256, 0, cx.stream>>>(d_W.p, n, mm.p);
-                            cx.st.kernel_launches += 1;
-                            std::vector<double> hmm(2 * (size_t)nblk);
-                            mm.download(hmm.data(), hmm.size(), cx.stream);
-                            cx.sync();
-                            double lo = hmm[0], hi = hmm[1];
-                            for (int b2 = 1; b2 < nblk; ++b2) { lo = std::min(lo, hmm[2 * b2]); hi = std::max(hi, hmm[2 * b2 + 1]); }
-                            int ex = 0;
-                            if (lo == hi && lo > 0.0 && std::frexp(lo, &ex) == 0.5) w_uniform = lo;      // exact power of two
-                        }
-                        gram_launch(cx, X.p, n, p, X.ld, {RowSegment{0, n, 0}}, 1, nullptr, w_uniform > 0.0 ? nullptr : d_W.p, G, false);
-                        if (w_uniform > 0.0 && w_uniform != 1.0) {
-                            scale_inplace_kernel<<<(unsigned)(((size_t)p * p + 255) / 256), 256, 0, cx.stream>>>(G, (size_t)p * p, w_uniform);
+                            scale_inplace_kernel<<<(unsigned)(((size_t)p * p + 255) / 256), 256, 0, cx.stream>>>(G, (size_t)p * p, 0.25);
                             cx.st.kernel_launches += 1;
                         }
                         const size_t tc = tm.start(&cx.st.ms_colstats);
@@ -397,51 +381,12 @@ void fit_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *
                     }
                     form_xy = true;           // XY = XX beta + grad (:999): formed by the path launch below
                 }
-                PathProblem pr = irls_path_problem(tb, su, pp, i, o);
-                pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p; pr.compute_eig = rebuilt;
-                pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
-                pr.scratch = scratch.s[0];
-                pr.skip = skip;
-                if (form_xy) { pr.xy_grad = d_g.p; pr.xy_cinv = cinv_dev; pr.xy_n = n_tot; pr.xy_icpt = icpt; pr.xy_out = d_XY.p; }
-                pr.t_acc = d_clk.p + 2;
-                // the outer loop's stop rule, its verdicts and the next pass's coefficients are the launch's last step
-                pr.irls_conv = d_conv.p; pr.irls_host_flag = flag.p + (gi & 3); pr.irls_iters_total = d_iters_total.p;
-                pr.irls_tol = o->irls_tol; pr.irls_cinv = cinv_dev; pr.irls_p = p; pr.irls_icpt = icpt;
-                pr.irls_b = d_b.p; pr.irls_b0 = d_b0.p;
-                path_launch(cx, pr);
-                OEM_CUDA(cudaEventRecord(ev_done[gi & 1], cx.stream));
-                ++gi;
+                path_launch(cx, irls_path_problem(tb, su, pp, i, o, md, cur, nxt, verdict, rebuilt, form_xy ? d_g.p : nullptr, n_tot));
             };
 
-            int it = 0;
-            bool broke = false;
-            enqueue_iteration(0);
-            for (;;) {
-                // iteration `it` is in the stream (event (gi - 1) & 1 if nothing was enqueued after it)
-                const bool ahead = speculate && it + 1 < o->irls_maxit;
-                const oemb200_stats before = cx.st;
-                if (ahead) enqueue_iteration(it + 1);
-                const long long gi_it = gi - 1 - (ahead ? 1 : 0);
-                cx.st.host_syncs += 1;
-                OEM_CUDA(cudaEventSynchronize(ev_done[gi_it & 1]));          // the one host round trip of the IRLS iteration
-                if (flag.p[gi_it & 3]) {
-                    broke = true;
-                    if (ahead) {           // the speculative iteration found d_conv set: nothing of it ran
-                        cx.st.data_passes = before.data_passes; cx.st.xb_launches = before.xb_launches;
-                        cx.st.gemv_bytes = before.gemv_bytes; cx.st.allreduce_calls = before.allreduce_calls;
-                        cx.st.allreduce_doubles = before.allreduce_doubles;
-                    }
-                    break;
-                }
-                ++it;
-                if (it >= o->irls_maxit) { it = o->irls_maxit - 1; break; }
-                if (!ahead) enqueue_iteration(it);
-            }
-            res->niter[(size_t)pp * L + i] = (broke ? it : o->irls_maxit) + 1;
-            par0 = (par0 + it + 1) & 1;                      // the iterate the last EXECUTED iteration produced
-            double *fin = d_iter.p + (size_t)par0 * q;
-            OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, fin, sizeof(double) * q, cudaMemcpyDeviceToDevice,
-                                     cx.stream));
+            res->niter[(size_t)pp * L + i] = loop.run(cx, o->irls_maxit, par0, enqueue_iteration);
+            OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, d_iter.p + (size_t)par0 * q, sizeof(double) * q,
+                                     cudaMemcpyDeviceToDevice, cx.stream));
             if (s->compute_loss && res->loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, yv.p, d_prob.p, n);
         }
     }
@@ -567,35 +512,40 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
     DBuf<double> d_iter(2 * (size_t)q), d_path((size_t)su.P * L * q);
     DBuf<double> d_prob(n + 2), d_res(n + 2), d_W(n + 2);
     DBuf<long long> d_iters_total(1);
-    DBuf<int> d_niter(1), d_lz(1);
+    DBuf<int> d_niter(1), d_lz(1), d_conv(1);
     d_prob.zero(cx.stream);
     d_iters_total.zero(cx.stream);
     d_path.zero(cx.stream);
     d_cinv.upload(cinv.data(), p, cx.stream);
-    PinnedFlags flag(1);
     PathScratches scratch(1);
     fill_common_outputs(su, res);
     const double *cinv_dev = stdz ? d_cinv.p : nullptr;
     double xxdiag = 0.0, intval = 0.0;
+    IrlsModel md;
+    md.XX = d_XX.p; md.XY = d_XY.p; md.d = d_d.p; md.niter = d_niter.p; md.lz = d_lz.p; md.scratch = scratch.s[0];
+    md.conv = d_conv.p; md.iters_total = d_iters_total.p; md.icpt = icpt; md.cinv = cinv_dev; md.b = d_b.p; md.b0 = d_b0.p;
+    IrlsLoop loop(false);          // the sparse Gram launch cannot be predicated
 
     for (int pp = 0; pp < su.P; ++pp) {
-        double *cur = d_iter.p, *nxt = d_iter.p + q;
-        OEM_CUDA(cudaMemsetAsync(cur, 0, sizeof(double) * q, cx.stream));
+        int par0 = 0;                            // d_iter.p + par0 * q holds the iterate the next iteration starts from
+        OEM_CUDA(cudaMemsetAsync(d_iter.p, 0, sizeof(double) * q, cx.stream));
         for (int i = 0; i < su.nlam_run[pp]; ++i) {
             const bool on_lam_1 = (i == 0);
-            int it = 0;
-            bool broke = false;
-            for (it = 0; it < o->irls_maxit; ++it) {
-                bool rebuilt = false;
-                if (!(it == 0 && !on_lam_1)) {
-                    irls_coef_kernel<<<(p + 255) / 256, 256, 0, cx.stream>>>(cur, cinv_dev, p, icpt, d_b.p, d_b0.p, nullptr);
-                    cx.st.kernel_launches += 1;
+            OEM_CUDA(cudaMemsetAsync(d_conv.p, 0, sizeof(int), cx.stream));
+            auto enqueue_iteration = [&](int k, volatile int *verdict) {
+                double *cur = d_iter.p + (size_t)((par0 + k) & 1) * q, *nxt = d_iter.p + (size_t)((par0 + k + 1) & 1) * q;
+                const bool pass = !(k == 0 && !on_lam_1);
+                if (pass) {
+                    if (k == 0) {      // later passes of this lambda get b from the previous iteration's path launch (IRLS epilogue)
+                        irls_coef_kernel<<<(p + 255) / 256, 256, 0, cx.stream>>>(cur, cinv_dev, p, icpt, d_b.p, d_b0.p, nullptr);
+                        cx.st.kernel_launches += 1;
+                    }
                     const size_t t1 = tm.start(&cx.st.ms_irls_xb);
                     sparse_xb_logistic_launch(cx, sd.get(), d_b.p, d_b0.p, yv.p, d_prob.p, d_res.p, d_W.p);
                     tm.stop(t1);
                     cx.st.data_passes += 1;
-                    if (cx.rank == 0 && it < n) {            // W(i) clamp, sic (:948-954)
-                        clamp_one_kernel<<<1, 1, 0, cx.stream>>>(d_W.p, it, 1e-5, nullptr);
+                    if (cx.rank == 0 && k < n) {             // W(i) clamp, sic (:948-954)
+                        clamp_one_kernel<<<1, 1, 0, cx.stream>>>(d_W.p, k, 1e-5, nullptr);
                         cx.st.kernel_launches += 1;
                     }
                     sparse_gram_launch(cx, sd.get(), d_W.p, G);                                   // X'WX
@@ -628,28 +578,22 @@ void fit_logistic_sparse(const int *row_idx, const int *col_ptr, const double *v
                         p, icpt, G, statsW + (size_t)p, cinv_dev, intval, xxdiag, n_tot, d_XX.p);
                     irls_pack_grad_kernel<<<(p + 255) / 256, 256, 0, cx.stream>>>(statsR + (size_t)p, rs, p, d_g.p);
                     cx.st.kernel_launches += 2;
-                    path_xy_launch(cx, q, icpt, d_XX.p, cur, d_g.p, cinv_dev, n_tot, d_XY.p, nullptr);
-                    rebuilt = true;
                 }
-                PathProblem pr = irls_path_problem(tb, su, pp, i, o);
-                pr.XX = d_XX.p; pr.XY = d_XY.p; pr.d = d_d.p; pr.compute_eig = rebuilt;
-                pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p; pr.lanczos_steps = d_lz.p;
-                pr.scratch = scratch.s[0];
+                // X'WX is rebuilt on every pass, so the eigenvalue is too; XY = XX beta + grad is formed by the launch
                 const size_t t3 = tm.start(&cx.st.ms_path);
-                path_launch(cx, pr);
+                path_launch(cx, irls_path_problem(tb, su, pp, i, o, md, cur, nxt, verdict, pass, pass ? d_g.p : nullptr, n_tot));
                 tm.stop(t3);
-                irls_stop_kernel<<<1, 256, 0, cx.stream>>>(nxt, cur, q, o->irls_tol, d_niter.p, d_iters_total.p, flag.p, nullptr);
+            };
+
+            res->niter[(size_t)pp * L + i] = loop.run(cx, o->irls_maxit, par0, enqueue_iteration);
+            double *fin = d_iter.p + (size_t)par0 * q;
+            if (icpt) {
+                // get_beta(): beta(0) *= intval, in place (:1040-1043).  The next lambda starts without a data pass, and its
+                // path launch derives the following pass's b0 from its own output
+                scale_first_kernel<<<1, 1, 0, cx.stream>>>(fin, intval);
                 cx.st.kernel_launches += 1;
-                cx.sync();
-                std::swap(cur, nxt);
-                if (*flag.p) { broke = true; break; }
             }
-            res->niter[(size_t)pp * L + i] = (broke ? it : o->irls_maxit) + 1;
-            if (icpt) {                                      // get_beta(): beta(0) *= intval, in place (:1040-1043)
-                scale_first_kernel<<<1, 1, 0, cx.stream>>>(cur, intval);
-                cx.st.kernel_launches += 1;
-            }
-            OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, cur, sizeof(double) * q, cudaMemcpyDeviceToDevice,
+            OEM_CUDA(cudaMemcpyAsync(d_path.p + ((size_t)pp * L + i) * q, fin, sizeof(double) * q, cudaMemcpyDeviceToDevice,
                                      cx.stream));
             if (s->compute_loss && res->loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, yv.p, d_prob.p, n);
         }

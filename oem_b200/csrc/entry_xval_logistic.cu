@@ -125,21 +125,15 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
                     const size_t qm = (size_t)m * q;
                     double *base = d_iter.p + 2 * qm;
                     double *cur = base + (size_t)((par0[m] + k) & 1) * q, *nxt = base + (size_t)((par0[m] + k + 1) & 1) * q;
-                    const double *cinv_m = cinv_all ? cinv_all + (size_t)m * p : nullptr;
-                    PathProblem pr = irls_path_problem(tb, su, pp, i, o);
-                    pr.XX = xs.XX.p + qm * q; pr.XY = d_XY.p + qm; pr.d = d_d.p + m; pr.compute_eig = (k == 0 && i == 0);
-                    pr.beta_init = cur; pr.beta_out = nxt; pr.niter_out = d_niter.p + m; pr.lanczos_steps = d_lz.p + m;
-                    pr.scratch = scratch.s[m];
-                    pr.skip = d_conv.p + m;
-                    if (pass) {
-                        pr.xy_grad = d_G.p + (size_t)m * (p + 1); pr.xy_cinv = cinv_m; pr.xy_n = xs.hn[m];
-                        pr.xy_icpt = icpt; pr.xy_out = d_XY.p + qm;
-                    }
-                    pr.t_acc = d_clk.p;
-                    pr.irls_conv = d_conv.p + m; pr.irls_host_flag = flags.p + m; pr.irls_iters_total = d_iters_total.p;
-                    pr.irls_tol = o->irls_tol; pr.irls_cinv = cinv_m; pr.irls_p = p; pr.irls_icpt = icpt;
-                    pr.irls_b = d_B.p + (size_t)m * p; pr.irls_b0 = d_b0.p + m;
-                    path_launch(cx, pr);
+                    IrlsModel md;
+                    md.XX = xs.XX.p + qm * q; md.XY = d_XY.p + qm; md.d = d_d.p + m;
+                    md.niter = d_niter.p + m; md.lz = d_lz.p + m; md.scratch = scratch.s[m];
+                    md.conv = d_conv.p + m; md.iters_total = d_iters_total.p;
+                    md.icpt = icpt; md.cinv = cinv_all ? cinv_all + (size_t)m * p : nullptr;
+                    md.b = d_B.p + (size_t)m * p; md.b0 = d_b0.p + m;
+                    md.t_acc = d_clk.p;
+                    path_launch(cx, irls_path_problem(tb, su, pp, i, o, md, cur, nxt, flags.p + m, k == 0 && i == 0,
+                                                      pass ? d_G.p + (size_t)m * (p + 1) : nullptr, xs.hn[m]));
                 }
                 cx.sync();                                   // the one host round trip of the round
                 int left = 0;

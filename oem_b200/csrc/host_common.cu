@@ -173,7 +173,7 @@ void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_
 
     PathProblem pp;
     pp.q = q; pp.ngram = ngram; pp.XX = XX; pp.XY = XY; pp.d = pb.d.p;
-    pp.compute_eig = true; pp.eig_factor = eig_factor; pp.eig_tol = 1e-10;
+    pp.compute_eig = true; pp.eig_factor = eig_factor;
     for (int g = 0; g < ngram; ++g)
         for (int k = 0; k < P; ++k) {
             ChainDesc c;
@@ -203,17 +203,28 @@ void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_
     for (int v : pb.h_lz) cx.st.lanczos_steps += v;
 }
 
-PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o) {
+PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o, const IrlsModel &m,
+                              const double *cur, double *nxt, volatile int *verdict, bool compute_eig, const double *grad,
+                              double n_rows) {
     PathProblem pr;
     pr.q = tb.q; pr.ngram = 1;
-    pr.eig_factor = 1.0005; pr.eig_tol = 1e-10;
+    pr.XX = m.XX; pr.XY = m.XY; pr.d = m.d;
+    pr.compute_eig = compute_eig; pr.eig_factor = 1.0005;
     ChainDesc c;
     c.gram = 0; c.penalty = su.pen[pp]; c.nlam = 1; c.lam_off = 0; c.alpha = su.alpha;
     c.gamma = su.gamma[pp]; c.tau = su.tau; c.out_off = 0;
     pr.chains.push_back(c);
     pr.lambdas = tb.lambdas.p + (size_t)pp * tb.Lmax + i; pr.Lmax = 1;
     use_tables(pr, tb);
+    pr.beta_init = cur; pr.beta_out = nxt;
     pr.maxit = o->maxit; pr.tol = o->tol;
+    pr.niter_out = m.niter; pr.lanczos_steps = m.lz; pr.scratch = m.scratch;
+    pr.skip = m.conv;
+    pr.t_acc = m.t_acc;
+    pr.irls_conv = m.conv; pr.irls_host_flag = verdict; pr.irls_iters_total = m.iters_total;
+    pr.irls_tol = o->irls_tol; pr.irls_cinv = m.cinv; pr.irls_p = tb.q - m.icpt; pr.irls_icpt = m.icpt;
+    pr.irls_b = m.b; pr.irls_b0 = m.b0;
+    if (grad) { pr.xy_grad = grad; pr.xy_cinv = m.cinv; pr.xy_n = n_rows; pr.xy_icpt = m.icpt; pr.xy_out = m.XY; }
     return pr;
 }
 

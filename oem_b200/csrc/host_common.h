@@ -68,10 +68,30 @@ struct PathBuffers {
 void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int ngram, const double *XX,
                const double *XY, double eig_factor, bool accelerate, const double *post_scale_dev, PathBuffers &pb);
 
-// The inner OEM loop of one IRLS iteration (src/oem_logistic_dense.h:1010-1022): one chain, lambda i of penalty pp, warm
-// start, eigenvalue factor 1.0005.  The caller sets XX / XY / d, compute_eig, beta_init / beta_out, niter_out /
-// lanczos_steps / scratch, skip and the irls_* / xy_* / t_acc fields.
-PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o);
+// The device slots of one model of an IRLS loop: its system XX / XY (q = tb.q) and eigenvalue bound d, the path launch's
+// iteration count, Lanczos steps and tables, the convergence flag that predicates the model's work, the running count of
+// inner iterations (may be shared by models), and the coefficients of the model's next data pass, b (p = q - icpt) and
+// *b0, with the column scaling cinv (device, p; NULL when not standardised).  t_acc (may be NULL): see PathProblem.
+struct IrlsModel {
+    const double *XX = nullptr;
+    double *XY = nullptr, *d = nullptr;
+    int *niter = nullptr, *lz = nullptr;
+    PathScratch *scratch = nullptr;
+    int *conv = nullptr;
+    long long *iters_total = nullptr;
+    int icpt = 0;
+    const double *cinv = nullptr;
+    double *b = nullptr, *b0 = nullptr;
+    unsigned long long *t_acc = nullptr;
+};
+// One IRLS iteration's path launch (src/oem_logistic_dense.h:999-1033) for model m: lambda i of penalty pp, one chain, warm
+// started from cur, eigenvalue factor 1.0005 (recomputed when compute_eig), predicated on *m.conv.  Its last step is the
+// outer stop rule on (nxt, cur), whose verdict goes to *m.conv and *verdict, and b / b0 from nxt.  With grad (device,
+// [sum r, X'r] over n_rows rows) it first forms XY = XX cur + grad / n_rows (scaled by cinv); without, it keeps the XY of
+// the model's previous data pass.
+PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o, const IrlsModel &m,
+                              const double *cur, double *nxt, volatile int *verdict, bool compute_eig, const double *grad,
+                              double n_rows);
 
 // res->beta (P x Lmax x (p + 1): intercept row first, zero where no lambda ran) from the raw q-vectors of a fit, iterate
 // (pp, i) at raw + (pp * Lmax + i) * q with q = p + icpt; cinv (host, p) undoes the standardisation, NULL if none.

@@ -84,7 +84,7 @@ struct PathArgs {
     const double *lambdas, *pen_fact;
     const int *unique_groups, *grp_ptr, *grp_idx, *grp_cover;
     const double *group_weights, *post_scale, *beta_init;
-    double *beta_final, *beta_out;
+    double *beta_out;
     int *niter_out, *lanczos_steps;
     double *ubuf;            // ngram x 2 x max_ct x q
     unsigned *barriers;      // ngram counters, zero-initialised
@@ -1163,13 +1163,6 @@ __global__ void __launch_bounds__(PK_THREADS, 1) oem_path_kernel(const PathArgs 
                 a.prof[8] += tA - t2; a.prof[9] += tB - tA; a.prof[10] += tC - tB; a.prof[11] += tD - tC; a.prof[12] += t3 - tD;
             }
         }
-        if (a.beta_final && rank == 0) {
-            const double *Bc = cur ? B1 : B0;
-            for (int e = threadIdx.x; e < nct * q; e += PK_THREADS) {
-                const int c = e / q, j = e - c * q;
-                a.beta_final[(size_t)chi[2 * PK_MAXCT + c] * q + j] = Bc[(size_t)c * qs + j];
-            }
-        }
         // ---- IRLS epilogue: the outer loop's stop rule on (final iterate, warm start), verdicts, next pass's coefficients ----
         if (a.irls_conv && blockIdx.x == 0) {
             __syncthreads();
@@ -1478,8 +1471,8 @@ __global__ void path_xy_kernel(int q, int icpt, const double *__restrict__ XX, c
     }
 }
 
-void path_xy_launch(Ctx &cx, int q, int icpt, const double *XX, const double *beta, const double *g, const double *cinv, double n_tot,
-                    double *XY, const int *skip) {
+static void path_xy_launch(Ctx &cx, int q, int icpt, const double *XX, const double *beta, const double *g, const double *cinv,
+                           double n_tot, double *XY, const int *skip) {
     path_xy_kernel<<<(q + 7) / 8, 256, 0, cx.stream>>>(q, icpt, XX, beta, g, cinv, n_tot, XY, skip);
     OEM_CUDA(cudaGetLastError());
     cx.st.kernel_launches += 1;
@@ -1533,7 +1526,7 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
 
     // ---- small coordinate-wise problems: register-resident variant (d comes from a Lanczos-only generic launch) ----
     {
-        bool reg_ok = q <= 256 && !pp.accelerate && !pp.post_scale && !pp.beta_init && !pp.beta_final && !pp.skip &&
+        bool reg_ok = q <= 256 && !pp.accelerate && !pp.post_scale && !pp.beta_init && !pp.skip &&
                       !pp.irls_conv && max_ct <= PR_MAXCT && !pp.chains.empty();
         for (auto &c : pp.chains) reg_ok = reg_ok && c.penalty < OEMB200_PEN_GRP_LASSO;
         const int NC = q <= 128 ? 1 : (q + 31) / 32;
@@ -1716,7 +1709,7 @@ void path_launch(Ctx &cx, const PathProblem &pp) {
     a.lambdas = pp.lambdas; a.pen_fact = pp.pen_fact;
     a.unique_groups = pp.unique_groups; a.grp_ptr = pp.grp_ptr; a.grp_idx = pp.grp_idx; a.grp_cover = pp.grp_cover;
     a.group_weights = pp.group_weights; a.post_scale = pp.post_scale; a.beta_init = pp.beta_init;
-    a.beta_final = pp.beta_final; a.beta_out = pp.beta_out; a.niter_out = pp.niter_out;
+    a.beta_out = pp.beta_out; a.niter_out = pp.niter_out;
     a.lanczos_steps = pp.lanczos_steps; a.ubuf = d_ubuf.p; a.barriers = d_bar.p; a.gflags = d_gflags_p;
     a.skip = pp.skip; a.t_acc = pp.t_acc;
     if (pp.irls_conv) {

@@ -202,7 +202,7 @@ struct PathProblem {
     double *d = nullptr;           // device, ngram: in (compute_eig=0) or out (compute_eig=1)
     bool compute_eig = true;
     double eig_factor = 1.005;
-    double eig_tol = 1e-11;
+    double eig_tol = 1e-10;
     std::vector<ChainDesc> chains;
     const double *lambdas = nullptr;   // device, concatenated
     int Lmax = 0;                      // stride (in lambdas) of a chain's output block
@@ -215,7 +215,6 @@ struct PathProblem {
     const int *grp_cover = nullptr;       // device, q: 1 if the variable belongs to a listed group
     const double *post_scale = nullptr;   // oem_xtx scale.factor quirk: beta *= post_scale after each lambda
     const double *beta_init = nullptr;    // device, nchains x q warm start (NULL = zeros)
-    double *beta_final = nullptr;         // device, nchains x q: iterate after the last lambda (may be NULL)
     int maxit = 500;
     double tol = 1e-7;
     bool accelerate = false;
@@ -239,16 +238,14 @@ struct PathProblem {
     unsigned long long *t_acc = nullptr;   // optional device word: += the kernel's duration in ns (%globaltimer of team 0's first member)
     // Logistic inner loop (src/oem_logistic_dense.h:970-999): with xy_grad set the launch first forms
     //   XY = XX beta_init + [g[0] / n, (g[1 + j] / n) o cinv[j]]
-    // into xy_out (which must be the buffer XY points at; one Gram, one chain).  The register-mode kernel does it with the
-    // XX slice it has just loaded; the other modes run path_xy_launch in front.
+    // into xy_out (which must be the buffer XY points at; one Gram, one chain).  The register-resident global mode does it
+    // with the XX slice its members have just loaded; the other modes launch path_xy_kernel in front.
     const double *xy_grad = nullptr, *xy_cinv = nullptr;
     double xy_n = 0.0;
     int xy_icpt = 0;
     double *xy_out = nullptr;
 };
 void path_launch(Ctx &cx, const PathProblem &pp);
-void path_xy_launch(Ctx &cx, int q, int icpt, const double *XX, const double *beta, const double *g, const double *cinv, double n_tot,
-                    double *XY, const int *skip);
 // throws OEMB200_EUNSUPPORTED if a beta of dimension q (chains_per_gram penalties, Lmax lambdas) cannot be held by the path kernel
 void path_check_fits(Ctx &cx, int q, int chains_per_gram, int Lmax, int ngroups, int ngidx);
 
@@ -267,8 +264,6 @@ void assemble_dense_launch(Ctx &cx, int p, int flag, double n, const double *G, 
 // oem_xtx scale.factor (sinv may be NULL = plain copy)
 void scale_sym_launch(Ctx &cx, int p, const double *sinv, const double *XXin, const double *XYin, double *XX,
                       double *XY);
-// y = M x + add for a symmetric q x q M
-void symv_add_launch(Ctx &cx, int q, const double *M, const double *x, const double *add, double *y);
 
 // ---------------- logit_slab.cu ----------------
 int logit_slab_rows(int p);                       // rows per slab (0: the slab route does not apply to this p; it does for 8 <= p <= 2048)

@@ -2,6 +2,8 @@
 src/oem_sparse.cpp / oem_sparse.h -- all penalties, the four standardize / intercept combinations (the intercept column
 is the constant `intval`, get_beta() rescales beta(0) in place), compute.loss, empty rows / columns, device-resident
 slots, run-to-run determinism of the atomics-free Gram."""
+import re
+
 import numpy as np
 import pytest
 
@@ -199,6 +201,30 @@ def test_logistic_sparse_gram_routes_and_device_slots(lib, oracle, monkeypatch, 
             torch.from_numpy(X.data).cuda(), X.shape)
     a[1] = torch.from_numpy(y).cuda()
     assert_same_fit(lib.oem_fit_logistic_sparse(*a), ref, tol=1e-8)
+
+
+@pytest.mark.parametrize("irls_maxit", [1, 2, 3])
+def test_logistic_sparse_irls_maxit_exhausted(lib, oracle, irls_maxit):
+    # the IRLS cap cuts every loop short: niter reports irls_maxit + 1, and the iterate handed to the next lambda (after
+    # get_beta()'s in-place intval scaling) is the one the last executed iteration produced
+    X, y = _sparse_binomial(94, 3000, 60, 0.08)
+    a = args_xy(X, y, "binomial", ["lasso", "mcp"], nlambda=8, lmin_ratio=2e-2, opts=dict(irls_maxit=irls_maxit, irls_tol=1e-9))
+    got, ref = lib.oem_fit_logistic_sparse(*a), oracle.oem_fit_logistic_sparse(*a)
+    assert_same_fit(got, ref, tol=1e-8)
+    for ng, nr in zip(got["niter"], ref["niter"]):
+        assert np.array_equal(ng, nr) and ng.max() == irls_maxit + 1
+
+
+def test_logistic_sparse_register_resident_global_mode(lib, oracle, monkeypatch, capfd):
+    # p = 599 (q = 600 with the intercept): the path launch of an IRLS iteration takes the cooperative global mode with the
+    # register-resident mat-vec (rpt > 0), which forms XY = XX beta + grad inside the kernel instead of path_xy_kernel
+    monkeypatch.setenv("OEMB200_PATH_PROF", "1")
+    X, y = _sparse_binomial(93, 4000, 599, 0.03)
+    a = args_xy(X, y, "binomial", ["lasso", "mcp"], nlambda=6, lmin_ratio=5e-2)
+    got = lib.oem_fit_logistic_sparse(*a)
+    prof = [line for line in capfd.readouterr().err.splitlines() if line.startswith("[path prof] mode=")]
+    assert prof and all(re.search(r"mode=2 rpt=[2-5] ", line) for line in prof), prof[:3]
+    assert_same_fit(got, oracle.oem_fit_logistic_sparse(*a), tol=1e-8)
 
 
 def test_logistic_sparse_rejects_the_undefined_combination(lib):

@@ -13,8 +13,9 @@
 //   2. per penalty, lambda and IRLS round: ONE fused data pass for all still-active models (logit_fold_launch; a pass
 //      is ceil(M / logit_fold_models(p)) sweeps), then one single-chain path launch per active model, which forms
 //      XY = XX beta + grad, runs the inner OEM loop, applies the outer stop rule and leaves the model's next
-//      coefficients (PathProblem::irls_*).  The host waits once per round and reads the M verdicts; a converged model
-//      idles until lambda advances, so every model does exactly the arithmetic of a separate fit;
+//      coefficients (PathProblem::irls_*).  The rounds are IrlsLoop's (host_common.h), the outer loop of the dense and
+//      sparse drivers, with M models and no speculation: the host waits once per round and reads the M verdicts; a
+//      converged model idles until lambda advances, so every model does exactly the arithmetic of a separate fit;
 //   3. one fold-segmented scoring GEMM with the binomial epilogue (cvscore_binomial_launch).
 // The reference's logistic quirks come along: no data pass on the first IRLS iteration of every lambda after the first,
 // eigenvalue factor 1.0005, uncentred standardisation from each model's own rows.
@@ -84,87 +85,37 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
     // ---- device state: one slice per model ----
     const int L = su.Lmax, P = su.P;
     PenaltyTables tb(cx, su, s, p, icpt);
-    DBuf<double> d_B((size_t)M * p), d_b0(M), d_G((size_t)M * (p + 1)), d_XY((size_t)M * q), d_d(M);
-    DBuf<double> d_iter((size_t)M * 2 * q), d_path((size_t)M * P * L * q), d_prob(npad);
-    DBuf<long long> d_iters_total(1);
-    DBuf<int> d_niter(M), d_lz(M), d_conv(M);
+    DBuf<double> d_G((size_t)M * (p + 1)), d_XY((size_t)M * q), d_d(M), d_prob(npad);
     DBuf<unsigned long long> d_clk(1);
     d_prob.zero(cx.stream);
-    d_path.zero(cx.stream);
-    d_iters_total.zero(cx.stream);
     d_clk.zero(cx.stream);
-    PinnedFlags flags(M);         // one verdict slot per model, written by its path launch
-    PathScratches scratch(M);
+    IrlsLoop loop(cx, su, tb, o, M, icpt, /*speculate=*/false);
+    for (int m = 0; m < M; ++m)
+        loop.set_model(m, xs.XX.p + (size_t)m * q * q, d_XY.p + (size_t)m * q, d_d.p + m,
+                       stdz ? xs.cinv.p + (size_t)m * p : nullptr, d_clk.p);
     fill_common_outputs(su, res);
-    const double *cinv_all = stdz ? xs.cinv.p : nullptr;
     const bool want_loss = s->compute_loss && res->loss;
 
-    std::vector<int> par0(M), it_m(M);
-    std::vector<char> active(M), broke(M);
-    for (int pp = 0; pp < P; ++pp) {
-        // init(): beta = 0 for every model, so the first pass multiplies X with b = 0, b0 = 0
-        OEM_CUDA(cudaMemsetAsync(d_iter.p, 0, d_iter.n * sizeof(double), cx.stream));
-        OEM_CUDA(cudaMemsetAsync(d_B.p, 0, d_B.n * sizeof(double), cx.stream));
-        OEM_CUDA(cudaMemsetAsync(d_b0.p, 0, d_b0.n * sizeof(double), cx.stream));
-        std::fill(par0.begin(), par0.end(), 0);
-        for (int i = 0; i < su.nlam_run[pp]; ++i) {
-            OEM_CUDA(cudaMemsetAsync(d_conv.p, 0, sizeof(int) * M, cx.stream));
-            std::fill(active.begin(), active.end(), 1);
-            std::fill(broke.begin(), broke.end(), 0);
-            for (int k = 0;; ++k) {
-                const bool pass = !(k == 0 && i > 0);      // the reference skips the data pass on a warm lambda's first iteration
-                if (pass) {
-                    const size_t t1 = tm.start(&cx.st.ms_irls_xb);
-                    const int sweeps = logit_fold_launch(cx, slabs.p, npad, p, d_B.p, d_b0.p, xs.ys.p, d_rowfold.p, M,
-                                                         d_conv.p, &active, want_loss ? d_prob.p : nullptr, d_G.p);
-                    tm.stop(t1);
-                    cx.st.gemv_bytes += 8.0 * (double)npad * p * sweeps;
-                }
-                for (int m = 0; m < M; ++m) {
-                    if (!active[m]) continue;
-                    const size_t qm = (size_t)m * q;
-                    double *base = d_iter.p + 2 * qm;
-                    double *cur = base + (size_t)((par0[m] + k) & 1) * q, *nxt = base + (size_t)((par0[m] + k + 1) & 1) * q;
-                    IrlsModel md;
-                    md.XX = xs.XX.p + qm * q; md.XY = d_XY.p + qm; md.d = d_d.p + m;
-                    md.niter = d_niter.p + m; md.lz = d_lz.p + m; md.scratch = scratch.s[m];
-                    md.conv = d_conv.p + m; md.iters_total = d_iters_total.p;
-                    md.icpt = icpt; md.cinv = cinv_all ? cinv_all + (size_t)m * p : nullptr;
-                    md.b = d_B.p + (size_t)m * p; md.b0 = d_b0.p + m;
-                    md.t_acc = d_clk.p;
-                    path_launch(cx, irls_path_problem(tb, su, pp, i, o, md, cur, nxt, flags.p + m, k == 0 && i == 0,
-                                                      pass ? d_G.p + (size_t)m * (p + 1) : nullptr, xs.hn[m]));
-                }
-                cx.sync();                                   // the one host round trip of the round
-                int left = 0;
-                for (int m = 0; m < M; ++m) {
-                    if (!active[m]) continue;
-                    if (flags.p[m]) { active[m] = 0; broke[m] = 1; it_m[m] = k; }
-                    else left++;
-                }
-                if (!left) break;
-                if (k + 1 >= o->irls_maxit) {
-                    for (int m = 0; m < M; ++m)
-                        if (active[m]) { active[m] = 0; it_m[m] = o->irls_maxit - 1; }
-                    break;
-                }
-            }
-            for (int m = 0; m < M; ++m) {
-                if (m == 0) res->niter[(size_t)pp * L + i] = (broke[0] ? it_m[0] : o->irls_maxit) + 1;
-                par0[m] = (par0[m] + it_m[m] + 1) & 1;       // the iterate the model's last executed iteration produced
-                const double *fin = d_iter.p + (size_t)m * 2 * q + (size_t)par0[m] * q;
-                OEM_CUDA(cudaMemcpyAsync(d_path.p + (((size_t)m * P + pp) * L + i) * q, fin, sizeof(double) * q,
-                                         cudaMemcpyDeviceToDevice, cx.stream));
-            }
-            // padding rows hold prob = 0 and y = 0: their terms are log(1) = 0
-            if (want_loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, xs.ys.p, d_prob.p, npad);
+    loop.run(res, [&](int i, int k, bool pass) {
+        if (pass) {
+            const size_t t1 = tm.start(&cx.st.ms_irls_xb);
+            const int sweeps = logit_fold_launch(cx, slabs.p, npad, p, loop.b.p, loop.b0.p, xs.ys.p, d_rowfold.p, M,
+                                                 loop.conv.p, &loop.active, want_loss ? d_prob.p : nullptr, d_G.p);
+            tm.stop(t1);
+            cx.st.gemv_bytes += 8.0 * (double)npad * p * sweeps;
         }
-    }
+        for (int m = 0; m < M; ++m)
+            if (loop.active[m])
+                loop.path_step(m, k == 0 && i == 0, pass ? d_G.p + (size_t)m * (p + 1) : nullptr, xs.hn[m]);
+    }, [&](int pp, int i) {
+        // padding rows hold prob = 0 and y = 0: their terms are log(1) = 0
+        if (want_loss) res->loss[(size_t)pp * L + i] = logistic_loss(cx, xs.ys.p, d_prob.p, npad);
+    });
 
     // ---- full model back to the host, un-scaled (get_beta) ----
     unsigned long long hclk = 0;
     d_clk.download(&hclk, 1, cx.stream);
-    irls_write_path(cx, su, p, icpt, d_path.p, d_iters_total.p, d_d.p, stdz ? xs.hcinv.data() : nullptr, res);
+    loop.write_path(stdz ? xs.hcinv.data() : nullptr, res);
     cx.st.ms_path += (double)hclk * 1e-6;
 
     // ---- CV scoring: fold k's rows against fold model k ----
@@ -172,7 +123,7 @@ void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const dou
     DBuf<double> dB((size_t)F * p * ncld), db0((size_t)F * ncld), out3(3 * (size_t)nc);
     DBuf<int> d_nlam(P);
     d_nlam.upload(su.nlam_run.data(), P, cx.stream);
-    cv_build_coef_launch(cx, d_path.p, xs.cinv.p, F, P, L, p, q, icpt, stdz, d_nlam.p, dB.p, db0.p);
+    cv_build_coef_launch(cx, loop.path.p, xs.cinv.p, F, P, L, p, q, icpt, stdz, d_nlam.p, dB.p, db0.p);
     std::vector<std::array<int64_t, 3>> cs;
     for (int k = 0; k < F; ++k) cs.push_back({xs.off[k], xs.off[k + 1], xs.off[k] + xs.cnt[k]});
     cvscore_binomial_launch(cx, xs.Xs.p, npad, p, npad, xs.ys.p, F, cs, dB.p, db0.p, nc, measure, out3.p);

@@ -1,6 +1,6 @@
 // host_common.cu -- see host_common.h.  Host logic only (no kernels): penalty / group / lambda
-// bookkeeping restated from the reference's entry functions, its device tables, the path-kernel round trip and the
-// write-back of the raw iterates into the reported beta.
+// bookkeeping restated from the reference's entry functions, its device tables, the path-kernel round trip, the
+// write-back of the raw iterates into the reported beta, and the logistic init step and IRLS loop.
 #include <algorithm>
 #include <cstring>
 #include "host_common.h"
@@ -203,9 +203,14 @@ void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_
     for (int v : pb.h_lz) cx.st.lanczos_steps += v;
 }
 
-PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o, const IrlsModel &m,
-                              const double *cur, double *nxt, volatile int *verdict, bool compute_eig, const double *grad,
-                              double n_rows) {
+// One IRLS iteration's path launch (src/oem_logistic_dense.h:999-1033) for model m: lambda i of penalty pp, one chain, warm
+// started from cur, eigenvalue factor 1.0005 (recomputed when compute_eig), predicated on *m.conv.  Its last step is the
+// outer stop rule on (nxt, cur), whose verdict goes to *m.conv and *verdict, and b / b0 from nxt.  With grad (device,
+// [sum r, X'r] over n_rows rows) it first forms XY = XX cur + grad / n_rows (scaled by cinv); without, it keeps the XY of
+// the model's previous data pass.
+static PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o,
+                                     const IrlsModel &m, const double *cur, double *nxt, volatile int *verdict,
+                                     bool compute_eig, const double *grad, double n_rows) {
     PathProblem pr;
     pr.q = tb.q; pr.ngram = 1;
     pr.XX = m.XX; pr.XY = m.XY; pr.d = m.d;
@@ -240,18 +245,152 @@ void write_beta(const Setup &su, const double *raw, int p, int icpt, const doubl
         }
 }
 
-void irls_write_path(Ctx &cx, const Setup &su, int p, int icpt, const double *path_dev, const long long *iters_total_dev,
-                     const double *d_dev, const double *cinv, oemb200_result *res) {
-    std::vector<double> hpath((size_t)su.P * su.Lmax * (p + icpt));
+LogisticInit logistic_init(Ctx &cx, int64_t n, int p, int q, bool stdz, const std::function<void(double *)> &colstats,
+                           const char *refusal) {
+    LogisticInit r;
+    const size_t nb = 3 * (size_t)p + 1;
+    r.stats.alloc(nb);
+    PhaseTimers &tm = *cx.tm;
+    const size_t t_c = tm.start(&cx.st.ms_colstats);
+    colstats(r.stats.p);
+    tm.stop(t_c);
+    const double nd = (double)n;
+    OEM_CUDA(cudaMemcpyAsync(r.stats.p + 3 * (size_t)p, &nd, 8, cudaMemcpyHostToDevice, cx.stream));
+    const size_t t_ar = tm.start(&cx.st.ms_allreduce);
+    cx.all_reduce(r.stats.p, (int64_t)nb);
+    tm.stop(t_ar);
+    std::vector<double> h(nb);
+    r.stats.download(h.data(), nb, cx.stream);
+    cx.sync();
+    r.n_tot = h[3 * (size_t)p];
+    if (!(r.n_tot > q)) fail(OEMB200_EUNSUPPORTED, "%s", refusal);
+    // 1 / sd of every column from its sum of squares (uncentred, divisor n - 1, a zero column keeps scale 1)
+    r.cinv.assign(p, 1.0);
+    for (int j = 0; j < p; ++j) {
+        if (stdz) {
+            double sq = h[2 * (size_t)p + j] / (r.n_tot - 1.0);
+            if (sq == 0.0) sq = 1.0;
+            r.cinv[j] = 1.0 / std::sqrt(sq);
+        }
+        double v = h[(size_t)p + j];
+        if (stdz) v *= r.cinv[j];
+        r.lmax = std::max(r.lmax, std::fabs(v / r.n_tot));
+    }
+    return r;
+}
+
+IrlsLoop::IrlsLoop(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int M, int icpt, bool speculate)
+    : b((size_t)M * (tb.q - icpt)), b0(M), conv(M), path((size_t)M * su.P * su.Lmax * tb.q), active(M), cx_(cx), su_(su),
+      tb_(tb), o_(o), M_(M), q_(tb.q), speculate_(speculate), iter_((size_t)M * 2 * tb.q), niter_(M), lz_(M),
+      iters_total_(1), scratch_(M), md_(M), flag_(4 * M), par0_(M), last_(M), niter_h_(M) {
+    if (speculate && M > 1) fail(OEMB200_EINVAL, "IRLS loop: only a single model may be enqueued ahead (M = %d)", M);
+    ev_[0] = event_acquire();
+    ev_[1] = event_acquire();
+    iters_total_.zero(cx.stream);
+    path.zero(cx.stream);
+    for (int m = 0; m < M; ++m) {
+        IrlsModel &d = md_[m];
+        d.niter = niter_.p + m; d.lz = lz_.p + m; d.scratch = scratch_.s[m]; d.conv = conv.p + m;
+        d.iters_total = iters_total_.p; d.icpt = icpt; d.b = b.p + (size_t)m * (q_ - icpt); d.b0 = b0.p + m;
+    }
+}
+
+IrlsLoop::~IrlsLoop() { event_release(ev_[0]); event_release(ev_[1]); }
+
+void IrlsLoop::set_model(int m, const double *XX, double *XY, double *d, const double *cinv, unsigned long long *t_acc) {
+    md_[m].XX = XX; md_[m].XY = XY; md_[m].d = d; md_[m].cinv = cinv; md_[m].t_acc = t_acc;
+}
+
+void IrlsLoop::path_step(int m, bool compute_eig, const double *grad, double n_rows) {
+    double *slots = iter_.p + (size_t)m * 2 * q_;
+    const int cur = (par0_[m] + k_) & 1;
+    path_launch(cx_, irls_path_problem(tb_, su_, pp_, i_, o_, md_[m], slots + (size_t)cur * q_, slots + (size_t)(cur ^ 1) * q_,
+                                       flag_.p + (gi_ & 3) * M_ + m, compute_eig, grad, n_rows));
+}
+
+double *IrlsLoop::final_iterate(int m) { return iter_.p + ((size_t)m * 2 + par0_[m]) * q_; }
+
+// Waits for round g (iteration k of the lambda) and reads the verdicts of the models it ran; false once none is left.
+// Without speculation nothing is enqueued behind round g, and a stream sync is cheaper than an event record per round.
+bool IrlsLoop::wait_round(long long g, int k) {
+    if (speculate_) {
+        cx_.st.host_syncs += 1;
+        OEM_CUDA(cudaEventSynchronize(ev_[g & 1]));
+    } else {
+        cx_.sync();
+    }
+    const int *verdict = flag_.p + (g & 3) * M_;
+    bool left = false;
+    for (int m = 0; m < M_; ++m) {
+        if (!active[m]) continue;
+        if (verdict[m]) { active[m] = 0; last_[m] = k; niter_h_[m] = k + 1; }
+        else left = true;
+    }
+    return left;
+}
+
+// niter as the reference reports it: executed iterations + 1 on convergence, irls_maxit + 1 at the cap
+void IrlsLoop::run(oemb200_result *res, const std::function<void(int, int, bool)> &round,
+                   const std::function<void(int, int)> &lambda_end) {
+    const int maxit = o_->irls_maxit, L = su_.Lmax;
+    auto enqueue = [&](int k) {
+        k_ = k;
+        round(i_, k, !(k == 0 && i_ > 0));
+        if (speculate_) OEM_CUDA(cudaEventRecord(ev_[gi_ & 1], cx_.stream));
+        ++gi_;
+    };
+    for (pp_ = 0; pp_ < su_.P; ++pp_) {
+        iter_.zero(cx_.stream);                          // init(): beta = 0, on_lam_1 = true
+        b.zero(cx_.stream);
+        b0.zero(cx_.stream);
+        std::fill(par0_.begin(), par0_.end(), 0);
+        for (i_ = 0; i_ < su_.nlam_run[pp_]; ++i_) {
+            conv.zero(cx_.stream);
+            std::fill(active.begin(), active.end(), 1);
+            int it = 0;
+            enqueue(0);
+            for (;;) {
+                // round `it` is in the stream (the last one, unless round it + 1 is enqueued ahead of its verdict)
+                const bool ahead = speculate_ && it + 1 < maxit;
+                const oemb200_stats before = cx_.st;
+                if (ahead) enqueue(it + 1);
+                if (!wait_round(gi_ - 1 - (ahead ? 1 : 0), it)) {
+                    if (ahead) {           // the speculative round found the lambda converged: nothing of it ran
+                        cx_.st.data_passes = before.data_passes; cx_.st.xb_launches = before.xb_launches;
+                        cx_.st.gemv_bytes = before.gemv_bytes; cx_.st.allreduce_calls = before.allreduce_calls;
+                        cx_.st.allreduce_doubles = before.allreduce_doubles;
+                    }
+                    break;
+                }
+                if (++it >= maxit) {
+                    for (int m = 0; m < M_; ++m)
+                        if (active[m]) { active[m] = 0; last_[m] = maxit - 1; niter_h_[m] = maxit + 1; }
+                    break;
+                }
+                if (!ahead) enqueue(it);
+            }
+            for (int m = 0; m < M_; ++m) par0_[m] = (par0_[m] + last_[m] + 1) & 1;
+            lambda_end(pp_, i_);
+            for (int m = 0; m < M_; ++m)
+                OEM_CUDA(cudaMemcpyAsync(path.p + (((size_t)m * su_.P + pp_) * L + i_) * q_, final_iterate(m),
+                                         sizeof(double) * q_, cudaMemcpyDeviceToDevice, cx_.stream));
+            res->niter[(size_t)pp_ * L + i_] = niter_h_[0];
+        }
+    }
+}
+
+void IrlsLoop::write_path(const double *cinv, oemb200_result *res) {
+    const int icpt = md_[0].icpt, p = q_ - icpt;
+    std::vector<double> hpath((size_t)su_.P * su_.Lmax * q_);
     long long iters_total = 0;
     double dval = 0.0;
-    OEM_CUDA(cudaMemcpyAsync(hpath.data(), path_dev, hpath.size() * 8, cudaMemcpyDeviceToHost, cx.stream));
-    OEM_CUDA(cudaMemcpyAsync(&iters_total, iters_total_dev, sizeof iters_total, cudaMemcpyDeviceToHost, cx.stream));
-    OEM_CUDA(cudaMemcpyAsync(&dval, d_dev, sizeof dval, cudaMemcpyDeviceToHost, cx.stream));
-    cx.sync();
-    cx.st.d2h_bytes += (int64_t)hpath.size() * 8;
-    cx.st.total_oem_iters += iters_total;
-    write_beta(su, hpath.data(), p, icpt, cinv, res);
+    OEM_CUDA(cudaMemcpyAsync(hpath.data(), path.p, hpath.size() * 8, cudaMemcpyDeviceToHost, cx_.stream));
+    OEM_CUDA(cudaMemcpyAsync(&iters_total, iters_total_.p, sizeof iters_total, cudaMemcpyDeviceToHost, cx_.stream));
+    OEM_CUDA(cudaMemcpyAsync(&dval, md_[0].d, sizeof dval, cudaMemcpyDeviceToHost, cx_.stream));
+    cx_.sync();
+    cx_.st.d2h_bytes += (int64_t)hpath.size() * 8;
+    cx_.st.total_oem_iters += iters_total;
+    write_beta(su_, hpath.data(), p, icpt, cinv, res);
     *res->d = dval;
 }
 

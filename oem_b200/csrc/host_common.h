@@ -1,9 +1,10 @@
 // host_common.h -- host-side bookkeeping shared by the fit drivers: penalty / group / lambda setup (the part of the
 // reference's entry functions that is not arithmetic on X) and its device mirror, the helper that runs a set of chains
-// through the path kernel and brings the raw iterates back, the one-lambda path problem of the IRLS drivers, and the
-// layout of the reported beta.
+// through the path kernel and brings the raw iterates back, the layout of the reported beta, and the parts of the three
+// logistic (IRLS) drivers that are not their data passes: the init step and the outer loop with its per-model state.
 #pragma once
 #include <cmath>
+#include <functional>
 #include <string>
 #include <vector>
 #include "runtime.h"
@@ -68,6 +69,22 @@ struct PathBuffers {
 void run_paths(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int ngram, const double *XX,
                const double *XY, double eig_factor, bool accelerate, const double *post_scale_dev, PathBuffers &pb);
 
+// res->beta (P x Lmax x (p + 1): intercept row first, zero where no lambda ran) from the raw q-vectors of a fit, iterate
+// (pp, i) at raw + (pp * Lmax + i) * q with q = p + icpt; cinv (host, p) undoes the standardisation, NULL if none.
+void write_beta(const Setup &su, const double *raw, int p, int icpt, const double *cinv, oemb200_result *res);
+
+// init_oem of the dense and sparse logistic drivers (src/oem_logistic_dense.h:721-793, oem_logistic_sparse.h:727-818):
+// colstats(out) enqueues [sum x | X'y | sum x^2] (3p) of this rank's rows into out; the sums and n are all-reduced and
+// brought to the host.  Refuses n <= q with `refusal`.  stats keeps the all-reduced sums on the device (then n at 3p).
+struct LogisticInit {
+    double n_tot = 0.0;
+    std::vector<double> cinv;     // host, p: 1 / sd of every column (ones when not standardised)
+    double lmax = 0.0;            // compute_lambda_zero: max_j |X'y o cinv| / n
+    DBuf<double> stats;
+};
+LogisticInit logistic_init(Ctx &cx, int64_t n, int p, int q, bool stdz, const std::function<void(double *)> &colstats,
+                           const char *refusal);
+
 // The device slots of one model of an IRLS loop: its system XX / XY (q = tb.q) and eigenvalue bound d, the path launch's
 // iteration count, Lanczos steps and tables, the convergence flag that predicates the model's work, the running count of
 // inner iterations (may be shared by models), and the coefficients of the model's next data pass, b (p = q - icpt) and
@@ -84,22 +101,6 @@ struct IrlsModel {
     double *b = nullptr, *b0 = nullptr;
     unsigned long long *t_acc = nullptr;
 };
-// One IRLS iteration's path launch (src/oem_logistic_dense.h:999-1033) for model m: lambda i of penalty pp, one chain, warm
-// started from cur, eigenvalue factor 1.0005 (recomputed when compute_eig), predicated on *m.conv.  Its last step is the
-// outer stop rule on (nxt, cur), whose verdict goes to *m.conv and *verdict, and b / b0 from nxt.  With grad (device,
-// [sum r, X'r] over n_rows rows) it first forms XY = XX cur + grad / n_rows (scaled by cinv); without, it keeps the XY of
-// the model's previous data pass.
-PathProblem irls_path_problem(const PenaltyTables &tb, const Setup &su, int pp, int i, const oemb200_opts *o, const IrlsModel &m,
-                              const double *cur, double *nxt, volatile int *verdict, bool compute_eig, const double *grad,
-                              double n_rows);
-
-// res->beta (P x Lmax x (p + 1): intercept row first, zero where no lambda ran) from the raw q-vectors of a fit, iterate
-// (pp, i) at raw + (pp * Lmax + i) * q with q = p + icpt; cinv (host, p) undoes the standardisation, NULL if none.
-void write_beta(const Setup &su, const double *raw, int p, int icpt, const double *cinv, oemb200_result *res);
-// End of an IRLS driver: one sync brings the raw path (P x Lmax x q at path_dev), d of the first model and the count of
-// inner iterations to the host, after whatever the caller enqueued before; then res->beta (write_beta) and *res->d.
-void irls_write_path(Ctx &cx, const Setup &su, int p, int icpt, const double *path_dev, const long long *iters_total_dev,
-                     const double *d_dev, const double *cinv, oemb200_result *res);
 
 // n mapped pinned ints: the IRLS verdict slots a path launch writes (PathProblem::irls_host_flag) and the host reads
 struct PinnedFlags {
@@ -115,6 +116,60 @@ struct PathScratches {
     std::vector<PathScratch *> s;
     explicit PathScratches(int n) { for (int i = 0; i < n; ++i) s.push_back(path_scratch_create()); }
     ~PathScratches() { for (auto *x : s) path_scratch_destroy(x); }
+};
+
+// The outer IRLS loop (src/oem_logistic_dense.h:1000-1035) of M logistic models in lockstep, and their device state.  Per
+// penalty every model starts from beta = 0, so the first data pass multiplies X with b = 0, b0 = 0.  Per lambda, round k
+// enqueues iteration k of every model still iterating: the driver's data pass, then one path launch per model
+// (path_step), which writes the model's stop-rule verdict to the device flag that predicates the model's later kernels of
+// the lambda and to a mapped host slot.  The host's one round trip per round is a wait for the round (an event wait
+// with speculation, else a stream sync) and a read of those verdicts.  With `speculate` (M = 1 only) round k + 1 is
+// enqueued before round k's verdict is read, so the GPU never waits for the host (the gap was ~100 us per iteration: 5 %
+// of a dense fit on one GPU, 25 % row-sharded over eight); a round enqueued after convergence is a few empty launches,
+// and its counters are rolled back.  Only a driver whose every kernel of the chain can be predicated may speculate.
+class IrlsLoop {
+public:
+    IrlsLoop(Ctx &cx, const Setup &su, const PenaltyTables &tb, const oemb200_opts *o, int M, int icpt, bool speculate);
+    IrlsLoop(const IrlsLoop &) = delete;
+    ~IrlsLoop();
+    // the device slots of model m that the driver owns (see IrlsModel)
+    void set_model(int m, const double *XX, double *XY, double *d, const double *cinv, unsigned long long *t_acc = nullptr);
+
+    DBuf<double> b, b0;          // M x p, M: the coefficients of each model's next data pass
+    DBuf<int> conv;              // M: the model has converged in this lambda (the predicate of its kernels)
+    DBuf<double> path;           // M x P x Lmax x q raw iterates, model m's penalty pp at chain m * P + pp
+    std::vector<char> active;    // host, M: the models still iterating in this lambda
+
+    // Every lambda of every penalty: round(i, k, pass) enqueues round k of lambda i (pass = false on a warm lambda's first
+    // iteration, where the reference skips the data pass), ending with path_step for every active model.  When every
+    // model has stopped, lambda_end(pp, i) runs, then the final iterates go into `path` and model 0's niter into res.
+    void run(oemb200_result *res, const std::function<void(int, int, bool)> &round,
+             const std::function<void(int, int)> &lambda_end);
+    // model m's path launch of this round.  compute_eig: the Hessian was rebuilt; with grad (device, [sum r, X'r] over
+    // n_rows rows) the launch first forms XY = XX beta + grad / n_rows (scaled by cinv), without it keeps the last XY
+    void path_step(int m, bool compute_eig, const double *grad, double n_rows);
+    double *final_iterate(int m);       // in lambda_end: the iterate of the model's last executed iteration
+    // after the loop: model 0's path, d and the count of inner iterations into res (cinv: host, p; NULL if none)
+    void write_path(const double *cinv, oemb200_result *res);
+
+private:
+    Ctx &cx_;
+    const Setup &su_;
+    const PenaltyTables &tb_;
+    const oemb200_opts *o_;
+    const int M_, q_;
+    const bool speculate_;
+    DBuf<double> iter_;                  // M x 2 x q: the model's iterate ping-pongs between its two slots
+    DBuf<int> niter_, lz_;
+    DBuf<long long> iters_total_;
+    PathScratches scratch_;
+    std::vector<IrlsModel> md_;
+    PinnedFlags flag_;                   // 4 x M verdict slots: round g writes row g & 3
+    cudaEvent_t ev_[2];                  // with speculation, recorded after round g: ev_[g & 1]
+    long long gi_ = 0;                   // rounds enqueued so far
+    int pp_ = 0, i_ = 0, k_ = 0;         // the round being enqueued
+    std::vector<int> par0_, last_, niter_h_;   // per model: slot of iteration 0, last executed iteration, reported niter
+    bool wait_round(long long g, int k);
 };
 
 // ---- shared by the entry drivers (entries.cu) ----

@@ -265,16 +265,18 @@ def test_against_the_oracle_twin(lib, oracle, standardize, intercept):
 @pytest.mark.gpu
 def test_irls_maxit_exhausted_and_bit_reproducible(lib):
     X, y, foldid = problem(seed=5, n=2500, p=20, nfolds=4)
-    a = args_xy(X, y, "binomial", ["lasso"], nlambda=10, lmin_ratio=1e-3, opts=dict(irls_maxit=2, irls_tol=1e-12))
-    r1 = lib.oem_xval_logistic_dense(*xargs(a, 4, foldid))
-    r2 = lib.oem_xval_logistic_dense(*xargs(a, 4, foldid))
-    ref = lib.oem_fit_logistic_dense(*a)
-    assert np.all(r1["niter"][0] == 3)                          # maxit + 1, as the reference reports an exhausted loop
-    assert_same_fit(r1, ref, tol=1e-8)
-    for key in ("beta", "niter", "cvm", "cvsd"):
-        for u, v in zip(r1[key], r2[key]):
-            assert np.array_equal(u, v), key
-    assert r1["d"] == r2["d"]
+    for maxit in (1, 2, 3):
+        a = args_xy(X, y, "binomial", ["lasso"], nlambda=10, lmin_ratio=1e-3, opts=dict(irls_maxit=maxit, irls_tol=1e-12))
+        r1 = lib.oem_xval_logistic_dense(*xargs(a, 4, foldid))
+        r2 = lib.oem_xval_logistic_dense(*xargs(a, 4, foldid))
+        ref = lib.oem_fit_logistic_dense(*a)
+        assert np.all(r1["niter"][0] == maxit + 1), maxit      # as the reference reports an exhausted loop
+        assert np.array_equal(r1["niter"][0], ref["niter"][0]), maxit
+        assert_same_fit(r1, ref, tol=1e-8)
+        for key in ("beta", "niter", "cvm", "cvsd"):
+            for u, v in zip(r1[key], r2[key]):
+                assert np.array_equal(u, v), (key, maxit)
+        assert r1["d"] == r2["d"]
 
 
 @pytest.mark.gpu

@@ -7,6 +7,7 @@
  *   oemb200_fit_dense            replaces  oem_fit_dense            src/oem_dense.cpp:30-48
  *   oemb200_xtx                  replaces  oem_xtx                  src/oem_xtx.cpp:29-44
  *   oemb200_xval_dense           replaces  oem_xval_dense           src/oem_xval_dense.cpp:31-52
+ *   oemb200_xval_big             oem_xval_dense on an x streamed in row chunks (no reference counterpart)
  *   oemb200_fit_logistic_dense   replaces  oem_fit_logistic_dense   src/oem_logistic_dense.cpp:29-47
  *   oemb200_fit_big              replaces  oem_fit_big / oem_fit_fb_big   src/oem_big.cpp:30-48
  *   oemb200_fit_sparse           replaces  oem_fit_sparse           src/oem_sparse.cpp:30
@@ -191,6 +192,22 @@ int oemb200_xtx(const double *xtx, const double *xty, int p,
 int oemb200_xval_dense(const double *x, int64_t n, int p, int64_t ldx, const double *y,
                        const oemb200_spec *spec, int nfolds, const int *foldid,
                        const char *type_measure, const oemb200_opts *opts, oemb200_result *res);
+
+/* oemb200_xval_dense on an x that is never resident on the device: same arguments, same meaning, same result layout
+ * (weights, the standardize x intercept flags, "mse" | "mae" | "deviance" (= mse), compute_loss, foldid on the host or
+ * the device, more than 64 folds with a host foldid).  x (and y, weights, foldid) may be pageable or pinned host memory
+ * or device memory (e.g. the data of an oemb200_matrix whose fold-sorted copy would not fit beside it); x is read in row
+ * chunks of opts->gigs GB, twice: one pass forms the fold Grams, one scores the fold models after the path.  Device
+ * memory does not grow with n: two staging chunks (host x only), one fold-sorted chunk, the fold Grams, the nfolds + 1
+ * systems, the path and the coefficient matrices.  stats: data_passes = 2, gram_launches = the number of chunks,
+ * h2d_bytes = every host-to-device copy (a host x, y and weights once per pass, a host foldid three times: once to count
+ * the rows of every (chunk, fold), once per pass), host_syncs independent of the number of chunks.  Results agree with
+ * oemb200_xval_dense up to summation order (bit for bit when x is one chunk).  OEMB200_EUNSUPPORTED, before any device
+ * work, for the binomial family (each IRLS round would be another pass over the host link) and row-sharded calls
+ * (world > 1, comm or allreduce). */
+int oemb200_xval_big(const double *x, int64_t n, int p, int64_t ldx, const double *y,
+                     const oemb200_spec *spec, int nfolds, const int *foldid,
+                     const char *type_measure, const oemb200_opts *opts, oemb200_result *res);
 
 /* Binomial cross-validation (the reference's xval.oem stops on the binomial family, R/oem_xval.R:160-163): the full-data
  * model is oemb200_fit_logistic_dense on all rows, fold model k the same fit on the rows with foldid != k at the full

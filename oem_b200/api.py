@@ -103,6 +103,7 @@ def load():
     L.oemb200_xtx.argtypes = [vp, vp, ci, sp, vp, ci, op, rp]
     L.oemb200_xval_dense.argtypes = [vp, i64, ci, i64, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
     L.oemb200_xval_logistic_dense.argtypes = [vp, i64, ci, i64, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
+    L.oemb200_xval_big.argtypes = [vp, i64, ci, i64, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
     L.oemb200_xval_logistic_dense_h.argtypes = [vp, vp, sp, ci, vp, ctypes.c_char_p, op, rp]
     L.oemb200_logit_fold_pass.argtypes = [vp, i64, ci, i64, vp, vp, vp, vp, ci, vp, vp, ci, vp, ctypes.POINTER(dbl),
                                           ctypes.POINTER(dbl), ctypes.POINTER(ci)]
@@ -146,7 +147,7 @@ EXPORTS = ["oemb200_last_error", "oemb200_version", "oemb200_device_count", "oem
            "oemb200_fit_dense_h", "oemb200_fit_big_h", "oemb200_fit_logistic_dense_h", "oemb200_xval_dense_h",
            "oemb200_predict_h", "oemb200_comm_unique_id", "oemb200_comm_create", "oemb200_comm_from_nccl", "oemb200_comm_destroy",
            "oemb200_comm_allreduce", "oemb200_comm_p2p_enabled", "oemb200_xval_logistic_dense",
-           "oemb200_xval_logistic_dense_h", "oemb200_logit_fold_pass"]
+           "oemb200_xval_logistic_dense_h", "oemb200_logit_fold_pass", "oemb200_xval_big"]
 
 
 def lambda_grid(lmax, nlambda, lmin_ratio):
@@ -225,7 +226,12 @@ class _Keep:
 
 
 def _matrix_arg(x, keep):
-    """-> (pointer, n, p, ld) for a column-major matrix on host (numpy) or device (torch)."""
+    """-> (pointer, n, p, ld) for a column-major matrix on host (numpy), on device (torch) or held by a DeviceMatrix."""
+    if isinstance(x, DeviceMatrix):
+        if not x.handle:
+            raise ValueError("DeviceMatrix has been closed")
+        keep.refs.append(x)
+        return x.data_ptr, x.shape[0], x.shape[1], x.ld
     if _is_torch_cuda(x):
         import torch
         if x.dtype != torch.float64 or x.dim() != 2:
@@ -361,7 +367,7 @@ def _run_xy(fn_name, x, y, family, penalty, weights, groups, unique_groups, grou
             extra=None):
     L = load()
     keep = _Keep()
-    handle = isinstance(x, DeviceMatrix)
+    handle = isinstance(x, DeviceMatrix) and fn_name != "oemb200_xval_big"
     if handle:
         if not x.handle:
             raise ValueError("DeviceMatrix has been closed")
@@ -377,7 +383,8 @@ def _run_xy(fn_name, x, y, family, penalty, weights, groups, unique_groups, grou
                       lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept, compute_loss)
     o = opts if isinstance(opts, Opts) else make_opts(opts, comm)
     Lmax = L.oemb200_nlambda_max(ctypes.byref(spec))
-    out = _Out(len(penalty), Lmax, p + 1, xval=fn_name.startswith(("oemb200_xval_dense", "oemb200_xval_logistic_dense")))
+    out = _Out(len(penalty), Lmax, p + 1,
+               xval=fn_name.startswith(("oemb200_xval_dense", "oemb200_xval_logistic_dense", "oemb200_xval_big")))
     fn = getattr(L, fn_name)
     if extra is None:
         rc = fn(*xargs, yp, ctypes.byref(spec), ctypes.byref(o), ctypes.byref(out.res))
@@ -480,6 +487,20 @@ def oem_xval_dense(x, y, family, penalty, weights, groups, unique_groups, group_
         f = keep.arr(foldid, np.int32)
         return [int(nfolds), f.ctypes.data, type_measure.encode()]
     return _run_xy("oemb200_xval_dense", x, y, family, penalty, weights, groups, unique_groups, group_weights,
+                   lambda_, nlambda, lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept,
+                   compute_loss, opts, comm, extra=extra)
+
+
+def oem_xval_big(x, y, family, penalty, weights, groups, unique_groups, group_weights, lambda_, nlambda,
+                 lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept, nfolds, foldid,
+                 compute_loss, type_measure, opts, comm=None):
+    """oem_xval_dense on an x that is never resident on the device (include/oem_b200.h: oemb200_xval_big): x is read
+    in row chunks of opts["gigs"] GB, once to form the fold Grams and once to score the fold models.  x is a numpy
+    array, an np.memmap (e.g. oem_b200.bigmatrix.attach of a .bk file; pinned memory is copied without staging), a
+    column-major CUDA tensor or a DeviceMatrix (read in place, no fold-sorted copy).  Gaussian family, one GPU."""
+    def extra(keep):
+        return [int(nfolds), _int_array_arg(foldid, keep), type_measure.encode()]
+    return _run_xy("oemb200_xval_big", x, y, family, penalty, weights, groups, unique_groups, group_weights,
                    lambda_, nlambda, lmin_ratio, alpha, gamma, tau, penalty_factor, standardize, intercept,
                    compute_loss, opts, comm, extra=extra)
 

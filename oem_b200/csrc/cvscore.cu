@@ -160,6 +160,27 @@ fold_rank_kernel(const int *__restrict__ foldid, long long n, int F, const int *
     }
 }
 
+// Per-fold row counts of foldid[0, n): fold_count_kernel's per-tile histogram, turned by fold_scan_kernel into each tile's
+// exclusive prefix (tcount, what fold_rank_launch reads) and the fold totals (device, F).  Bad ids set *err.
+void fold_count_launch(Ctx &cx, const int *foldid_dev, int64_t n, int F, int *tcount, int *err, long long *total) {
+    const int ntiles = (int)((n + FG_ROWS - 1) / FG_ROWS);
+    fold_count_kernel<<<ntiles, 256, 0, cx.stream>>>(foldid_dev, n, F, tcount, err);
+    fold_scan_kernel<<<1, FB_MAXF, 0, cx.stream>>>(tcount, ntiles, F, total);
+    OEM_CUDA(cudaGetLastError());
+    cx.st.kernel_launches += 2;
+}
+
+// dest / order of foldid[0, n) from fold_count_launch's tile prefixes and the first sorted row of every fold (base, device)
+void fold_rank_launch(Ctx &cx, const int *foldid_dev, int64_t n, int F, const int *tcount, const long long *base, int *dest,
+                      int *order) {
+    const int ntiles = (int)((n + FG_ROWS - 1) / FG_ROWS);
+    fold_rank_kernel<<<ntiles, 256, 0, cx.stream>>>(foldid_dev, n, F, tcount, base, dest, order);
+    OEM_CUDA(cudaGetLastError());
+    cx.st.kernel_launches += 1;
+}
+
+int fold_bucket_max_folds() { return FB_MAXF; }
+
 // Device-side bucketing: fills dest / order (device) and counts (host).  Returns false if nfolds is too large for
 // this path (the caller then buckets on the host).
 bool fold_bucket_device(Ctx &cx, const int *foldid_dev, int64_t n, int F, int64_t align, int *dest, int *order,
@@ -169,9 +190,7 @@ bool fold_bucket_device(Ctx &cx, const int *foldid_dev, int64_t n, int F, int64_
     DBuf<int> tcount((size_t)ntiles * F), err(1);
     DBuf<long long> total(F), base(F);
     err.zero(cx.stream);
-    fold_count_kernel<<<ntiles, 256, 0, cx.stream>>>(foldid_dev, n, F, tcount.p, err.p);
-    fold_scan_kernel<<<1, FB_MAXF, 0, cx.stream>>>(tcount.p, ntiles, F, total.p);
-    OEM_CUDA(cudaGetLastError());
+    fold_count_launch(cx, foldid_dev, n, F, tcount.p, err.p, total.p);
     std::vector<long long> ht(F);
     int herr = 0;
     total.download(ht.data(), F, cx.stream);
@@ -187,9 +206,7 @@ bool fold_bucket_device(Ctx &cx, const int *foldid_dev, int64_t n, int F, int64_
         hb[k] = off[k];
     }
     base.upload(hb.data(), F, cx.stream);
-    fold_rank_kernel<<<ntiles, 256, 0, cx.stream>>>(foldid_dev, n, F, tcount.p, base.p, dest, order);
-    OEM_CUDA(cudaGetLastError());
-    cx.st.kernel_launches += 3;
+    fold_rank_launch(cx, foldid_dev, n, F, tcount.p, base.p, dest, order);
     cx.sync();      // tcount / base go back to the pool
     return true;
 }
@@ -496,13 +513,16 @@ cvscore_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
     }
 }
 
-// out[c] = (count, mean, M2) merged over this column block's items in item order
+// out[c] = (count, mean, M2) merged over this column block's items in item order.  accumulate: the merge starts from the
+// (count, mean, M2) already in out3 instead of the empty state, so that row chunks scored one launch at a time merge in
+// chunk order (Chan's update; from the empty state the first merge reproduces its operand exactly).
 __global__ void cv_merge_kernel(const double *__restrict__ partial, int part_stride, const CvItem *__restrict__ items,
-                                int nitems, int nc, int cols, double *__restrict__ out3) {
+                                int nitems, int nc, int cols, double *__restrict__ out3, int accumulate) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= nc) return;
     const int cb = c / cols, cl = c - cb * cols;
     double n = 0.0, mean = 0.0, m2 = 0.0;
+    if (accumulate) { n = out3[c]; mean = out3[nc + c]; m2 = out3[2 * nc + c]; }
     for (int i = 0; i < nitems; ++i) {
         if (items[i].colblock != cb) continue;
         const double *pp = partial + (size_t)i * part_stride;
@@ -539,7 +559,8 @@ int cv_ncld(int nc) { return (nc + CV_COLS - 1) / CV_COLS * CV_COLS + 8; }
 // fold-sorted order.  epi < EPI_LINK: out = 3 x nc (count, mean, M2); else out = predictions, column-major, ld ldo.
 static void cv_gemm_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys,
                            const double *ws, int nfolds, const std::vector<std::array<int64_t, 3>> &segs,
-                           const double *B, const double *b0, int nc, int epi, double *out, int64_t ldo) {
+                           const double *B, const double *b0, int nc, int epi, double *out, int64_t ldo,
+                           bool accumulate = false) {
     const int ncld = cv_ncld(nc);
     const int nh = nc <= CV_BHALF ? 1 : 2;                  // narrow problems: 128 x 160 tiles
     const int cols = CV_BHALF * nh, rows = nh == 2 ? 64 : 128;
@@ -618,7 +639,8 @@ static void cv_gemm_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p
     OEM_CUDA(cudaGetLastError());
     cx.st.kernel_launches += 1;
     if (!store) {
-        cv_merge_kernel<<<(nc + 127) / 128, 128, 0, cx.stream>>>(partial.p, part_stride, d_items.p, (int)items.size(), nc, cols, out);
+        cv_merge_kernel<<<(nc + 127) / 128, 128, 0, cx.stream>>>(partial.p, part_stride, d_items.p, (int)items.size(), nc, cols, out,
+                                                                 accumulate ? 1 : 0);
         OEM_CUDA(cudaGetLastError());
         cx.st.kernel_launches += 1;
     }
@@ -627,8 +649,8 @@ static void cv_gemm_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p
 
 void cvscore_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys,
                     const double *ws, int nfolds, const std::vector<std::array<int64_t, 3>> &segs, const double *B,
-                    const double *b0, int nc, bool mae, double *out3) {
-    cv_gemm_launch(cx, Xs, nrows_total, p, lds, ys, ws, nfolds, segs, B, b0, nc, mae ? EPI_MAE : EPI_MSE, out3, 0);
+                    const double *b0, int nc, bool mae, double *out3, bool accumulate) {
+    cv_gemm_launch(cx, Xs, nrows_total, p, lds, ys, ws, nfolds, segs, B, b0, nc, mae ? EPI_MAE : EPI_MSE, out3, 0, accumulate);
 }
 
 void cvscore_binomial_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys, int nfolds,

@@ -69,6 +69,14 @@ void fill_common_outputs(const Setup &su, oemb200_result *res) {
     }
 }
 
+int64_t big_chunk_rows(const oemb200_opts *o, int64_t n, int p) {
+    const double gigs = o->gigs > 0 ? o->gigs : 1.0;
+    int64_t rows = (int64_t)(gigs * 1e9 / (8.0 * p));
+    const int64_t align = 2 * gram_kt();
+    rows = std::max<int64_t>(align, rows / align * align);
+    return std::min<int64_t>(rows, (n + align - 1) / align * align);
+}
+
 void finish_stats(Ctx &cx, PhaseTimers &tm, size_t total_id, oemb200_result *res) {
     tm.stop(total_id);
     cx.finish();
@@ -106,31 +114,11 @@ static void fit_big(const double *x, int64_t n, int p, int64_t ldx, const double
         gram_launch(cx, x, n, p, ldx, {RowSegment{0, n, 0}}, 1, nullptr, nullptr, G, false, yv.p, stats);
     } else {
         // host X: double-buffered row chunks; H2D of chunk c+1 overlaps the kernels of chunk c
-        const double gigs = o->gigs > 0 ? o->gigs : 1.0;
-        int64_t rows = (int64_t)(gigs * 1e9 / (8.0 * p));
-        const int64_t align = 2 * gram_kt();
-        rows = std::max<int64_t>(align, rows / align * align);
-        rows = std::min<int64_t>(rows, (n + align - 1) / align * align);
+        const int64_t rows = big_chunk_rows(o, n, p);
         DBuf<double> stage[2];
         stage[0].alloc((size_t)rows * p);
         stage[1].alloc((size_t)rows * p);
-        // copy stream + ping-pong events, released on every exit path (a throwing launch included)
-        struct CopyLane {
-            cudaStream_t s = nullptr;
-            cudaEvent_t ready[2] = {nullptr, nullptr}, freed[2] = {nullptr, nullptr};
-            CopyLane() {
-                OEM_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-                for (int b = 0; b < 2; ++b) {
-                    OEM_CUDA(cudaEventCreateWithFlags(&ready[b], cudaEventDisableTiming));
-                    OEM_CUDA(cudaEventCreateWithFlags(&freed[b], cudaEventDisableTiming));
-                }
-            }
-            ~CopyLane() {
-                if (s) cudaStreamSynchronize(s);
-                for (int b = 0; b < 2; ++b) { if (ready[b]) cudaEventDestroy(ready[b]); if (freed[b]) cudaEventDestroy(freed[b]); }
-                if (s) cudaStreamDestroy(s);
-            }
-        } lane;
+        CopyLane lane;
         cudaStream_t cs = lane.s;
         cudaEvent_t *ready = lane.ready, *freed = lane.freed;
         const int64_t nchunks = (n + rows - 1) / rows;
@@ -477,6 +465,8 @@ void fit_xval(const double *x, int64_t n, int p, int64_t ldx, const double *y, c
               const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res);
 void fit_xval_logistic(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s, int nfolds,
                        const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res);
+void fit_xval_big(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *s, int nfolds,
+                  const int *foldid, const char *type_measure, const oemb200_opts *o, oemb200_result *res);
 
 template <typename F>
 static int guarded(F &&f) {
@@ -620,6 +610,10 @@ int oemb200_xval_dense(const double *x, int64_t n, int p, int64_t ldx, const dou
                        int nfolds, const int *foldid, const char *type_measure, const oemb200_opts *opts,
                        oemb200_result *res) {
     return guarded([&] { fit_xval(x, n, p, ldx, y, spec, nfolds, foldid, type_measure, opts, res); });
+}
+int oemb200_xval_big(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *spec, int nfolds,
+                     const int *foldid, const char *type_measure, const oemb200_opts *opts, oemb200_result *res) {
+    return guarded([&] { fit_xval_big(x, n, p, ldx, y, spec, nfolds, foldid, type_measure, opts, res); });
 }
 int oemb200_xval_logistic_dense(const double *x, int64_t n, int p, int64_t ldx, const double *y, const oemb200_spec *spec,
                                 int nfolds, const int *foldid, const char *type_measure, const oemb200_opts *opts,

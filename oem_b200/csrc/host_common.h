@@ -172,6 +172,26 @@ private:
     bool wait_round(long long g, int k);
 };
 
+// Copy stream of a streamed pass over host row chunks, with ping-pong events: ready[b] = staging buffer b holds its chunk,
+// freed[b] = the compute stream is done reading it.  Released on every exit path (a throwing launch included).
+struct CopyLane {
+    cudaStream_t s = nullptr;
+    cudaEvent_t ready[2] = {nullptr, nullptr}, freed[2] = {nullptr, nullptr};
+    CopyLane() {
+        OEM_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+        for (int b = 0; b < 2; ++b) {
+            OEM_CUDA(cudaEventCreateWithFlags(&ready[b], cudaEventDisableTiming));
+            OEM_CUDA(cudaEventCreateWithFlags(&freed[b], cudaEventDisableTiming));
+        }
+    }
+    CopyLane(const CopyLane &) = delete;
+    ~CopyLane() {
+        if (s) cudaStreamSynchronize(s);
+        for (int b = 0; b < 2; ++b) { if (ready[b]) cudaEventDestroy(ready[b]); if (freed[b]) cudaEventDestroy(freed[b]); }
+        if (s) cudaStreamDestroy(s);
+    }
+};
+
 // ---- shared by the entry drivers (entries.cu) ----
 void check_common(const oemb200_spec *s, const oemb200_opts *o, const oemb200_result *r, const char *want_family,
                   bool allow_weights = false);
@@ -180,6 +200,9 @@ struct DevVector { const double *p = nullptr; DBuf<double> own; };
 void to_device_matrix(Ctx &cx, const double *x, int64_t n, int p, int64_t ldx, DevMatrix &m);
 void to_device_vector(Ctx &cx, const double *v, int64_t n, DevVector &d);
 void fill_common_outputs(const Setup &su, oemb200_result *res);
+// rows per chunk of a pass that streams X: opts->gigs GB (1 when unset), a multiple of the fold-segment alignment
+// 2 * gram_kt(), at most n rounded up to it
+int64_t big_chunk_rows(const oemb200_opts *o, int64_t n, int p);
 
 // ---- entry_sparse.cu: a dgCMatrix design on the device (validated CSC slots + CSR copy) and the passes over it ----
 struct SparseDesign;
@@ -207,6 +230,10 @@ struct XvalSystems {
 // upper-bound Hessian X'WX at beta = 0 has W = 1/4; a power of two, so the scaled sums are exact); 1 = no launch.
 void xval_build_systems(Ctx &cx, const double *x, int64_t n, int p, int64_t ldx, const double *y, const double *weights,
                         int F, const int *foldid, int icpt, bool stdz, double hess_scale, XvalSystems &xs);
+// stable counting sort of the rows by fold on the host (more folds than fold_bucket_max_folds()): cnt / off as in
+// XvalSystems, dest / order (n ints each) for fold_gather_launch; refuses ids outside 1..F
+void xval_bucket_host(const int *foldid, int64_t n, int F, int64_t align, std::vector<int64_t> &cnt, std::vector<int64_t> &off,
+                      int *dest, int *order);
 
 // ---- entry_logistic.cu ----
 // get_loss() of prob (src/oem_logistic_dense.h:1057-1088) summed over the n rows and over ranks

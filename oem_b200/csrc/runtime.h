@@ -295,12 +295,20 @@ int fold_gather_tile_rows();
 // stable counting sort of the rows by fold on the device (nfolds <= 64): dest, order (device), cnt / off (host)
 bool fold_bucket_device(Ctx &cx, const int *foldid_dev, int64_t n, int F, int64_t align, int *dest, int *order,
                         std::vector<int64_t> &cnt, std::vector<int64_t> &off);
+// its two halves, with no host round trip in between: per-tile prefixes tcount (ceil(n / fold_gather_tile_rows()) x F),
+// fold totals (device, F) and *err (set on an id outside 1..F); then dest / order from tcount and each fold's first
+// sorted row base (device, F)
+void fold_count_launch(Ctx &cx, const int *foldid_dev, int64_t n, int F, int *tcount, int *err, long long *total);
+void fold_rank_launch(Ctx &cx, const int *foldid_dev, int64_t n, int F, const int *tcount, const long long *base, int *dest,
+                      int *order);
+int fold_bucket_max_folds();     // largest nfolds of the device bucketing
 int cv_ncld(int nc);     // leading dimension (columns) of the coefficient matrices handed to cvscore_launch
 // out3 = 3 x nc: (count, mean, M2) of t = (y - pred)^2 | |y - pred| over all valid rows, per column
-// ws: optional observation weights (fold-sorted like ys): t is multiplied by w_i
+// ws: optional observation weights (fold-sorted like ys): t is multiplied by w_i.  accumulate: merge these rows' moments
+// into the (count, mean, M2) already in out3 (after them, in a fixed order), for rows scored one chunk at a time
 void cvscore_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys,
                     const double *ws, int nfolds, const std::vector<std::array<int64_t, 3>> &segs, const double *B,
-                    const double *b0, int nc, bool mae, double *out3);
+                    const double *b0, int nc, bool mae, double *out3, bool accumulate = false);
 // the same moments of cv.oem's binomial measures (R/cv_oem.R:288-330) on p = 1 / (1 + exp(-(x . b + b0))), unweighted:
 // measure 0 = deviance (p clamped to [1e-5, 1 - 1e-5]), 1 = class error (p > 0.5) != y, 2 = 2 (y - p)^2, 3 = 2 |y - p|
 void cvscore_binomial_launch(Ctx &cx, const double *Xs, int64_t nrows_total, int p, int64_t lds, const double *ys, int nfolds,

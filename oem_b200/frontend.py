@@ -246,15 +246,20 @@ def xval_oem(x, y, nfolds=10, foldid=None, type_measure=None, ncores=-1, family=
              lambda_=(), nlambda=100, lambda_min_ratio=None, alpha=1.0, gamma=3.0, tau=0.5, groups=(),
              penalty_factor=None, group_weights=None, standardize=True, intercept=True, maxit=500, tol=1e-7,
              irls_maxit=100, irls_tol=1e-3, compute_loss=False, varnames=None, seed=None, comm=None,
-             hessian_type="upper.bound"):
+             hessian_type="upper.bound", gigs=None):
     """R/oem_xval.R:107-460: fit + fast cross-validation in one call; adds lambda.min / lambda.1se / cvup / cvlo.
     type.measure: gaussian mse (default) | deviance | mae; binomial deviance (default) | class | mse | mae.
     family = "binomial" (which the reference's xval.oem refuses, R/oem_xval.R:160-163) runs oem_xval_logistic_dense:
     the full-data logistic fit of oem() plus one fit per fold at its lambdas, scored with cv.oem's binomial measures
-    over all rows; `auc` needs per-fold ranks and stays with cv_oem()."""
+    over all rows; `auc` needs per-fold ranks and stays with cv_oem().
+    gigs (gaussian only): stream x to the GPU in row chunks of `gigs` GB instead of holding it there (oem_xval_big), for
+    an x larger than device memory, e.g. xval_oem(bigmatrix.attach("x.desc"), y, gigs=4); the same fit and scores."""
     if family not in ("gaussian", "binomial"):
         raise ValueError("'arg' should be one of 'gaussian', 'binomial'")
     binomial = family == "binomial"
+    if binomial and gigs is not None:
+        raise ValueError("gigs streams x for the gaussian family only: every IRLS round of a binomial fit would be "
+                         "another pass over the host link")
     if type_measure is None:
         type_measure = "deviance" if binomial else "mse"
     if binomial:
@@ -293,9 +298,13 @@ def xval_oem(x, y, nfolds=10, foldid=None, type_measure=None, ncores=-1, family=
                                           float(tau), pf, bool(standardize), bool(intercept), int(nfolds),
                                           foldid.astype(np.int32), bool(compute_loss), type_measure, opts, comm=comm)
     else:
-        res = api.oem_xval_dense(x, y, family, penalty, weights, g, ug, gw, lam, int(nlambda), lmr, float(alpha), gamma,
-                                 float(tau), pf, bool(standardize), bool(intercept), int(nfolds), foldid.astype(np.int32),
-                                 bool(compute_loss), "mse" if type_measure == "deviance" else type_measure, opts, comm=comm)
+        fn = api.oem_xval_dense
+        if gigs is not None:
+            fn = api.oem_xval_big
+            opts["gigs"] = float(gigs)
+        res = fn(x, y, family, penalty, weights, g, ug, gw, lam, int(nlambda), lmr, float(alpha), gamma, float(tau), pf,
+                 bool(standardize), bool(intercept), int(nfolds), foldid.astype(np.int32), bool(compute_loss),
+                 "mse" if type_measure == "deviance" else type_measure, opts, comm=comm)
     out = _decorate(res, penalty, n, p, family, varnames)
     out.update(getmin(out["lambda"], out["cvm"], out["cvsd"]))
     out["cvup"] = [m + s for m, s in zip(out["cvm"], out["cvsd"])]
